@@ -17,6 +17,12 @@ default workload is BASELINE.json configs[3]: synthetic, 100 000 points, 99 % mi
              achieved = algorithmic flop per iteration / kernel time, peak = FFMA rate measured live by
              topolow_microbench on the same GPU.  `hbm` gives the edge stream against MEASURED_PEAKS.
   cpu_baseline / --impl reference: oracle/ (the CPU restatement of src/optimization.cpp) on the host.
+
+  --dump-outputs DIR   after the timed steps, what the resident leg hands its caller as float64 DIR/<name>.npy:
+                       the best-iteration positions (the snapshot topolow_shard_result / topolow_plan_result
+                       return, as in the reference), the MAE at each check iteration and the controller scalars;
+                       the inputs are seeded, so two builds run with the same arguments can be compared output
+                       for output.
 """
 from __future__ import annotations
 
@@ -148,6 +154,26 @@ def map_config(workload, n, d, missing, E, early_stop=None):
             "early_stop": early_stop or "disabled (convergence_counter = n_iter + 1): every step is one full iteration",
             "l2": "inputs larger than L2: the edge records streamed every iteration (%.0f MB over all ranks) exceed the 126 MB L2; "
                   "the %.1f MB position replica is the resident working set, as in production" % (E * 16 / 1e6, n * d * 4 / 1e6)}
+
+
+DUMP_SCALARS = ("final_mae", "final_k", "iterations", "iterations_run", "converged", "pair_updates")
+
+
+def dump_outputs(out_dir, res):
+    """Write the result dict of the timed leg (positions are n x ndim: 12.8 MB at cfg4) as float64 .npy files.
+    The MAE trace is NaN at iterations without a check (and past the last one run): only the checked entries are
+    written, with their iteration numbers."""
+    tr = np.asarray(res["trace_mae"])
+    checked = np.flatnonzero(~np.isnan(tr))
+    arrays = {"positions": res["positions"], "trace_iteration": checked, "trace_mae": tr[checked]}
+    arrays.update({k: np.array([res[k]]) for k in DUMP_SCALARS})
+    arrays = {name: np.asarray(a, dtype=np.float64) for name, a in arrays.items()}
+    bad = [name for name, a in arrays.items() if not np.all(np.isfinite(a))]
+    if bad:
+        raise SystemExit(f"--dump-outputs: non-finite values in {', '.join(bad)}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_reference(args, n, d, missing):
@@ -370,7 +396,13 @@ def main():
                          "(mapping_max_iter 1000, early stopping on) with 10 %% of the exact cells held out; prints held-out MAE, "
                          "iterations and wall time, and the same fit against the CPU reference loop at --oracle-n points")
     ap.add_argument("--oracle-n", type=int, default=4000, help="--converge: size of the CPU comparison (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the result they leave (best-iteration positions as "
+                         "topolow_shard_result / topolow_plan_result return them, MAE trace, controller scalars) as "
+                         "float64 DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.workload == "cfg5" or args.impl == "reference" or args.converge):
+        ap.error("--dump-outputs applies to the map throughput run (--impl ours, workloads cfg4 / cfg3 / small)")
     n, d, missing = WORKLOADS[args.workload]
     if args.workload == "cfg5":
         return main_cfg5(args, n, missing)
@@ -521,6 +553,7 @@ def main_map(args, n, d, missing):
             barrier()
             wall_ms = (time.perf_counter() - t0) * 1e3
         launches = m.info()["launches"] - launches_before
+        timed = m.result(trace=True) if args.dump_outputs else None   # before the probe iterations move the map on
         kt = m.time_kernels(probe_iters)                  # events around every launch (all ranks step together)
         res = m.result()
         info0["tensor_form_iterations"] = m.info().get("tensor_form_iterations", -1)   # read back by result(): of all iterations run
@@ -537,8 +570,11 @@ def main_map(args, n, d, missing):
             barrier()
             wall_ms = (time.perf_counter() - t0) * 1e3
         launches = plan.info()["launches"] - launches_before
-        res = plan.result()
+        res = timed = plan.result(trace=bool(args.dump_outputs))
         plan.close()
+    if args.dump_outputs and rank == 0:
+        assert timed["iterations_run"] == warm + args.steps, (timed["iterations_run"], warm, args.steps)
+        dump_outputs(args.dump_outputs, timed)
     ms_max, wall_max = max_over_ranks(ms, wall_ms)
     # one map: every unordered pair once per iteration whatever the rank count (strong scaling);
     # exact mode on several GPUs: `world` independent maps (weak scaling)

@@ -47,6 +47,7 @@ constexpr uint64_t kRowLayoutSeed = 0x726f77626c6f636bULL;
 constexpr int kStageJ = 128;   // partners per shared-memory stage
 constexpr int kStages = 3;
 constexpr int kFlagStride = 32;   // 32-bit words between the flag words of two ranks (128 bytes)
+constexpr int kWalkRegs = 112;    // register cap of spring_kernel (see there)
 constexpr unsigned long long kWaitNs = 20ull * 1000ull * 1000ull * 1000ull;
 
 struct RowDev {
@@ -218,7 +219,7 @@ TL_D bool last_cta(unsigned* counter) {
 // ---------------------------------------------------------------------------------------------------
 // repulsion: one work item = 256 own rows (R per thread) x one chunk of <= 2048 partners
 // ---------------------------------------------------------------------------------------------------
-// Items are handed out by an atomic counter (reset by the spring kernel's last CTA): the partial sums of an
+// Items are handed out by an atomic counter (reset by combine_kernel's last CTA): the partial sums of an
 // item do not depend on which CTA computed it, so the result is the same whatever the residency pattern.
 template <int H, int R, int U, int MAXR, bool kPow>
 __global__ void __maxnreg__(MAXR) repulse_kernel(RowDev dv, int cur, unsigned epoch) {
@@ -649,8 +650,11 @@ TL_D void walk_rows(const float* __restrict__ P, const uint2* __restrict__ rec /
 // ---------------------------------------------------------------------------------------------------
 // springs: one thread per own row, Gauss-Seidel along the row
 // ---------------------------------------------------------------------------------------------------
+// Launched with kBlockRows threads; a CTA walks row blocks blockIdx.x, + gridDim.x, ...  112 registers: 128 x 112 =
+// 14,336, what two CTAs of repulse_tc2_kernel (320 x 80) leave of the SM's 65,536, so one walk CTA per SM runs beside
+// them (launch_iteration; tests/test_resource_budget.py).
 template <int H, int kRing>
-__global__ void __launch_bounds__(kBlockRows) spring_kernel(RowDev dv, FitParams prm, int cur, unsigned epoch) {
+__global__ void __maxnreg__(kWalkRegs) spring_kernel(RowDev dv, FitParams prm, int cur, unsigned epoch) {
   constexpr int Dp = Row<H>::kStride;
   extern __shared__ float4 smem4[];
   asm volatile("griddepcontrol.launch_dependents;");   // a repulsion pass launched as programmatic dependent may start now
@@ -707,10 +711,11 @@ __global__ void __launch_bounds__(kBlockRows) spring_kernel(RowDev dv, FitParams
 // ---------------------------------------------------------------------------------------------------
 // combine: P'_i = (position after the springs) + (repulsion of the iteration), stored into every replica
 // ---------------------------------------------------------------------------------------------------
-// The spring walk (a long dependent chain per row: latency) and the repulsion pass (FMA throughput) both read
-// only the iteration's snapshot, so they run side by side (the repulsion pass is a programmatic dependent launch of
-// the walk: it starts as soon as the walk's CTAs are resident); this kernel, a normal launch, joins them.  The
-// repulsion sums of a row are added chunk by chunk in a fixed order (the result does not depend on the rank count).
+// The spring walk (a long dependent chain per row: latency) and the repulsion pass (issue and special-function
+// throughput) both read only the iteration's snapshot, so they run side by side (the walk is a programmatic dependent
+// launch of the pass: it starts as soon as the pass's CTAs are resident); this kernel, a normal launch after both,
+// waits for both grids and joins them.  The repulsion sums of a row are added chunk by chunk in a fixed order (the
+// result does not depend on the rank count).
 template <int H>
 __global__ void __launch_bounds__(kBlockRows) combine_kernel(RowDev dv, FitParams prm, int cur, unsigned epoch) {
   constexpr int Dp = Row<H>::kStride;
@@ -1019,14 +1024,14 @@ struct RowPlan {
   int64_t launches = 0;
   int64_t n_recs = 0, n_mrecs = 0;
   int64_t tensor_iters = -1;  // adaptive runs: iterations that ran the tensor form (read back by row_result; -1 = not adaptive / not read yet)
-  int rep_ctas = 0, rep_threads = 128;
+  int rep_ctas = 0;
   double near_limit = 0.0;    // adaptive runs: the tensor form while the probed near-pair fraction is at most this
   int rep_form = 0;           // shape of the repulsion pass in use (repulse_variant / configure_repulse)
   bool deep_ring = false;
   bool overlap = true;        // repulsion pass launched as programmatic dependent of the spring walk (TOPOLOW_OVERLAP=0: in order)
+  int walk_ctas = 0;          // grid of the spring walk under the repulsion pass
   int sm_count = 148;
   void* rep_fn = nullptr;
-  size_t rep_smem = 0;
   int f32_ctas = 0, f32_threads = 128;   // the FP32 difference form beside a tensor form (adaptive runs launch both)
   size_t f32_smem = 0;
   double total_ms = 0.0;
@@ -1178,14 +1183,22 @@ void launch_repulse_tc(RowPlan& rp, cudaStream_t s, int cur, bool dependent) {
 
 template <int H, int kRing> constexpr size_t kWalkSmem = (size_t)(kBlockRows / 32) * Ring<H, kRing>::kWarpBytes;
 
+// The overlap of launch_iteration: two CTAs of the two-GEMM pass and one walk CTA (either ring) share an SM's 233,472 bytes
+// of shared memory.  The system reserves 1 KiB per CTA; kWalkStaticSmem is the walk's static shared memory with that
+// reserve, as cuobjdump -res-usage reports it (tests/test_resource_budget.py checks it and the register caps).
+constexpr size_t kSmPerSm = 233472, kSmReserved = 1024, kWalkStaticSmem = 1152;
+static_assert(2 * (T2Smem::kTotal + kSmReserved) + kWalkSmem<8, 4> + kWalkStaticSmem <= kSmPerSm &&
+              2 * (T2Smem::kTotal + kSmReserved) + kWalkSmem<8, 8> + kWalkStaticSmem <= kSmPerSm,
+              "two repulse_tc2_kernel CTAs and a spring_kernel CTA no longer fit in one SM's shared memory");
+
 // the spring / MAE launches of one rank (deep ring when the rank owns few rows)
 template <int H>
-void launch_spring(const RowPlan& rp, cudaStream_t s, int cur, unsigned e_spring);
+void launch_spring(const RowPlan& rp, cudaStream_t s, int cur, unsigned e_spring, int ctas);
 template <int H>
 void launch_mae(const RowPlan& rp, cudaStream_t s, int nxt, unsigned e_spring, unsigned e_mae);
 
-// One iteration of one rank.  overlap: the repulsion pass starts while the spring walk is still running (ranks
-// with few rows: the walk is a latency chain on a few warps); otherwise the kernels run one after another.
+// One iteration of one rank.  overlap: the spring walk runs beside the repulsion pass; otherwise the kernels run one
+// after another.
 template <int H>
 void launch_iteration(RowPlan& rp, cudaStream_t s, cudaEvent_t* ev /* 7 events or null */, bool overlap) {
   RowDev& dv = rp.dv;
@@ -1200,18 +1213,20 @@ void launch_iteration(RowPlan& rp, cudaStream_t s, cudaEvent_t* ev /* 7 events o
   if (overlap) {
     // The walk first: its CTAs announce themselves at once (griddepcontrol.launch_dependents), which lets the
     // repulsion grid - launched as a programmatic dependent, it has no data dependence on the walk - fill the
-    // rest of the chip while the walk's few warps are already resident.  (Launched from two streams the
-    // repulsion grid usually won the race for the SMs and the walk ran after it.)
-    launch_spring<H>(rp, s, cur, e_prev);
+    // rest of the chip while the walk's warps are already resident.  Under the two-GEMM pass the walk is one CTA per
+    // SM (walk_ctas), each walking several row blocks: two pass CTAs fit beside it (static_assert above), and its warps,
+    // the older ones on the SM, keep their issue priority - launched after the pass, the walk's latency chain got a
+    // fraction of the issue slots and ended 0.8 ms after the pass (cfg4).  (Launched from two streams the repulsion grid
+    // usually won the race for the SMs and the walk ran after it.)
+    launch_spring<H>(rp, s, cur, e_prev, rp.walk_ctas);
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)rp.rep_ctas); cfg.blockDim = dim3((unsigned)rp.rep_threads);
-    cfg.dynamicSmemBytes = rp.rep_smem; cfg.stream = s;
+    cfg.gridDim = dim3((unsigned)rp.f32_ctas); cfg.blockDim = dim3((unsigned)rp.f32_threads);
+    cfg.dynamicSmemBytes = rp.f32_smem; cfg.stream = s;
     cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at; cfg.numAttrs = 1;
     if (!rp.tc_form || dv.adaptive) {
-      cfg.gridDim = dim3((unsigned)rp.f32_ctas); cfg.blockDim = dim3((unsigned)rp.f32_threads); cfg.dynamicSmemBytes = rp.f32_smem;
       TL_CUDA(cudaLaunchKernelEx(&cfg, (RepulseFn)rp.rep_fn, dv, cur, e_prev));
       rp.launches += dv.adaptive ? 1 : 0;
     }
@@ -1223,7 +1238,7 @@ void launch_iteration(RowPlan& rp, cudaStream_t s, cudaEvent_t* ev /* 7 events o
     }
     if (rp.tc_form) launch_repulse_tc<H>(rp, s, cur, false);
     if (ev) TL_CUDA(cudaEventRecord(ev[1], s));
-    launch_spring<H>(rp, s, cur, e_prev);
+    launch_spring<H>(rp, s, cur, e_prev, dv.rows / kBlockRows);
     if (ev) TL_CUDA(cudaEventRecord(ev[2], s));
   }
   const unsigned e_iter = ++rp.epoch;
@@ -1245,8 +1260,7 @@ void launch_iteration(RowPlan& rp, cudaStream_t s, cudaEvent_t* ev /* 7 events o
 }
 
 template <int H>
-void launch_spring(const RowPlan& rp, cudaStream_t s, int cur, unsigned e_spring) {
-  const int ctas = rp.dv.rows / kBlockRows;
+void launch_spring(const RowPlan& rp, cudaStream_t s, int cur, unsigned e_spring, int ctas) {
   if (rp.deep_ring) spring_kernel<H, 8><<<ctas, kBlockRows, kWalkSmem<H, 8>, s>>>(rp.dv, rp.prm, cur, e_spring);
   else spring_kernel<H, 4><<<ctas, kBlockRows, kWalkSmem<H, 4>, s>>>(rp.dv, rp.prm, cur, e_spring);
 }
@@ -1342,7 +1356,7 @@ void configure_repulse(RowPlan& rp, int sms) {
     if (const char* ec = std::getenv("TOPOLOW_TC_CPI")) rp.tc_cpi = std::max(1, std::atoi(ec));
     const long long items = (long long)(rp.dv.rows / kRowTile) * ((rp.dv.chunks + rp.tc_cpi - 1) / rp.tc_cpi);
     rp.rep_ctas = (int)std::min<long long>((long long)sms * per_sm, std::max<long long>(items, 1));
-    rp.rep_threads = kTcThreads; rp.rep_smem = TcSmem::kTotal; rp.rep_fn = nullptr;
+    rp.rep_fn = nullptr;
   }
   repulse_variant<H>(rp.tc_form ? 5 : variant, &fn, &threads, &rp.dot_form, &stage);
   const size_t smem = rp.dot_form ? (size_t)kStages * stage * Img<H>::kStride * sizeof(float) + (size_t)2 * H * threads * sizeof(float2)
@@ -1356,7 +1370,7 @@ void configure_repulse(RowPlan& rp, int sms) {
   rp.f32_ctas = (int)std::min<long long>((long long)sms * per_sm, std::max<long long>(items, 1));
   rp.f32_smem = smem; rp.f32_threads = threads;
   rp.rep_fn = (void*)fn;
-  if (!rp.tc_form) { rp.rep_ctas = rp.f32_ctas; rp.rep_smem = smem; rp.rep_threads = threads; }
+  if (!rp.tc_form) rp.rep_ctas = rp.f32_ctas;
   // The policy's tensor form is adaptive: the device picks the form of every iteration (image_tc_kernel's probe) and
   // the host launches both kernels.  A form asked for by name (TOPOLOW_REP_VARIANT) runs unconditionally.
   rp.dv.adaptive = (rp.tc_form && !ev) ? 1 : 0;
@@ -1375,6 +1389,7 @@ void configure_repulse(RowPlan& rp, int sms) {
   if (const char* eo = std::getenv("TOPOLOW_OVERLAP")) rp.overlap = std::atoi(eo) != 0;
   // spring / MAE walk: the deep ring needs more than the default 48 KB of dynamic shared memory
   rp.deep_ring = rp.dv.rows / kBlockRows <= 2 * sms;
+  rp.walk_ctas = rp.tc2_form ? std::min(rp.dv.rows / kBlockRows, sms) : rp.dv.rows / kBlockRows;
   if (const char* er = std::getenv("TOPOLOW_DEEP_RING")) rp.deep_ring = std::atoi(er) != 0;
   TL_CUDA(cudaFuncSetAttribute(spring_kernel<H, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWalkSmem<H, 8>));
   TL_CUDA(cudaFuncSetAttribute(mae_kernel<H, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWalkSmem<H, 8>));
@@ -1605,7 +1620,7 @@ double row_run_local(RowPlan* const* plans, int n, int n_iters) {
             rp.launches += rp.dv.adaptive ? 1 : 0;
           }
           if (rp.tc_form) launch_repulse_tc<H>(rp, s, cur, false);
-          launch_spring<H>(rp, s, cur, e_prev);
+          launch_spring<H>(rp, s, cur, e_prev, rp.dv.rows / kBlockRows);
           combine_kernel<H><<<rp.dv.rows / kBlockRows, kBlockRows, 0, s>>>(rp.dv, rp.prm, cur, ++rp.epoch);
         });
         rp.launches += 3; rp.iter_launched = t + 1;

@@ -34,10 +34,13 @@ constexpr int kT2Threads = 320;       // 8 consumer warps + the MMA warp + the c
 constexpr float kT2SeriesS = 0.005f;   // series form of the weight: pairs closer than 0.1 (d^2 / 2 < 0.005) are near pairs
 constexpr bool kT2LoPass = false;     // second pass of GEMM 2 over the TF32 remainders of the partner coordinates (see below)
 
+// The only A operand GEMM 1 reads from shared memory is the remainders of tile 1 (tile 0's and both tiles' -A_hi and norm
+// columns are in tensor memory): 4 planes x 128 rows x 16 B.  At 61.6 KB per CTA two CTAs leave room on the SM for a
+// CTA of the spring walk (rowblock.cu, launch_iteration).
 struct T2Smem {
-  static constexpr int kAHi = 0;                                   // 6 planes x 256 rows x 16 B
-  static constexpr int kALo = kAHi + 6 * kTcRows * 16;             // 4 planes
-  static constexpr int kStage0 = kALo + 4 * kTcRows * 16;
+  static constexpr int kALo1 = 0;                                  // 4 planes x 128 rows x 16 B
+  static constexpr int kATx = 4 * 128 * 16;                        // bytes landing per item
+  static constexpr int kStage0 = kALo1 + kATx;
   static constexpr int kBHi = 0;                                   // 6 planes x 32 x 16 B   (GEMM 1, K-major over coordinates)
   static constexpr int kBLo = 6 * kT2SJ * 16;                      // 4 planes
   static constexpr int kYHi = kBLo + 4 * kT2SJ * 16;               // 8 partner-quads x 32 rows x 16 B (GEMM 2, K-major over partners)
@@ -117,7 +120,6 @@ __global__ void __maxnreg__(80) repulse_tc2_kernel(RowDev dv, T2Image im, int cu
   const unsigned bar_a_free = sm0 + T2Smem::kBars + 8u * (1 + 2 * kT2Stages + 8);
   unsigned* tmem_ptr_s = reinterpret_cast<unsigned*>(tc_smem + T2Smem::kTmemPtr);
 
-  for (int x = tid; x < kTcRows * 4; x += kT2Threads) reinterpret_cast<float*>(tc_smem + T2Smem::kAHi + 5 * kTcRows * 16)[x] = 0.f;
   for (int s = 0; s < kT2Stages; ++s)
     for (int x = tid; x < kT2SJ * 4; x += kT2Threads)
       reinterpret_cast<float*>(tc_smem + T2Smem::kStage0 + s * T2Smem::kStageBytes + T2Smem::kBHi + 5 * kT2SJ * 16)[x] = 0.f;
@@ -148,7 +150,7 @@ __global__ void __maxnreg__(80) repulse_tc2_kernel(RowDev dv, T2Image im, int cu
   auto chunk_stages = [&](int c) { return (min(kChunk, dv.n - c * kChunk) + kT2SJ - 1) / kT2SJ; };
 
   // Work items are handed out by an atomic counter (the sums of an item do not depend on who computes it): CTAs that start
-  // late - the SMs the spring walk still occupies when the pass is launched under it - simply take fewer.  The copy warp
+  // late or share their SM with a CTA of the spring walk (it runs under the pass) simply take fewer.  The copy warp
   // draws the CTA's next item and publishes it in a two-entry ring in shared memory (bar_item, one phase per item); it
   // publishes item k + 1 only after the consumers have started item k (bar_a_tmem), so no waiter can miss a phase.
   volatile int* item_ring = reinterpret_cast<volatile int*>(tc_smem + T2Smem::kTmemPtr) + 2;
@@ -202,12 +204,9 @@ __global__ void __maxnreg__(80) repulse_tc2_kernel(RowDev dv, T2Image im, int cu
         if (item_g > 0) mbar_wait(bar_a_free, (item_g - 1) & 1);
         ++item_g;
         if (elect_one()) {
-          mbar_expect_tx(bar_a_full, TcSmem::kATx);
-          for (int c = 0; c < 4; ++c) {
-            bulk_g2s(sm0 + T2Smem::kAHi + c * kTcRows * 16, im.a.xhi + ((size_t)c * dv.cap_rows + ld.r0) * 4, kTcRows * 16, bar_a_full);
-            bulk_g2s(sm0 + T2Smem::kALo + c * kTcRows * 16, im.a.xlo + ((size_t)c * dv.cap_rows + ld.r0) * 4, kTcRows * 16, bar_a_full);
-          }
-          bulk_g2s(sm0 + T2Smem::kAHi + 4 * kTcRows * 16, im.a.aug_a + ld.r0 * 4, kTcRows * 16, bar_a_full);
+          mbar_expect_tx(bar_a_full, T2Smem::kATx);
+          for (int c = 0; c < 4; ++c)      // the remainders of tile 1 (rows 128..255 of the item)
+            bulk_g2s(sm0 + T2Smem::kALo1 + c * 128 * 16, im.a.xlo + ((size_t)c * dv.cap_rows + ld.r0 + 128) * 4, 128 * 16, bar_a_full);
         }
         __syncwarp();
       }
@@ -252,9 +251,9 @@ __global__ void __maxnreg__(80) repulse_tc2_kernel(RowDev dv, T2Image im, int cu
 #pragma unroll
         for (int m = 0; m < 2; ++m) {
           const unsigned d = tmem0 + col_s(b, m);
-          const unsigned a_t = tmem0 + col_a(m), a_lo = sm0 + T2Smem::kALo + m * 128 * 16;
+          const unsigned a_t = tmem0 + col_a(m), a_lo = sm0 + T2Smem::kALo1;
           const unsigned b_hi = stg + T2Smem::kBHi, b_lo = stg + T2Smem::kBLo;
-          constexpr unsigned kLboA = kTcRows * 16, kLboB = kT2SJ * 16;
+          constexpr unsigned kLboA = 128 * 16, kLboB = kT2SJ * 16;
 #pragma unroll
           for (int k = 0; k < 3; ++k)      // (-A_hi) B_hi^T, A from tensor memory (stored negated: no negate flag)
             tc_mma_tf32_ts(d, a_t + k * 8, tc_desc(b_hi + k * 2 * kLboB, kLboB, 128), kT2Idesc1T, k > 0);

@@ -58,12 +58,14 @@ enum {
 /* mode */
 enum {
   TOPOLOW_MODE_COLOURED = 0, /* production: hierarchical tournament of matchings (every pair once
-                                per iteration, updates within a matching commute) */
+                                per iteration, updates within a matching commute); ndim 1..16 */
   TOPOLOW_MODE_REPLAY = 1,   /* FP64, consumes a given / seeded std::mt19937 pair permutation and
-                                executes it by dependency levels: exactly the sequential loop */
+                                executes it by dependency levels: exactly the sequential loop; any ndim */
   TOPOLOW_MODE_ROWBLOCK = 2  /* relaxed, for large maps: every point's update is computed by the owner of its row
                                 against a replica of all positions (Gauss-Seidel along a row, Jacobi across
-                                rows); FP32; the scheme topolow_shard_* spreads over several GPUs */
+                                rows); FP32; the scheme topolow_shard_* spreads over several GPUs.  ndim 1..32:
+                                1..16 with the tensor-core repulsion pass, 17..32 with the FP32 difference form
+                                only (TOPOLOW_ERR_BAD_ARG beyond 32 and for another form asked for by name) */
 };
 /* precision (coloured mode) */
 enum {

@@ -268,7 +268,7 @@ std::shared_ptr<EdgeStore> make_store(const topolow_problem& pb, int T, int P, i
 std::unique_ptr<topolow_plan> make_plan(const topolow_problem& pb, const topolow_params& pr,
                                         std::shared_ptr<EdgeStore> shared, int* shared_flag) {
   validate(pb, pr);
-  if (pb.ndim > kMaxDim) throw BadArg("ndim > 16 is not built into libtopolow_b200 (coloured mode)");
+  if (pb.ndim > kMaxDim) throw BadArg("ndim > 16 is not built into libtopolow_b200 (coloured mode); the row-block mode takes ndim <= 32, the replay mode any ndim");
   if (pb.n > 1000000) throw BadArg("n > 1,000,000 is not supported (bucket table is T x T)");
   if (pr.n_shards < 0 || pr.n_shards > 64) throw BadArg("n_shards must be in 0..64");
   auto pl = std::make_unique<topolow_plan>();

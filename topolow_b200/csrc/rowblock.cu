@@ -48,6 +48,8 @@ constexpr int kStageJ = 128;   // partners per shared-memory stage
 constexpr int kStages = 3;
 constexpr int kFlagStride = 32;   // 32-bit words between the flag words of two ranks (128 bytes)
 constexpr int kWalkRegs = 112;    // register cap of spring_kernel (see there)
+constexpr int kWalkRegsWide = 168;   // ... for ndim 17..32 (H > 8), which never runs beside the two-GEMM pass
+constexpr int kRepUnrollWide = 1, kRepRegsWide = 128;   // repulse_kernel for ndim 17..32: partner unroll, register cap
 constexpr unsigned long long kWaitNs = 20ull * 1000ull * 1000ull * 1000ull;
 
 struct RowDev {
@@ -526,16 +528,18 @@ struct Ring {
   static constexpr int kRecRing = 2 * kRing;
   static constexpr int Dp = Row<H>::kStride;
   static constexpr int NC = Dp / 4;                         // 16-byte pieces of a row
-  static constexpr int kRowBytes = NC * 16;
+  static constexpr int kRowBytes = NC > 4 ? 128 : NC * 16;  // rows of 5..8 pieces (ndim 17..32) take 128 bytes
   static constexpr int kSlotBytes = 32 * kRowBytes;
   static constexpr int kWarpBytes = kRing * kSlotBytes + kRecRing * 32 * 8;
   // piece c of the row staged for `lane`.  Rows are stored lane-transposed ((lane & 3) * 8 + lane / 4): the 32
   // copies of one gather instruction (fixed quad member u, all quads, all pieces) then fill one contiguous
   // 8-row block - no bank conflict on the write side (the natural order gave 8-way conflicts: the L1 data pipe
   // was the limiter of the walk) - and 64-byte rows rotate their pieces by lane & 3 so that the eight lanes of a
-  // 128-bit read phase hit eight different bank groups.
+  // 128-bit read phase hit eight different bank groups.  128-byte rows rotate by lane & 7 for the same reason; on the
+  // write side the two quads of a phase (lane & 7 = 4 (quad & 1) + u) then cover pieces c ^ u and c ^ u ^ 4: again eight groups.
   static TL_D int piece(int lane, int c) {
     const int row = (lane & 3) * 8 + (lane >> 2);
+    if constexpr (NC > 4) return row * 128 + ((c ^ (lane & 7)) << 4);
     return NC == 4 ? row * 64 + ((c ^ (lane & 3)) << 4) : row * kRowBytes + (c << 4);
   }
 };
@@ -600,6 +604,12 @@ TL_D void walk_rows(const float* __restrict__ P, const uint2* __restrict__ rec /
         const unsigned j[4] = {ja.x & kSlotMask, ja.z & kSlotMask, jb.x & kSlotMask, jb.z & kSlotMask};
 #pragma unroll
         for (int u = 0; u < 4; ++u) cp_async16_ca(g_slot_a + dst_off[u], P_c + (size_t)j[u] * (R::Dp * 4));
+        if constexpr (R::NC > 4) {                  // rows of more than four pieces: this lane also fetches piece c + 4
+          if (c + 4 < R::NC) {                      // piece(l, c + 4) = piece(l, c) ^ 64 (c < 4: (c + 4) ^ f = (c ^ f) ^ 4)
+#pragma unroll
+            for (int u = 0; u < 4; ++u) cp_async16_ca(g_slot_a + (dst_off[u] ^ 64u), P_c + (size_t)j[u] * (R::Dp * 4) + 64);
+          }
+        }
       }
       --g_left;
     }
@@ -622,7 +632,11 @@ TL_D void walk_rows(const float* __restrict__ P, const uint2* __restrict__ rec /
     // ---- everything this step reads from shared memory ----
     uint4 qv[R::NC];
 #pragma unroll
-    for (int k = 0; k < H / 2; ++k) qv[k] = lds128(slot_a + own_off[k]);
+    for (int k = 0; k < H / 2; ++k) {
+      // 128-byte rows: piece(lane, k) = piece(lane, 0) ^ (k << 4); one register instead of eight
+      if constexpr (R::NC > 4) qv[k] = lds128(slot_a + (own_off[0] ^ ((unsigned)k << 4)));
+      else qv[k] = lds128(slot_a + own_off[k]);
+    }
     uint2 qt = make_uint2(0u, 0u);
     if constexpr (H % 2 == 1) qt = lds64(slot_a + own_off[H / 2]);
     const uint2 r = lds64(rslot_a + rec_own);
@@ -654,7 +668,7 @@ TL_D void walk_rows(const float* __restrict__ P, const uint2* __restrict__ rec /
 // 14,336, what two CTAs of repulse_tc2_kernel (320 x 80) leave of the SM's 65,536, so one walk CTA per SM runs beside
 // them (launch_iteration; tests/test_resource_budget.py).
 template <int H, int kRing>
-__global__ void __maxnreg__(kWalkRegs) spring_kernel(RowDev dv, FitParams prm, int cur, unsigned epoch) {
+__global__ void __maxnreg__(H <= 8 ? kWalkRegs : kWalkRegsWide) spring_kernel(RowDev dv, FitParams prm, int cur, unsigned epoch) {
   constexpr int Dp = Row<H>::kStride;
   extern __shared__ float4 smem4[];
   asm volatile("griddepcontrol.launch_dependents;");   // a repulsion pass launched as programmatic dependent may start now
@@ -696,8 +710,20 @@ __global__ void __maxnreg__(kWalkRegs) spring_kernel(RowDev dv, FitParams prm, i
     const float f = spring ? two_k_rnorm * (target - dist) * rcp_approx(dist + 0.01f) : 0.f;
     // x += -delta f + d0 w0  <=>  (-x) += delta f - d0 w0; the take-back term does not wait for f
     const float2 ff = make_float2(f, f), nw = make_float2(-w0, -w0);
+    if constexpr (H <= 8) {
 #pragma unroll
-    for (int kk = 0; kk < H; ++kk) xn[kk] = __ffma2_rn(dl[kk], ff, __ffma2_rn(d0[kk], nw, xn[kk]));
+      for (int kk = 0; kk < H; ++kk) xn[kk] = __ffma2_rn(dl[kk], ff, __ffma2_rn(d0[kk], nw, xn[kk]));
+    } else {
+      // ndim 17..32: both delta arrays held across the weights do not fit beside the rows (spills); they are recomputed
+      // from q, the same roundings.  q is passed through an empty asm so that the compiler cannot merge the two sums
+      // back into the ones of dist2 and keep dl / d0 alive after all.
+      float2 qr[H];
+#pragma unroll
+      for (int kk = 0; kk < H; ++kk) { qr[kk] = q[kk]; asm volatile("" : "+f"(qr[kk].x), "+f"(qr[kk].y)); }
+#pragma unroll
+      for (int kk = 0; kk < H; ++kk)
+        xn[kk] = __ffma2_rn(__fadd2_rn(qr[kk], xn[kk]), ff, __ffma2_rn(__fadd2_rn(qr[kk], p0n[kk]), nw, xn[kk]));
+    }
   });
   if (dp1 > 0.f) {
     float2 x[H];
@@ -977,9 +1003,18 @@ void dispatch_h(int H, F&& f) {
     case 6: f(std::integral_constant<int, 6>()); break;
     case 7: f(std::integral_constant<int, 7>()); break;
     case 8: f(std::integral_constant<int, 8>()); break;
-    default: throw BadArg("row-block mode supports ndim <= 16");
+    case 10: f(std::integral_constant<int, 10>()); break;
+    case 12: f(std::integral_constant<int, 12>()); break;
+    case 14: f(std::integral_constant<int, 14>()); break;
+    case 16: f(std::integral_constant<int, 16>()); break;
+    default: throw BadArg("row-block mode supports ndim <= 32 (the replay mode takes any ndim)");
   }
 }
+
+// Packed coordinate pairs a row is computed on.  ndim 17..32 runs on the whole padded row (Row<H>::kStride = 2 H): the
+// pad columns are zero, their deltas and updates stay +-0 and add +0 to every sum, so the real coordinates come out as
+// without the pad, and four instantiations cover sixteen ndims.
+int row_h(int ndim) { return ndim <= 16 ? (ndim + 1) / 2 : (ndim + 3) / 4 * 2; }
 
 }  // namespace
 
@@ -1157,6 +1192,7 @@ T2Image t2_image(const RowPlan& rp) {
 }
 template <int H>
 void launch_image_tc(RowPlan& rp, cudaStream_t s, int cur, unsigned e_prev) {
+  static_assert(H <= 8, "the tensor forms take ndim <= 16");
   image_tc_kernel<H><<<(unsigned)(rp.dv.cap_rows / kBlockRows), kBlockRows, 0, s>>>(rp.dv, tc_image(rp), cur, e_prev);
   rp.launches += 1;
   if (rp.tc2_form) {
@@ -1166,6 +1202,7 @@ void launch_image_tc(RowPlan& rp, cudaStream_t s, int cur, unsigned e_prev) {
 }
 template <int H>
 void launch_repulse_tc(RowPlan& rp, cudaStream_t s, int cur, bool dependent) {
+  static_assert(H <= 8, "the tensor forms take ndim <= 16");
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)rp.rep_ctas); cfg.blockDim = dim3(kTcThreads);
   cfg.dynamicSmemBytes = TcSmem::kTotal; cfg.stream = s;
@@ -1208,8 +1245,10 @@ void launch_iteration(RowPlan& rp, cudaStream_t s, cudaEvent_t* ev /* 7 events o
   const unsigned e_prev = rp.epoch;          // the epoch every rank reached when iteration t - 1 (and its check) ended
   const int row_ctas = dv.rows / kBlockRows;
   if (ev) TL_CUDA(cudaEventRecord(ev[0], s));
-  if (rp.dot_form) { image_kernel<H><<<dv.slots / kBlockRows, kBlockRows, 0, s>>>(dv, cur, e_prev); rp.launches += 1; }
-  if (rp.tc_form) launch_image_tc<H>(rp, s, cur, e_prev);
+  if constexpr (H <= 8) {                    // the inner-product and tensor forms exist for ndim <= 16 only
+    if (rp.dot_form) { image_kernel<H><<<dv.slots / kBlockRows, kBlockRows, 0, s>>>(dv, cur, e_prev); rp.launches += 1; }
+    if (rp.tc_form) launch_image_tc<H>(rp, s, cur, e_prev);
+  }
   if (overlap) {
     // The walk first: its CTAs announce themselves at once (griddepcontrol.launch_dependents), which lets the
     // repulsion grid - launched as a programmatic dependent, it has no data dependence on the walk - fill the
@@ -1230,13 +1269,13 @@ void launch_iteration(RowPlan& rp, cudaStream_t s, cudaEvent_t* ev /* 7 events o
       TL_CUDA(cudaLaunchKernelEx(&cfg, (RepulseFn)rp.rep_fn, dv, cur, e_prev));
       rp.launches += dv.adaptive ? 1 : 0;
     }
-    if (rp.tc_form) launch_repulse_tc<H>(rp, s, cur, true);
+    if constexpr (H <= 8) { if (rp.tc_form) launch_repulse_tc<H>(rp, s, cur, true); }
   } else {
     if (!rp.tc_form || dv.adaptive) {
       ((RepulseFn)rp.rep_fn)<<<rp.f32_ctas, rp.f32_threads, rp.f32_smem, s>>>(dv, cur, e_prev);
       rp.launches += dv.adaptive ? 1 : 0;
     }
-    if (rp.tc_form) launch_repulse_tc<H>(rp, s, cur, false);
+    if constexpr (H <= 8) { if (rp.tc_form) launch_repulse_tc<H>(rp, s, cur, false); }
     if (ev) TL_CUDA(cudaEventRecord(ev[1], s));
     launch_spring<H>(rp, s, cur, e_prev, dv.rows / kBlockRows);
     if (ev) TL_CUDA(cudaEventRecord(ev[2], s));
@@ -1272,7 +1311,7 @@ void launch_mae(const RowPlan& rp, cudaStream_t s, int nxt, unsigned e_spring, u
 }
 
 void launch_one(RowPlan& rp, cudaStream_t s, cudaEvent_t* ev = nullptr) {
-  dispatch_h((rp.dv.D + 1) / 2, [&](auto h) { launch_iteration<decltype(h)::value>(rp, s, ev, rp.overlap && !ev); });
+  dispatch_h(row_h(rp.dv.D), [&](auto h) { launch_iteration<decltype(h)::value>(rp, s, ev, rp.overlap && !ev); });
 }
 
 // Shapes of the repulsion kernel: {rows per thread, partner unroll, register cap, cube on the SFU}.
@@ -1295,16 +1334,23 @@ void repulse_variant(int v, RepulseFn* fn, int* threads, bool* dot, int* stage) 
   *dot = false;
   *stage = kStageJ;
   *threads = kRowTile / 2;
-  switch (v) {
-    case 1: *fn = repulse_kernel<H, 2, 2, 128, false>; break;
-    case 2: *fn = repulse_kernel<H, 2, 2, 120, false>; break;
-    case 3: *fn = repulse_kernel<H, 2, 2, 120, true>; break;
-    case 4: *fn = repulse_dot_kernel<H, 2, 2, 128>; *dot = true; break;
-    case 6: *fn = repulse_dot_kernel<H, 2, 1, 128>; *dot = true; break;
-    case 7: *fn = repulse_dot_kernel<H, 2, 2, 168>; *dot = true; break;
-    case 8: *fn = repulse_dot_kernel<H, 2, 1, 128, kStageJ, true>; *dot = true; break;
-    case 9: *fn = repulse_dot_kernel<H, 2, 2, 128, kStageJ, true>; *dot = true; break;
-    default: *fn = repulse_kernel<H, 2, 2, 128, true>; break;
+  if constexpr (H > 8) {
+    // ndim 17..32: the difference form only, one row per thread (two rows and their accumulators alone are 4 H float2)
+    (void)v;
+    *fn = repulse_kernel<H, 1, kRepUnrollWide, kRepRegsWide, true>;
+    *threads = kRowTile;
+  } else {
+    switch (v) {
+      case 1: *fn = repulse_kernel<H, 2, 2, 128, false>; break;
+      case 2: *fn = repulse_kernel<H, 2, 2, 120, false>; break;
+      case 3: *fn = repulse_kernel<H, 2, 2, 120, true>; break;
+      case 4: *fn = repulse_dot_kernel<H, 2, 2, 128>; *dot = true; break;
+      case 6: *fn = repulse_dot_kernel<H, 2, 1, 128>; *dot = true; break;
+      case 7: *fn = repulse_dot_kernel<H, 2, 2, 168>; *dot = true; break;
+      case 8: *fn = repulse_dot_kernel<H, 2, 1, 128, kStageJ, true>; *dot = true; break;
+      case 9: *fn = repulse_dot_kernel<H, 2, 2, 128, kStageJ, true>; *dot = true; break;
+      default: *fn = repulse_kernel<H, 2, 2, 128, true>; break;
+    }
   }
 }
 template <int H>
@@ -1316,9 +1362,16 @@ void configure_repulse(RowPlan& rp, int sms) {
   // policy, measured on B200 (ms per repulsion pass, forms 11 / 10 / 5): ndim 16, 100k: 7.5 / 13.4 / 16.8; ndim 12, 40k: 1.24 / 1.82 /
   // 2.32; ndim 10, 10k: 0.16 / 0.19 / 0.23; ndim 6, 30k: 0.69 / 0.84 / 0.75.  The two-GEMM form costs the same at every ndim (K is
   // padded to 16 coordinates); the difference form's cost falls with ndim and takes over below ndim 5.
-  if (variant == 0) variant = H >= 3 ? 11 : 5;
+  if constexpr (H > 8) {
+    // ndim 17..32: the tensor forms pad K to 16 coordinates and the inner-product forms hold 2 rows per thread; only the
+    // difference form is built, and a form asked for by name that is not it is an error, not a silent substitute
+    if (variant != 0 && variant != 5) throw BadArg("ndim > 16 runs only the FP32 difference form (TOPOLOW_REP_VARIANT=5) in row-block mode");
+    variant = 5;
+  } else if (variant == 0) {
+    variant = H >= 3 ? 11 : 5;
+  }
   rp.rep_form = variant;
-  if (variant == 10 || variant == 11) {          // distances (10) / distances and accumulation (11) on the tensor cores
+  if constexpr (H <= 8) if (variant == 10 || variant == 11) {          // distances (10) / distances and accumulation (11) on the tensor cores
     rp.tc_form = true;
     rp.tc2_form = variant == 11;
     rp.dv.rparts = (rp.tc2_form ? 3 : 2) * rp.dv.chunks;
@@ -1361,7 +1414,10 @@ void configure_repulse(RowPlan& rp, int sms) {
   repulse_variant<H>(rp.tc_form ? 5 : variant, &fn, &threads, &rp.dot_form, &stage);
   const size_t smem = rp.dot_form ? (size_t)kStages * stage * Img<H>::kStride * sizeof(float) + (size_t)2 * H * threads * sizeof(float2)
                                   : (size_t)kStages * kStageJ * Row<H>::kStride * sizeof(float);
-  if (smem > 48 * 1024) TL_CUDA(cudaFuncSetAttribute((const void*)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  cudaFuncAttributes fa;
+  TL_CUDA(cudaFuncGetAttributes(&fa, (const void*)fn));
+  // the static shared memory counts against the same 48 KB default (ndim 32: 48 KB of stages + item_s)
+  if (smem + fa.sharedSizeBytes > 48 * 1024) TL_CUDA(cudaFuncSetAttribute((const void*)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int per_sm = 0;
   TL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, threads, smem));
   if (per_sm < 1) per_sm = 1;
@@ -1393,6 +1449,10 @@ void configure_repulse(RowPlan& rp, int sms) {
   if (const char* er = std::getenv("TOPOLOW_DEEP_RING")) rp.deep_ring = std::atoi(er) != 0;
   TL_CUDA(cudaFuncSetAttribute(spring_kernel<H, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWalkSmem<H, 8>));
   TL_CUDA(cudaFuncSetAttribute(mae_kernel<H, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWalkSmem<H, 8>));
+  if constexpr (kWalkSmem<H, 4> > 48 * 1024) {   // 128-byte ring rows (ndim 17..32): the 4-deep ring needs it too
+    TL_CUDA(cudaFuncSetAttribute(spring_kernel<H, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWalkSmem<H, 4>));
+    TL_CUDA(cudaFuncSetAttribute(mae_kernel<H, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWalkSmem<H, 4>));
+  }
 }
 
 }  // namespace
@@ -1400,7 +1460,7 @@ void configure_repulse(RowPlan& rp, int sms) {
 RowPlan* row_create(const topolow_problem& pb, const topolow_params& pr, int rank, int n_ranks) {
   validate(pb, pr);
   if (n_ranks < 1 || n_ranks > kMaxShards || rank < 0 || rank >= n_ranks) throw BadArg("rank / n_ranks out of range");
-  if (pb.ndim > 16) throw BadArg("row-block mode supports ndim <= 16");
+  if (pb.ndim > 32) throw BadArg("row-block mode supports ndim <= 32 (the replay mode takes any ndim)");
   if (pb.n >= (1ll << 30)) throw BadArg("n out of range");
   TL_CUDA(cudaSetDevice(pr.device));
   keep_pool_memory(pr.device);
@@ -1454,7 +1514,7 @@ RowPlan* row_create(const topolow_problem& pb, const topolow_params& pr, int ran
     }
     pool_alloc(rp->best, hp.size() * sizeof(float));
     pool_alloc(rp->dp1, hd.size() * sizeof(float));
-    pool_alloc(rp->rpart, (size_t)3 * dv.chunks * std::max(dv.rows, 1) * dv.Dp * sizeof(float));
+    pool_alloc(rp->rpart, (size_t)(pb.ndim <= 16 ? 3 : 1) * dv.chunks * std::max(dv.rows, 1) * dv.Dp * sizeof(float));   // 3: the two-GEMM form
     pool_alloc(rp->tc_buf, dv.cap_rows * (size_t)(16 + 16 + 4 + 4 + 16 + 32 + 16) * sizeof(float));
     pool_alloc(rp->xs, (size_t)std::max(dv.rows, 1) * dv.Dp * sizeof(float));
     pool_alloc(rp->img, dv.cap_rows * (size_t)(((dv.D + 1) / 2 * 2 + 2 + 3) / 4 * 4) * sizeof(float));   // Img<H>::kStride floats per row
@@ -1474,7 +1534,7 @@ RowPlan* row_create(const topolow_problem& pb, const topolow_params& pr, int ran
     // every rank, fixed for the fit; the map stays about where it starts, and a map that wanders only makes more
     // pairs take the difference form)
     for (int d = 0; d < 16; ++d) dv.centre[d] = 0.f;
-    for (int d = 0; d < pb.ndim; ++d) {
+    for (int d = 0; d < std::min(pb.ndim, 16); ++d) {   // ndim > 16 runs the difference form, which has no centre
       double sum = 0.0;
       for (int64_t i = 0; i < pb.n; ++i) sum += pb.initial_positions[(size_t)d * pb.n + i];
       const double c = sum / (double)pb.n;
@@ -1502,7 +1562,7 @@ RowPlan* row_create(const topolow_problem& pb, const topolow_params& pr, int ran
     rp->hold_truth.assign(pb.holdout_truth, pb.holdout_truth + pb.n_holdout);
   }
   pt.mark("rows: records + hold-out");
-  if (dv.rows > 0) dispatch_h((dv.D + 1) / 2, [&](auto h) { configure_repulse<decltype(h)::value>(*rp, sm_count); });
+  if (dv.rows > 0) dispatch_h(row_h(dv.D), [&](auto h) { configure_repulse<decltype(h)::value>(*rp, sm_count); });
   pt.mark("rows: kernel attributes");
   TL_CUDA(cudaDeviceSynchronize());
   pt.mark("rows: device synchronize");
@@ -1610,16 +1670,18 @@ double row_run_local(RowPlan* const* plans, int n, int n_iters) {
       const bool check = is_check_iter(t, p0.prm), fin = ((t + 1) % 10 == 0);
       for (int a = 0; a < n; ++a) {
         RowPlan& rp = *plans[a];
-        dispatch_h((rp.dv.D + 1) / 2, [&](auto h) {
+        dispatch_h(row_h(rp.dv.D), [&](auto h) {
           constexpr int H = decltype(h)::value;
           const unsigned e_prev = rp.epoch;
-          if (rp.dot_form) { image_kernel<H><<<rp.dv.slots / kBlockRows, kBlockRows, 0, s>>>(rp.dv, cur, e_prev); rp.launches += 1; }
-          if (rp.tc_form) launch_image_tc<H>(rp, s, cur, e_prev);
+          if constexpr (H <= 8) {
+            if (rp.dot_form) { image_kernel<H><<<rp.dv.slots / kBlockRows, kBlockRows, 0, s>>>(rp.dv, cur, e_prev); rp.launches += 1; }
+            if (rp.tc_form) launch_image_tc<H>(rp, s, cur, e_prev);
+          }
           if (!rp.tc_form || rp.dv.adaptive) {
             ((RepulseFn)rp.rep_fn)<<<rp.f32_ctas, rp.f32_threads, rp.f32_smem, s>>>(rp.dv, cur, e_prev);
             rp.launches += rp.dv.adaptive ? 1 : 0;
           }
-          if (rp.tc_form) launch_repulse_tc<H>(rp, s, cur, false);
+          if constexpr (H <= 8) { if (rp.tc_form) launch_repulse_tc<H>(rp, s, cur, false); }
           launch_spring<H>(rp, s, cur, e_prev, rp.dv.rows / kBlockRows);
           combine_kernel<H><<<rp.dv.rows / kBlockRows, kBlockRows, 0, s>>>(rp.dv, rp.prm, cur, ++rp.epoch);
         });
@@ -1628,7 +1690,7 @@ double row_run_local(RowPlan* const* plans, int n, int n_iters) {
       if (check || fin) {
         for (int a = 0; a < n; ++a) {
           RowPlan& rp = *plans[a];
-          dispatch_h((rp.dv.D + 1) / 2, [&](auto h) {
+          dispatch_h(row_h(rp.dv.D), [&](auto h) {
             constexpr int H = decltype(h)::value;
             const unsigned e_iter = rp.epoch;
             launch_mae<H>(rp, s, nxt, e_iter, ++rp.epoch);

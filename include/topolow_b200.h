@@ -18,6 +18,7 @@
  *       fits: parallel::mclapply over parameter samples / folds
  *       (R/adaptive_sampling.R:645-672, :1301-1320, :2670-2693).  One call, many
  *       fits, per-job status instead of exceptions (:2657-2666).
+ *       topolow_fit_batch_interruptible() is the same call with a user-interrupt callback.
  *   topolow_plan_*()                  device-resident form of one fit for callers
  *       that keep inputs in HBM and step the loop themselves (bench, sharded map).
  *   topolow_est_distances()           as.matrix(stats::dist(positions)), R/core.R:474.
@@ -135,7 +136,8 @@ typedef struct {
   char message[256];
 } topolow_result;
 
-/* Polled between device chunks (R_CheckUserInterrupt equivalent); non-zero aborts. */
+/* R_CheckUserInterrupt equivalent; non-zero aborts.  Polled between device chunks by topolow_fit_interruptible,
+ * while the fits run by topolow_fit_batch_interruptible. */
 typedef int (*topolow_interrupt_fn)(void* user);
 
 /* ---- single fit ------------------------------------------------------- */
@@ -163,9 +165,28 @@ TOPOLOW_API int topolow_optimize_layout_exact(
  * With 16 or more jobs every fit runs on one CTA (64-point tiles unless tile_points is set) and the fits
  * are launched many per kernel.  Jobs whose edge_i / edge_j / edge_dist / edge_thresh POINTERS (and n,
  * n_edges) are equal share one set of device records: hand the parameter samples of a CV grid the same
- * arrays per fold.  A batch is not interruptible. */
+ * arrays per fold.  topolow_fit_batch is topolow_fit_batch_interruptible with poll = NULL. */
 TOPOLOW_API int topolow_fit_batch(int32_t n_jobs, const topolow_problem* problems, const topolow_params* params,
                       topolow_result* results, int32_t device);
+
+/* The same batch, stoppable.  `poll` is called from the calling thread only: once before set-up, once after set-up
+ * (before the first launch), then at least every 100 ms (every 20 ms today) while any fit of the batch is on the
+ * device, and not again once every fit has ended.  When it returns non-zero the library raises the batch's abort
+ * word (mapped host memory the kernels read), issues no further launch, waits for every stream and returns
+ * TOPOLOW_ERR_INTERRUPTED with every result filled in:
+ *   - a job that had already ended (converged, ran all its iterations, non-finite) keeps the result it has without
+ *     the interrupt (positions, MAE, iterations and hold-out sums bit for bit);
+ *   - a job that was stopped has status TOPOLOW_ERR_INTERRUPTED, message "interrupted", iterations_run = the
+ *     iterations it completed, and the best state, trace, pair count and hold-out sums as of its last completed
+ *     iteration (before set-up: the starting positions and no iteration);
+ *   - a job that failed set-up (or has n < 2) keeps its status.
+ * How soon a fit stops: a fit on one CTA (every fit of a batch of 16 or more jobs) at the end of the iteration
+ * it is running; a fit on several CTAs at its next convergence check or finite check, i.e. after at most
+ * min(convergence_check_freq, 10) more iterations; a fit or chunk that had not started yet does not start.
+ * Everything the batch allocated is released before the call returns, the abort word included. */
+TOPOLOW_API int topolow_fit_batch_interruptible(int32_t n_jobs, const topolow_problem* problems,
+                                                const topolow_params* params, topolow_result* results, int32_t device,
+                                                topolow_interrupt_fn poll, void* user);
 
 /* ---- device-resident plan ----------------------------------------------- */
 typedef struct topolow_plan topolow_plan;

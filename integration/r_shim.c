@@ -5,7 +5,7 @@
  *                                   src/optimization.cpp:375-381)
  *   _topolow_fit_batch_b200         one call for a whole batch of independent fits (what the launchers do with
  *                                   parallel::mclapply today: R/adaptive_sampling.R:645-672, :2670-2693), every
- *                                   job with its own hold-out cells (R/adaptive_sampling.R:2639-2647)
+ *                                   job with its own hold-out cells (R/adaptive_sampling.R:2639-2647); Ctrl-C stops it
  *
  * No R exists in the build image.  The file is compiled and RUN there against the stand-in headers of
  * integration/r_stub/ (tests/test_host.py::test_r_shim_*: marshalling, error, interrupt and registration paths
@@ -97,7 +97,9 @@ SEXP _topolow_optimize_layout_b200(SEXP init, SEXP dmat, SEXP tmat, SEXP degrees
  * of device records - R lists hold references, so `job$edge_i <- fold$edge_i` is enough.  Returns a list of
  * per-job lists {converged, iterations, final_mae, final_k, holdout_sum_abs, holdout_count, status, message,
  * positions (only when keep_positions)}: a failed fit is a status + message, never an R error
- * (R/adaptive_sampling.R:2657-2666 turns failures into NA rows).  A batch is not interruptible. */
+ * (R/adaptive_sampling.R:2657-2666 turns failures into NA rows).  Ctrl-C stops the batch as it stops a single fit: the
+ * library is polled while the fits run, stops them, releases what it holds and returns TOPOLOW_ERR_INTERRUPTED, and
+ * the R condition is raised from this frame. */
 SEXP _topolow_fit_batch_b200(SEXP jobs, SEXP keep_positions, SEXP device) {
   if (TYPEOF(jobs) != VECSXP) Rf_error("jobs must be a list");
   const R_xlen_t nj = XLENGTH(jobs);
@@ -139,7 +141,8 @@ SEXP _topolow_fit_batch_b200(SEXP jobs, SEXP keep_positions, SEXP device) {
     SET_VECTOR_ELT(res, 8, pos);
     rs[j].positions = keep ? REAL(pos) : NULL;
   }
-  const int rc = topolow_fit_batch((int32_t)nj, pb, pr, rs, dev);
+  const int rc = topolow_fit_batch_interruptible((int32_t)nj, pb, pr, rs, dev, poll_interrupt, NULL);
+  if (rc == TOPOLOW_ERR_INTERRUPTED) { UNPROTECT(1); Rf_onintr(); Rf_error("interrupted"); }   /* the library has unwound */
   if (rc != TOPOLOW_OK) { UNPROTECT(1); Rf_error("topolow_fit_batch failed with status %d%s%s", rc, nj > 0 ? ": " : "", nj > 0 ? rs[0].message : ""); }
   for (R_xlen_t j = 0; j < nj; ++j) {
     SEXP res = VECTOR_ELT(out, j);

@@ -1,4 +1,4 @@
-/* integration/r_stub/fake_topolow.c - a recording fake of the two library entries the shim calls, for the CPU-only
+/* integration/r_stub/fake_topolow.c - a recording fake of the library entries the shim calls, for the CPU-only
  * marshalling test (no GPU, no fit): it checks what arrives and answers with values that are functions of the
  * inputs, so that the harness can tell whether every field crossed the boundary in the right place. */
 #include <stdio.h>
@@ -51,4 +51,19 @@ int topolow_fit_batch(int32_t n_jobs, const topolow_problem* pb, const topolow_p
     snprintf(rs[0].message + at, sizeof rs[0].message - at, " shared=%d", shared);
   }
   return TOPOLOW_OK;
+}
+
+/* Polls once before each job; without an interrupt it answers what topolow_fit_batch answers. */
+int topolow_fit_batch_interruptible(int32_t n_jobs, const topolow_problem* pb, const topolow_params* pr, topolow_result* rs,
+                                    int32_t device, topolow_interrupt_fn poll, void* user) {
+  if (device < 0) return TOPOLOW_ERR_CUDA;
+  for (int32_t j = 0; j < n_jobs; ++j)
+    if (poll && poll(user)) {
+      for (int32_t k = j; k < n_jobs; ++k) {
+        rs[k].status = TOPOLOW_ERR_INTERRUPTED;
+        snprintf(rs[k].message, sizeof rs[k].message, "interrupted");
+      }
+      return TOPOLOW_ERR_INTERRUPTED;
+    }
+  return topolow_fit_batch(n_jobs, pb, pr, rs, device);
 }

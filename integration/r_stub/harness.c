@@ -7,6 +7,8 @@
  *   harness single    problem.bin out.bin n_iter k0 cooling c_rep rel_eps window freq [mode]
  *   harness interrupt problem.bin at_check
  *   harness batch     problem.bin out.bin n_jobs n_iter k0 cooling c_rep rel_eps window freq keep
+ *   harness batch_interrupt problem.bin out.bin n_jobs n_iter k0 cooling c_rep rel_eps window freq keep at_check
+ *                     (the batch call with R_CheckUserInterrupt firing at its at_check-th call; 0 = never)
  *
  * problem.bin: int64 n, d, E, H | init[n*d] f64 (column-major) | degrees[n] i32 | edge_i[E] edge_j[E] i32 | edge_dist[E]
  * f64 | edge_thresh[E] i32 | holdout_i[H] holdout_j[H] i32 | holdout_truth[H] f64.  out.bin: the doubles named in the
@@ -121,8 +123,10 @@ int main(int argc, char** argv) {
     printf("}\n");
     return 0;
   }
-  if (!strcmp(what, "batch") && argc >= 13) {
+  const int batch_interrupt = !strcmp(what, "batch_interrupt");
+  if ((!strcmp(what, "batch") && argc >= 13) || (batch_interrupt && argc >= 14)) {
     struct problem p = load(argv[2]);
+    if (batch_interrupt) stub.interrupt_after = atoi(argv[13]);
     const int nj = atoi(argv[4]), keep = atoi(argv[12]);
     SEXP jobs = stub_list(nj);
     for (int j = 0; j < nj; ++j) {
@@ -137,7 +141,7 @@ int main(int argc, char** argv) {
     int dev = 0;
     SEXP r = _topolow_fit_batch_b200(jobs, Rf_ScalarLogical(keep), stub_int(1, &dev));
     FILE* o = fopen(argv[3], "wb");
-    printf("{\"scenario\": \"batch\", \"n\": %d, \"names\": [", (int)XLENGTH(r));
+    printf("{\"scenario\": \"%s\", \"left_by\": \"return\", \"n\": %d, \"names\": [", what, (int)XLENGTH(r));
     for (int i = 0; nj > 0 && i < (int)XLENGTH(VECTOR_ELT(r, 0)); ++i) printf("%s\"%s\"", i ? ", " : "", stub_name(VECTOR_ELT(r, 0), i));
     printf("], \"jobs\": [");
     for (int j = 0; j < nj; ++j) {

@@ -51,6 +51,7 @@ INTERRUPT_FN = C.CFUNCTYPE(C.c_int, C.c_void_p)
 
 EXPORTS = [
     "topolow_fit", "topolow_fit_interruptible", "topolow_optimize_layout_exact", "topolow_fit_batch",
+    "topolow_fit_batch_interruptible",
     "topolow_plan_create", "topolow_plan_run", "topolow_plan_result", "topolow_plan_info",
     "topolow_plan_destroy", "topolow_plan_enumerate", "topolow_schedule_enumerate", "topolow_plan_run_job",
     "topolow_plan_end_iteration", "topolow_plan_layout", "topolow_plan_positions", "topolow_plan_enumerate_job",
@@ -90,6 +91,9 @@ def lib() -> C.CDLL:
         _dp, _dp, C.c_char_p, C.c_int32]
     L.topolow_fit_batch.restype = C.c_int
     L.topolow_fit_batch.argtypes = [C.c_int32, C.POINTER(Problem), C.POINTER(Params), C.POINTER(Result), C.c_int32]
+    L.topolow_fit_batch_interruptible.restype = C.c_int
+    L.topolow_fit_batch_interruptible.argtypes = [C.c_int32, C.POINTER(Problem), C.POINTER(Params), C.POINTER(Result),
+                                                  C.c_int32, INTERRUPT_FN, C.c_void_p]
     L.topolow_plan_create.restype = C.c_int
     L.topolow_plan_create.argtypes = [C.POINTER(Problem), C.POINTER(Params), C.POINTER(C.c_void_p), C.c_char_p,
                                       C.c_int32]
@@ -271,10 +275,15 @@ def fit(initial_positions, degrees, edge_i, edge_j, edge_dist, edge_thresh, n_it
     return result_dict(res, out, tr)
 
 
-def fit_batch(jobs, device=0):
+def fit_batch(jobs, device=0, interrupt=None):
     """jobs: list of dicts with the keyword arguments of `fit` (coloured mode).  Returns a list of
     result dicts; a failed job yields {'status': code, 'message': ...} instead of raising
-    (R/adaptive_sampling.R:2657-2666 turns fit errors into NA rows)."""
+    (R/adaptive_sampling.R:2657-2666 turns fit errors into NA rows).
+
+    interrupt: a callable polled while the batch runs (topolow_fit_batch_interruptible); when it returns True the
+    fits stop and TopolowError(ERR_INTERRUPTED) is raised with the per-job list attached as `.results`.  There a job
+    that was stopped is a full result dict with status ERR_INTERRUPTED and a 'message' (its best state as of its last
+    completed iteration); jobs that had already ended are what the uninterrupted call returns."""
     L = lib()
     n = len(jobs)
     probs, pars, ress = (Problem * n)(), (Params * n)(), (Result * n)()
@@ -290,15 +299,25 @@ def fit_batch(jobs, device=0):
         ress[j].positions = out.ctypes.data_as(_dp)
         keep.append((pa, k2))
         outs.append(out)
-    rc = L.topolow_fit_batch(n, probs, pars, ress, device)
-    if rc != OK:
+    if interrupt is None:
+        rc = L.topolow_fit_batch(n, probs, pars, ress, device)
+    else:
+        cb = INTERRUPT_FN(lambda _u: int(bool(interrupt())))
+        rc = L.topolow_fit_batch_interruptible(n, probs, pars, ress, device, cb, None)
+    if rc not in (OK, ERR_INTERRUPTED):
         raise TopolowError(rc, f"topolow_fit_batch failed with status {rc}")
     results = []
     for j in range(n):
-        if ress[j].status != OK:
+        if ress[j].status == ERR_INTERRUPTED:
+            results.append(dict(result_dict(ress[j], outs[j]), message=ress[j].message.decode()))
+        elif ress[j].status != OK:
             results.append(dict(status=int(ress[j].status), message=ress[j].message.decode()))
         else:
             results.append(result_dict(ress[j], outs[j]))
+    if rc == ERR_INTERRUPTED:
+        err = TopolowError(rc, "interrupted")
+        err.results = results
+        raise err
     return results
 
 

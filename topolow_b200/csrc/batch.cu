@@ -8,6 +8,7 @@
 #include <atomic>
 #include <chrono>
 #include <cstdlib>
+#include <cstring>
 #include <functional>
 #include <map>
 #include <string>
@@ -46,14 +47,44 @@ int batch_tile_points() {
   return 64;
 }
 
+// Result of a job the batch stopped before it ran: the starting positions, no iteration.
+void result_not_run(const topolow_problem& pb, topolow_result& r) {
+  double* pos = r.positions;
+  double* trace = r.trace_mae;
+  std::memset(&r, 0, sizeof r);
+  r.positions = pos; r.trace_mae = trace;
+  if (pb.n < 2) {
+    r.status = TOPOLOW_ERR_TOO_FEW_POINTS;
+    set_msg(r.message, sizeof r.message, "Need at least 2 points for embedding");
+    return;
+  }
+  if (pos && pb.initial_positions) std::memcpy(pos, pb.initial_positions, sizeof(double) * (size_t)pb.n * (size_t)pb.ndim);
+  r.status = TOPOLOW_ERR_INTERRUPTED;
+  set_msg(r.message, sizeof r.message, "interrupted");
+}
+
 }  // namespace
 
 extern "C" int topolow_fit_batch(int32_t n_jobs, const topolow_problem* problems, const topolow_params* params,
                       topolow_result* results, int32_t device) {
+  return topolow_fit_batch_interruptible(n_jobs, problems, params, results, device, nullptr, nullptr);
+}
+
+extern "C" int topolow_fit_batch_interruptible(int32_t n_jobs, const topolow_problem* problems, const topolow_params* params,
+                                               topolow_result* results, int32_t device, topolow_interrupt_fn poll,
+                                               void* user) {
   if (n_jobs < 0 || (n_jobs > 0 && (!problems || !params || !results))) return TOPOLOW_ERR_BAD_ARG;
+  if (poll && poll(user)) {
+    for (int j = 0; j < n_jobs; ++j) result_not_run(problems[j], results[j]);
+    return TOPOLOW_ERR_INTERRUPTED;
+  }
   // Independent fits: every job gets its own plan and stream; chunks of all jobs are issued
   // round-robin so that the device always has several fits in flight.
   std::unique_ptr<PinnedBuf<int>> flags;   // declared before the plans: outlives them
+  // The abort word (when the batch can be interrupted): mapped, and 16 aligned bytes, the unit the kernels copy.
+  std::unique_ptr<PinnedBuf<int>> abort_block;
+  volatile int* abort_word = nullptr;
+  const int* d_abort = nullptr;            // its device address
   std::vector<std::unique_ptr<topolow_plan>> plans(n_jobs);
   std::vector<int> left(n_jobs, 0);
   const bool dbg = std::getenv("TOPOLOW_DEBUG") != nullptr;
@@ -139,6 +170,7 @@ extern "C" int topolow_fit_batch(int32_t n_jobs, const topolow_problem* problems
         store = sl.store;
       }
       plans[j] = make_plan(problems[j], pr, store, flags ? (int*)*flags + 2 * j : nullptr);
+      plans[j]->d_abort = d_abort;
       left[j] = pr.n_iter;
     } catch (const CudaError& e) {
       r.status = TOPOLOW_ERR_CUDA; set_msg(r.message, sizeof r.message, e.what()); cudaGetLastError();
@@ -147,10 +179,37 @@ extern "C" int topolow_fit_batch(int32_t n_jobs, const topolow_problem* problems
     }
   };
   try {
-    if (n_jobs > 0) { TL_CUDA(cudaSetDevice(device)); flags.reset(new PinnedBuf<int>(2 * (size_t)n_jobs, cudaHostAllocMapped)); }
+    if (n_jobs > 0) {
+      TL_CUDA(cudaSetDevice(device));
+      flags.reset(new PinnedBuf<int>(2 * (size_t)n_jobs, cudaHostAllocMapped));
+    }
   } catch (const CudaError&) { cudaGetLastError(); flags.reset(); }   // plans then allocate their own
+  if (poll && n_jobs > 0) {
+    try {
+      abort_block.reset(new PinnedBuf<int>(4, cudaHostAllocMapped));   // (page-aligned)
+      abort_word = *abort_block;
+      abort_word[0] = abort_word[1] = abort_word[2] = abort_word[3] = 0;
+      TL_CUDA(cudaHostGetDevicePointer((void**)&d_abort, (void*)*abort_block, 0));
+    } catch (const CudaError&) {   // the fits then cannot see a stop request; the host still stops issuing launches
+      cudaGetLastError();
+      abort_block.reset(); abort_word = nullptr; d_abort = nullptr;
+    }
+  }
   run_pool(n_jobs, setup_one);
   if (dbg) std::fprintf(stderr, "[topolow] batch set-up of %d jobs: %.3f s\n", n_jobs, since());
+  // Interrupt: from the calling thread only (R is single-threaded).  Once it fires, the abort word tells every fit on
+  // the device to stop at its next decision point and no further launch is issued.
+  bool aborted = false;
+  auto last_poll = std::chrono::steady_clock::now();
+  auto poll_now = [&]() {
+    last_poll = std::chrono::steady_clock::now();
+    if (poll(user)) {
+      aborted = true;
+      if (abort_word) { *abort_word = 1; std::atomic_thread_fence(std::memory_order_seq_cst); }
+    }
+    return aborted;
+  };
+  constexpr auto kPollPeriod = std::chrono::milliseconds(20);
   try {
     // Single-CTA fits with 64-point tiles are launched many per kernel (one CTA each), grouped by
     // (ndim, precision, warps): the device runs at most 128 kernels side by side, fewer than it has SMs.
@@ -174,12 +233,13 @@ extern "C" int topolow_fit_batch(int32_t n_jobs, const topolow_problem* problems
     }
     for (int j = 0; j < n_jobs; ++j)
       if (plans[j] && !grouped[j]) TL_CUDA(cudaEventRecord(plans[j]->ev0, plans[j]->stream));
-    bool any = true;
+    if (poll) poll_now();   // after set-up, before the first launch
+    bool any = !aborted;
     while (any) {
       any = false;
-      // (reverse key order = highest ndim first: the longest fits are handed to the SMs first.  A batch
-      // cannot be interrupted, so every fit runs to its own stop in one launch - no chunk boundaries at
-      // which a group would have to wait for its slowest member.)
+      // (reverse key order = highest ndim first: the longest fits are handed to the SMs first.  Every fit
+      // of a group runs to its own stop in one launch - no chunk boundaries at which a group would have to
+      // wait for its slowest member; an interrupt reaches the fits through the abort word instead.)
       for (auto it = groups.rbegin(); it != groups.rend(); ++it) {
         auto& kv = *it;
         Group& g = kv.second;
@@ -197,6 +257,7 @@ extern "C" int topolow_fit_batch(int32_t n_jobs, const topolow_problem* problems
       }
       for (int j = 0; j < n_jobs; ++j) {
         if (!plans[j] || grouped[j] || left[j] <= 0 || plans[j]->h_flag[0]) continue;
+        if (poll && std::chrono::steady_clock::now() - last_poll >= kPollPeriod && poll_now()) { any = false; break; }
         const int c = std::min(left[j], plans[j]->chunk_iters);
         launch_chunk(*plans[j], c, plans[j]->stream);
         left[j] -= c;
@@ -204,9 +265,34 @@ extern "C" int topolow_fit_batch(int32_t n_jobs, const topolow_problem* problems
       }
     }
     if (dbg) std::fprintf(stderr, "[topolow] batch launches issued: %.3f s\n", since());
+    for (auto& kv : groups) TL_CUDA(cudaEventRecord(*kv.second.ev1, *kv.second.stream));
+    for (int j = 0; j < n_jobs; ++j)
+      if (plans[j] && !grouped[j]) TL_CUDA(cudaEventRecord(plans[j]->ev1, plans[j]->stream));
+    if (poll && !aborted) {   // wait with event queries, polling, until every fit has ended or the poll fires
+      std::vector<cudaEvent_t> pending;
+      for (auto& kv : groups) pending.push_back(*kv.second.ev1);
+      for (int j = 0; j < n_jobs; ++j)
+        if (plans[j] && !grouped[j]) pending.push_back(plans[j]->ev1);
+      while (true) {
+        for (size_t i = 0; i < pending.size();) {
+          const cudaError_t q = cudaEventQuery(pending[i]);
+          if (q == cudaErrorNotReady) { ++i; continue; }
+          TL_CUDA(q);
+          pending[i] = pending.back();
+          pending.pop_back();
+        }
+        if (pending.empty()) break;
+        if (std::chrono::steady_clock::now() - last_poll >= kPollPeriod) {
+          if (poll_now()) break;
+        } else {
+          std::this_thread::sleep_for(std::chrono::microseconds(200));
+        }
+      }
+      if (cudaPeekAtLastError() == cudaErrorNotReady) cudaGetLastError();
+      if (dbg) std::fprintf(stderr, "[topolow] batch %s: %.3f s\n", aborted ? "interrupted" : "fits ended", since());
+    }
     for (auto& kv : groups) {
       Group& g = kv.second;
-      TL_CUDA(cudaEventRecord(*g.ev1, *g.stream));
       TL_CUDA(cudaEventSynchronize(*g.ev1));
       float ms = 0.f;
       TL_CUDA(cudaEventElapsedTime(&ms, *g.ev0, *g.ev1));
@@ -215,13 +301,15 @@ extern "C" int topolow_fit_batch(int32_t n_jobs, const topolow_problem* problems
     for (int j = 0; j < n_jobs; ++j) {
       if (!plans[j]) continue;
       if (!grouped[j]) {
-        TL_CUDA(cudaEventRecord(plans[j]->ev1, plans[j]->stream));
         TL_CUDA(cudaEventSynchronize(plans[j]->ev1));
         float ms = 0.f;
         TL_CUDA(cudaEventElapsedTime(&ms, plans[j]->ev0, plans[j]->ev1));
         plans[j]->total_ms = ms;
       }
-      fill_result(*plans[j], results[j], false);
+      // After an interrupt, a fit that neither stopped (converged, non-finite, or stopped by the abort word: that
+      // one carries kStatusStopped) nor ran all its iterations was cut short on the host: it is interrupted too.
+      const bool cut = aborted && !plans[j]->h_flag[0] && plans[j]->h_flag[1] < plans[j]->prm.n_iter;
+      fill_result(*plans[j], results[j], cut);
     }
     if (dbg) std::fprintf(stderr, "[topolow] batch results read: %.3f s\n", since());
     plans.clear();
@@ -232,6 +320,6 @@ extern "C" int topolow_fit_batch(int32_t n_jobs, const topolow_problem* problems
     cudaGetLastError();
     return TOPOLOW_ERR_CUDA;
   }
-  return TOPOLOW_OK;
+  return aborted ? TOPOLOW_ERR_INTERRUPTED : TOPOLOW_OK;
 }
 

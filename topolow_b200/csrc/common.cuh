@@ -148,11 +148,15 @@ struct FitState {
   int stop;              // loop must not run further iterations (converged or failed)
   int iter;              // iterations completed so far
   int snapshot;          // set by controller_check when best_* was updated by this check
-  int status;            // 0 ok, 2 non-finite
+  int status;            // 0 ok, 2 non-finite, kStatusStopped
   int fail_iter;
   int pad;
   unsigned long long pair_updates;
 };
+
+// FitState::status of a fit that the caller stopped through the batch's abort word (TileDev::abort) before it
+// converged or ran all its iterations (the value of TOPOLOW_ERR_INTERRUPTED).
+constexpr int kStatusStopped = 5;
 
 TL_HD void state_init(FitState& s, const FitParams& p) {
   s.k = p.k0;

@@ -438,7 +438,7 @@ void fill_result(topolow_plan& pl, topolow_result& res, bool interrupted) {
     res.status = TOPOLOW_ERR_NONFINITE;
     std::snprintf(res.message, sizeof res.message,
                   "Numerical instability at iteration %d. Reduce k0 or c_repulsion.", st.fail_iter);
-  } else if (interrupted) {
+  } else if (interrupted || st.status == kStatusStopped) {
     res.status = TOPOLOW_ERR_INTERRUPTED;
     std::snprintf(res.message, sizeof res.message, "interrupted");
   }

@@ -40,6 +40,7 @@ struct topolow_plan {
   tl::FitState* state = nullptr; double* partials = nullptr; unsigned* barrier = nullptr; double* trace = nullptr;
   int64_t n_holdout = 0; int32_t* hold_si = nullptr; int32_t* hold_sj = nullptr; double* hold_truth = nullptr;   // slots of the hold-out cells
   volatile int* h_flag = nullptr; int* d_flag = nullptr; bool owns_flag = true;   // mapped host words: stop flag, iterations done
+  const int* d_abort = nullptr;   // the abort word of the batch the plan runs in (mapped, owned by the batch), or null
   cudaStream_t stream = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   int chunk_iters = 1;
@@ -81,7 +82,7 @@ template <class real>
 TileDev<real> device_view(const topolow_plan& pl) {
   const unsigned long long ppi = (unsigned long long)pl.n * (unsigned long long)(pl.n - 1) / 2ull;
   return TileDev<real>{(real*)pl.pos, (real*)pl.best, (const real*)pl.dp1, pl.store->edges, pl.store->bucket_off, pl.state,
-                       pl.partials, pl.barrier, pl.trace, (long long)pl.E, ppi};
+                       pl.partials, pl.barrier, pl.trace, (long long)pl.E, ppi, pl.d_abort};
 }
 void launch_chunk(topolow_plan& pl, int n_iters, cudaStream_t stream);
 void fill_result(topolow_plan& pl, topolow_result& res, bool interrupted);

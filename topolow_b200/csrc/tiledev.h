@@ -28,6 +28,7 @@ struct TileDev {
   double* trace;         // [n_iter] or null
   long long n_edges;
   unsigned long long pairs_per_iter;
+  const volatile int* abort;   // mapped host word: non-zero = the caller asks the fit to stop (null = never)
 };
 
 // One entry of a many-fits launch (tile_batch_kernel).

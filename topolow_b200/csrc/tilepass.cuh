@@ -351,6 +351,30 @@ TL_D unsigned ld_acquire_u32(const unsigned* p) {
   return v;
 }
 
+// The caller's stop request (TileDev::abort, 16 readable bytes of mapped host memory) is fetched into shared memory by the
+// bulk-copy unit at the start of an iteration and read at its end: nothing waits for the host round trip and no
+// register holds the value across the pair passes.  One copy per iteration, so the barrier's phase is the parity of
+// the copies issued before.
+TL_D unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
+TL_D void stop_word_init(unsigned long long* bar) {
+  asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(bar)) : "memory");
+  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+}
+TL_D void stop_word_fetch(int* dst, unsigned long long* bar, const volatile int* src) {
+  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], 16;" ::"r"(smem_u32(bar)) : "memory");
+  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], 16, [%2];"
+               ::"r"(smem_u32(dst)), "l"(src), "r"(smem_u32(bar)) : "memory");
+}
+TL_D int stop_word_read(const int* s, unsigned long long* bar, unsigned parity) {
+  unsigned done = 0;
+  do {
+    asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
+                 : "=r"(done) : "r"(smem_u32(bar)), "r"(parity) : "memory");
+  } while (!done);
+  return *reinterpret_cast<const volatile int*>(s);
+}
+
 // FitState moves between CTAs through L2 (never a stale L1 line).
 static_assert(sizeof(FitState) % 8 == 0, "FitState is copied as 64-bit words");
 TL_D void load_state(FitState& dst, const FitState* src) {
@@ -810,20 +834,35 @@ TL_D void tile_body(const TileDev<typename M::real>& dv, const Geometry& geo, co
   };
   const WarpTable<real> tb{s_tgt + (size_t)warp * kTableReals, s_mask + warp * kTableMasks};
 
+  __shared__ __align__(16) int s_stop_word[4];
+  __shared__ __align__(8) unsigned long long s_stop_bar;
+
   unsigned gen = 0;
   if (tid == 0) load_state(st, dv.state);
+  // Only CTA 0 reads the stop request (the CTAs of a fit must agree), and a stop never overrides a fit that has already
+  // ended.  A CTA or chunk that starts after the request runs no iteration.
+  if (cta == 0 && tid == 0 && dv.abort) {
+    stop_word_init(&s_stop_bar);
+    if (*dv.abort && !st.stop && st.iter < prm.n_iter) { st.stop = 1; st.status = kStatusStopped; }
+  }
   if (geo.G > 1) gen = ld_acquire_u32(&dv.barrier[1]);
   __syncthreads();
   unsigned* done = dv.barrier + kDoneOffset;
   unsigned epoch = 0;   // cross rounds completed since the start of this launch
   if (geo.G > 1) {
     for (int b = cta * blockDim.x + tid; b < geo.S; b += geo.G * blockDim.x) __stcg(done + b, 0u);
+    if (dv.abort && cta == 0 && tid == 0) store_state(dv.state, st);   // publish CTA 0's decision
     gang_barrier(dv.barrier, geo.G, gen);
+    if (dv.abort) {
+      if (cta != 0 && tid == 0) load_state(st, dv.state);
+      __syncthreads();
+    }
   }
 
   for (int it = 0; it < n_iters; ++it) {
     if (st.stop || st.iter >= prm.n_iter) break;   // never past n_iter: trace[] holds n_iter entries, the forced last check is iter == n_iter - 1
     const int iter = st.iter;
+    if (cta == 0 && tid == 0 && dv.abort && geo.do_end) stop_word_fetch(s_stop_word, &s_stop_bar, dv.abort);
     const typename M::Ctx ctx = M::make_ctx(st.k, prm.c_repulsion);
     if (tid < kIterKeys) s_key[tid] = iter_key(geo, iter, (uint32_t)tid);
     if (geo.table) {
@@ -985,6 +1024,9 @@ TL_D void tile_body(const TileDev<typename M::real>& dv, const Geometry& geo, co
         }
         if (!st.stop && fin && b > 0.0) { st.status = 2; st.fail_iter = iter + 1; st.stop = 1; }
         st.iter = iter + 1;
+        if (dv.abort && stop_word_read(s_stop_word, &s_stop_bar, it & 1) && !st.stop && st.iter < prm.n_iter) {
+          st.stop = 1; st.status = kStatusStopped;
+        }
         store_state(dv.state, st);
       }
       gang_barrier(dv.barrier, geo.G, gen);
@@ -997,7 +1039,14 @@ TL_D void tile_body(const TileDev<typename M::real>& dv, const Geometry& geo, co
         gang_barrier(dv.barrier, geo.G, gen);
       }
     } else {
-      if (tid == 0) st.iter = iter + 1;
+      if (tid == 0) {
+        st.iter = iter + 1;
+        // (every fetch is waited for; a fit of several CTAs stops only where CTA 0 publishes its state, above)
+        if (cta == 0 && dv.abort && stop_word_read(s_stop_word, &s_stop_bar, it & 1) && geo.G == 1 && !st.stop &&
+            st.iter < prm.n_iter) {
+          st.stop = 1; st.status = kStatusStopped;
+        }
+      }
       __syncthreads();
     }
   }

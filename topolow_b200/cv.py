@@ -199,7 +199,7 @@ def _fold_job(value, code, is_na, holdout, preserve_order):
 
 def likelihood_batch(dissimilarity_matrix, samples, mapping_max_iter, relative_epsilon, folds=20,
                      preserve_order=True, *, fold_indices=None, init_list=None, rng=None, seed=0, device=0,
-                     precision="f32"):
+                     precision="f32", interrupt=None):
     """Evaluate many parameter samples at once.  `samples` is a list of dicts with keys N, k0,
     cooling_rate, c_repulsion; returns one likelihood_function() result per sample.  All
     len(samples) x folds fits run in a single topolow_fit_batch call.
@@ -212,21 +212,25 @@ def likelihood_batch(dissimilarity_matrix, samples, mapping_max_iter, relative_e
     likelihood_function per sample for the reference's behaviour.
 
     preserve_order defaults to True here because fold residuals are aligned by position; the
-    reference re-aligns by row names (R/error_metrics.R:76-87) which an unnamed matrix lacks."""
+    reference re-aligns by row names (R/error_metrics.R:76-87) which an unnamed matrix lacks.
+
+    interrupt: a callable polled while the fits run (see _lib.fit_batch); when it returns True the batch stops and
+    TopolowError(ERR_INTERRUPTED) is raised."""
     rng = rng or np.random.default_rng(seed)
     value, code, is_na = parse_dissimilarity(dissimilarity_matrix)
     if fold_indices is None:
         fold_indices = make_folds(dissimilarity_matrix, folds, rng)
     fold_jobs = [_fold_job(value, code, is_na, np.asarray(h), preserve_order) for h in fold_indices]
-    return _run_folds(fold_jobs, samples, mapping_max_iter, relative_epsilon, init_list, rng, seed, device, precision)
+    return _run_folds(fold_jobs, samples, mapping_max_iter, relative_epsilon, init_list, rng, seed, device, precision,
+                      interrupt)
 
 
 def likelihood_batch_coo(n, rows, cols, values, samples, mapping_max_iter, relative_epsilon, folds=20, *, diagonal=True,
-                         fold_cells=None, init_list=None, rng=None, seed=0, device=0, precision="f32"):
+                         fold_cells=None, init_list=None, rng=None, seed=0, device=0, precision="f32", interrupt=None):
     """likelihood_batch for a dissimilarity table (0-based rows / cols, values numbers or threshold strings): the folds
     are drawn and masked on the cell list (make_folds_cells / fold_problem_cells), nothing n x n is built, and the
     hold-out cells are scored on the device inside each fit.  Row order is the table's (preserve_order = TRUE).
-    `fold_cells` injects the drawn cell ids (see make_folds_cells)."""
+    `fold_cells` injects the drawn cell ids (see make_folds_cells); `interrupt` as in likelihood_batch."""
     rng = rng or np.random.default_rng(seed)
     full = build_problem_coo(n, rows, cols, values, preserve_order=True, diagonal=diagonal)
     base = n if diagonal else 0
@@ -238,7 +242,8 @@ def likelihood_batch_coo(n, rows, cols, values, samples, mapping_max_iter, relat
         kept = prob["edge_thresh"] == 0       # R/core.R:407-409: the largest plain number of the fold's TRAINING matrix
         prob["init_step"] = (max(float(prob["edge_dist"][kept].max()), 0.0) if kept.any() else 0.0) / n
         fold_jobs.append((prob, hi, hj, ht))
-    return _run_folds(fold_jobs, samples, mapping_max_iter, relative_epsilon, init_list, rng, seed, device, precision)
+    return _run_folds(fold_jobs, samples, mapping_max_iter, relative_epsilon, init_list, rng, seed, device, precision,
+                      interrupt)
 
 
 def _initial_positions(prob, ndim, rng):
@@ -248,7 +253,8 @@ def _initial_positions(prob, ndim, rng):
     return np.vstack([np.zeros((1, ndim)), np.cumsum(steps, axis=0)])
 
 
-def _run_folds(fold_jobs, samples, mapping_max_iter, relative_epsilon, init_list, rng, seed, device, precision):
+def _run_folds(fold_jobs, samples, mapping_max_iter, relative_epsilon, init_list, rng, seed, device, precision,
+               interrupt=None):
     """All len(samples) x len(fold_jobs) fits in one topolow_fit_batch call, pooled as R/adaptive_sampling.R:2695-2725."""
     prec_c = {"f32": _lib.PREC_F32, "f64": _lib.PREC_F64_EXACT}[precision]
     # hold-out cells in the row numbering of the fold's training problem: they are scored on the device
@@ -278,7 +284,8 @@ def _run_folds(fold_jobs, samples, mapping_max_iter, relative_epsilon, init_list
                              c_repulsion=s["c_repulsion"], relative_epsilon=relative_epsilon, convergence_window=5,
                              precision=prec_c, seed=seed + 1000003 * s_idx + f_idx, holdout=fold_holdout[f_idx]))
             meta.append((s_idx, f_idx, len(jobs) - 1))
-    results = _lib.fit_batch(jobs, device=device) if jobs else []
+    extra = {} if interrupt is None else {"interrupt": interrupt}
+    results = _lib.fit_batch(jobs, device=device, **extra) if jobs else []
 
     per_sample = [[] for _ in samples]
     for s_idx, f_idx, j in meta:
@@ -306,9 +313,10 @@ def _run_folds(fold_jobs, samples, mapping_max_iter, relative_epsilon, init_list
 
 
 def likelihood_function(dissimilarity_matrix, mapping_max_iter, relative_epsilon, N, k0, cooling_rate, c_repulsion,
-                        folds=20, num_cores=1, preserve_order=True, **kw):
+                        folds=20, num_cores=1, preserve_order=True, *, interrupt=None, **kw):
     """Single-sample form with the reference's signature (R/adaptive_sampling.R:2552-2555);
-    num_cores is accepted and ignored (the folds already run concurrently on the device)."""
+    num_cores is accepted and ignored (the folds already run concurrently on the device).
+    `interrupt` as in likelihood_batch."""
     return likelihood_batch(dissimilarity_matrix, [dict(N=N, k0=k0, cooling_rate=cooling_rate,
                                                         c_repulsion=c_repulsion)], mapping_max_iter,
-                            relative_epsilon, folds, preserve_order, **kw)[0]
+                            relative_epsilon, folds, preserve_order, interrupt=interrupt, **kw)[0]

@@ -595,22 +595,6 @@ def test_exact_sharded_map_over_nccl_equals_the_emulation(tmp_path):
     assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-2000:]
 
 
-def test_rowblock_inner_product_variant_tracks_the_restatement(monkeypatch):
-    """The inner-product form of the repulsion pass (rowblock.cu, TOPOLOW_REP_VARIANT=6; not the default - see the
-    measurements next to repulse_variant) computes the same sums: near pairs and the point itself take the
-    difference form, everything else |p|^2 + |q|^2 - 2 p.q."""
-    from topolow_b200 import rowblock
-    monkeypatch.setenv("TOPOLOW_REP_VARIANT", "6")
-    for n, d, dens in ((700, 5, 0.1), (2100, 16, 0.02), (600, 10, 0.08)):
-        args = small_problem(n, d, dens, 10 * n + d, thresholds=True)
-        want = cpu_oracle.relaxed_optimize_layout(*args, 6, 5.0, 0.01, 0.02, 1e-4, 5, 3, seed=4, slot_of_point=rowblock.slot_order(n))
-        got = _lib.fit(*args, 6, 5.0, 0.01, 0.02, 1e-4, 5, 3, mode=_lib.MODE_ROWBLOCK, seed=4)
-        scale = max(np.abs(want["positions"]).max(), 1.0)
-        err = np.abs(got["positions"] - want["positions"])
-        assert np.quantile(err, 0.99) <= 2e-4 * scale and err.max() <= 2e-3 * scale
-        assert got["final_mae"] == pytest.approx(want["final_mae"], rel=1e-3)
-
-
 def test_sparse_table_entry_equals_the_matrix_entry():
     """euclidean_embedding_coo (nothing n x n is built) returns the positions, convergence fields and mae of
     euclidean_embedding on the matrix the table stands for; est_distances on the listed pairs and on extra

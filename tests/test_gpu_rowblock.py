@@ -83,7 +83,7 @@ def test_rowblock_holdout_trace_and_interrupt():
     assert e.value.status == _lib.ERR_INTERRUPTED and len(calls) == 3
 
 
-def test_rowblock_error_paths():
+def test_rowblock_error_paths(monkeypatch):
     init = np.zeros((300, 2)); init[:, 0] = np.arange(300)
     deg = np.full(300, 2, dtype=np.int32)
     with pytest.raises(_lib.TopolowError) as e:
@@ -102,6 +102,12 @@ def test_rowblock_error_paths():
     dup = [args[0], args[1]] + [np.r_[a, a[:5]] for a in args[2:]]      # a pair listed twice is tolerated
     r = _lib.fit(*dup, 5, 1.0, 0.01, 0.01, mode=_lib.MODE_ROWBLOCK)
     assert np.all(np.isfinite(r["positions"]))
+    args8 = small_problem(600, 8, 0.08, 8)
+    for form in ("6", "10"):                                          # forms that were measured and dropped
+        monkeypatch.setenv("TOPOLOW_REP_VARIANT", form)
+        with pytest.raises(_lib.TopolowError) as e:
+            _lib.fit(*args8, 4, 1.0, 0.01, 0.01, mode=_lib.MODE_ROWBLOCK)
+        assert e.value.status == _lib.ERR_BAD_ARG and "takes 5" in str(e.value)
 
 
 # ------------------------------------------------------------------ sharding ---------------------

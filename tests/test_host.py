@@ -582,20 +582,22 @@ def test_lhs_design_and_batched_chains():
         sampler.adaptive_mc_batch({k: v for k, v in t.items() if k != "NLL"}, None, 1, 2, 10, 1e-4, evaluate=evaluate)
 
 
-def test_series_weight_constants_of_the_tensor_repulsion_pass():
+def test_series_weight_constant_is_shared_by_the_probe_and_the_tensor_pass():
     """rowblock_tc2.cuh computes the repulsion weight (d + 0.01)^-3 of a pair from S = d^2 / 2 with one rsqrt and a cubic
     (src/optimization.cpp:257-267 is the formula it stands for).  The constants are read from the source: for every
-    pair the series form accepts (S >= kT2SeriesS, i.e. d >= 0.1) the result is within 1.2e-5 of the formula - far inside
-    the TF32 rounding (4.9e-4) the weight gets next -, the threshold is the one the probe in rowblock_tc.cuh counts
-    with, and the two-MUFU form's constants restate the same formula."""
+    pair the series form accepts (S >= kSeriesNearS, i.e. d >= 0.1) the result is within 1.2e-5 of the formula - far inside
+    the TF32 rounding (4.9e-4) the weight gets next -, the probe in image_tc_kernel counts near pairs of the series form
+    against the same constant, and the two-MUFU form's constants restate the same formula."""
     import re
     src = open(os.path.join(ROOT, "topolow_b200", "csrc", "rowblock_tc2.cuh")).read()
-    probe = open(os.path.join(ROOT, "topolow_b200", "csrc", "rowblock_tc.cuh")).read()
     m = re.search(r"float pl = fmaf\(([-0-9.e+]+)f, q, ([-0-9.e+]+)f\);\s*pl = fmaf\(pl, q, ([-0-9.e+]+)f\);\s*pl = fmaf\(pl, q, ([-0-9.e+]+)f\);", src)
     assert m, "series polynomial not found"
     c3, c2, c1, c0 = (float(x) for x in m.groups())
-    s_min = float(re.search(r"constexpr float kT2SeriesS = ([0-9.e+-]+)f;", src).group(1))
-    assert s_min == float(re.search(r"constexpr float kSeriesNearS = ([0-9.e+-]+)f;", probe).group(1)) == 0.005
+    consts = re.findall(r"constexpr float kSeriesNearS = ([0-9.e+-]+)f;", src)
+    assert len(consts) == 1 and float(consts[0]) == 0.005
+    s_min = float(consts[0])
+    assert re.search(r"0\.5f \* d2 < fmaxf\(3\.01e-3f \* h_hi, kSeriesNearS\)", src), "the probe does not use kSeriesNearS"
+    assert re.search(r"if \(series\) thr\[r\] = fmaxf\(thr\[r\], kSeriesNearS\);", src), "the pass does not use kSeriesNearS"
     d = np.concatenate([np.geomspace(np.sqrt(2 * s_min), 1e4, 20001), np.linspace(0.1, 0.3, 5001)])
     S = 0.5 * d * d
     q = 1.0 / np.sqrt(S)

@@ -55,3 +55,13 @@ def test_walk_and_pass_register_budget(usage):
         assert len(rep) == 1, f"repulse_tc2_kernel<{h}>: found {sorted(rep)}"
         for name, (regs, _shared) in rep.items():
             assert regs <= PASS_REGS, f"{name}: {regs} registers > {PASS_REGS}"
+
+
+def test_repulsion_kernels_are_the_two_forms_the_policy_runs(usage):
+    """For every H of ndim 1..16 the library holds the kernels of the two forms of the repulsion pass and nothing else:
+    one shape of the FP32 difference form (repulse_kernel) and the two-GEMM tensor-core form (image_tc_kernel,
+    repulse_tc2_kernel)."""
+    for h in H_VALUES:
+        found = sorted(re.search(r"((?:repulse|image)\w*?)ILi", n).group(1)
+                       for n in _kernels(usage, r"(?:repulse|image)\w*?ILi%dE" % h))
+        assert found == ["image_tc_kernel", "repulse_kernel", "repulse_tc2_kernel"], f"H = {h}: {found}"

@@ -2,8 +2,8 @@
 
 The built library (cuobjdump -res-usage) holds, for every H of that range (10, 12, 14, 16), the kernels the mode launches
 - spring and MAE walks with both ring depths, combine_kernel, the FP32 difference form of the repulsion pass - with no
-stack (no spills) and within the register caps of rowblock.cu, and none of the tensor-core or inner-product forms, which
-exist for ndim <= 16 only.  And the FP64 restatement shows the invariant the padded rows rely on: zero columns stay zero
+stack (no spills) and within the register caps of rowblock.cu, and not the tensor-core form, which exists for
+ndim <= 16 only.  And the FP64 restatement shows the invariant the padded rows rely on: zero columns stay zero
 and leave the other columns bit for bit as they are."""
 import os
 import re
@@ -47,10 +47,10 @@ def _kernels(usage, pattern):
 
 
 @pytest.mark.parametrize("h", H_WIDE)
-def test_wide_rows_kernels_exist_without_spills_within_their_caps(usage, h):
+def test_wide_rows_launched_kernels_exist_without_spills_within_their_caps(usage, h):
     for kernel, count, cap in ((r"spring_kernelILi%dELi\d+E", 2, WALK_REGS_WIDE), (r"mae_kernelILi%dELi\d+E", 2, MAE_REGS),
                                (r"combine_kernelILi%dEE", 1, COMBINE_REGS),
-                               (r"repulse_kernelILi%dELi1ELi\d+ELi%dELb1EE", 1, REP_REGS_WIDE)):
+                               (r"repulse_kernelILi%dELi1ELi\d+ELi%dEE", 1, REP_REGS_WIDE)):
         pat = kernel % ((h, REP_REGS_WIDE) if "repulse" in kernel else h)
         found = _kernels(usage, pat)
         assert len(found) == count, f"{pat}: expected {count}, found {sorted(found)}"
@@ -61,7 +61,7 @@ def test_wide_rows_kernels_exist_without_spills_within_their_caps(usage, h):
 
 @pytest.mark.parametrize("h", H_WIDE)
 def test_wide_rows_build_no_tensor_or_inner_product_form(usage, h):
-    for kernel in ("repulse_tc_kernel", "repulse_tc2_kernel", "repulse_dot_kernel", "image_tc_kernel", "image_kernel"):
+    for kernel in ("repulse_tc2_kernel", "image_tc_kernel"):
         found = _kernels(usage, r"%sILi%dE" % (kernel, h))
         assert not found, sorted(found)
     # only the one shape of the difference form

@@ -68,8 +68,6 @@ struct RowDev {
   const float* dp1;                  // [slots] degree + 1 (0 = padding row)
   float* rpart;                      // [chunks][rows][Dp] repulsion sums per partner chunk
   float* xs;                         // [rows][Dp] positions of the own rows after the spring walk (before the repulsion is added)
-  float* img;                        // [cap_rows][Img<H>::kStride] partner image of the iteration: -2 (P_j - centre) | |P_j - centre|^2 / 2 twice
-  float* hmax;                       // [2] max over all points of |P_j - centre|^2 / 2, per position buffer
   float centre[16];                  // centroid of the initial positions (fixed for the fit, the same on every rank)
   const uint2* recs;                 // spring records of the own rows, SELL-32: {partner | type << 30, target}
   const unsigned long long* soff;    // [rows / 32] first record of a slice
@@ -160,14 +158,14 @@ TL_D float lg2_approx(float x) { float r; asm("lg2.approx.ftz.f32 %0, %1;" : "=f
 TL_D float ex2_approx(float x) { float r; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x)); return r; }
 
 // One-sided repulsion of partner q on the point -np: acc += (q - p) / (|q - p| + 0.01)^3.
-// kPow: the cube and its reciprocal as 2^(-3 log2(ds)) on the special-function unit (two MUFU + one multiply)
-// instead of two multiplies + MUFU.RCP: one FMA-pipe slot less in a loop that is bound by that pipe.
-template <int H, bool kPow = false>
+// The cube and its reciprocal as 2^(-3 log2(ds)) on the special-function unit (two MUFU + one multiply) instead of two
+// multiplies + MUFU.RCP: one FMA-pipe slot less in a loop that is bound by that pipe.
+template <int H>
 TL_D void repel(const float2 (&np)[H], const float2 (&q)[H], float2 (&acc)[H]) {
   float2 dl[H];
   const float d2 = dist2<H, 1>(np, q, dl);
   const float ds = sqrt_approx(d2) + 0.01f;
-  const float w = kPow ? ex2_approx(-3.0f * lg2_approx(ds)) : rcp_approx(ds * ds * ds);
+  const float w = ex2_approx(-3.0f * lg2_approx(ds));
   const float2 ww = make_float2(w, w);
 #pragma unroll
   for (int k = 0; k < H; ++k) acc[k] = __ffma2_rn(dl[k], ww, acc[k]);
@@ -223,7 +221,7 @@ TL_D bool last_cta(unsigned* counter) {
 // ---------------------------------------------------------------------------------------------------
 // Items are handed out by an atomic counter (reset by combine_kernel's last CTA): the partial sums of an
 // item do not depend on which CTA computed it, so the result is the same whatever the residency pattern.
-template <int H, int R, int U, int MAXR, bool kPow>
+template <int H, int R, int U, int MAXR>
 __global__ void __maxnreg__(MAXR) repulse_kernel(RowDev dv, int cur, unsigned epoch) {
   extern __shared__ float4 smem4[];
   __shared__ long long item_s;
@@ -278,7 +276,7 @@ __global__ void __maxnreg__(MAXR) repulse_kernel(RowDev dv, int cur, unsigned ep
         float2 q[H];
         ld_point<H>(q_s + j * Dp, q);
 #pragma unroll
-        for (int r = 0; r < R; ++r) repel<H, kPow>(np[r], q, acc[r]);
+        for (int r = 0; r < R; ++r) repel<H>(np[r], q, acc[r]);
       }
     }
 #pragma unroll
@@ -288,225 +286,6 @@ __global__ void __maxnreg__(MAXR) repulse_kernel(RowDev dv, int cur, unsigned ep
   }
 }
 
-// ---------------------------------------------------------------------------------------------------
-// repulsion, inner-product form (ndim >= 5): |q - p|^2 = |p|^2 + |q|^2 - 2 p.q
-// ---------------------------------------------------------------------------------------------------
-// The difference form above spends 3 packed FMA-pipe instructions per coordinate pair and interaction
-// (q - p, its square, the accumulation of w (q - p)); the pass is bound by that pipe (ncu: 82 % busy).  Written
-// with inner products an interaction needs 2: p.q~ (q~ = -2 (q - centre), its half norm rides in the accumulator's
-// start value) and A += w q~, plus W += w; the sum over the partners comes out as -A / 2 - p W at the end of the
-// item.  image_kernel prepares q~ and the half norms once per iteration (6 MB read, 8 MB written).
-// Cancellation: the rounding error of the inner-product distance is about (H + 1) 2^-24 (|p|^2 + |q|^2), harmless for
-// a pair that is far apart and fatal for one that is not.  Pairs with d^2 < thr = (H + 1) 2^-13 (|p|^2 / 2 + max_j |q_j|^2 / 2)
-// ("near": relative error of d^2 could exceed 1e-3; a handful per point in 5 dimensions, none in 16, always the
-// point itself) get weight 0 in the main loop, raise a flag, and the stage is walked again for them in the
-// difference form into a thread-private accumulator in shared memory - the same arithmetic as repulse_kernel.
-template <int H> struct Img { static constexpr int kStride = (2 * H + 2 + 3) / 4 * 4; };
-
-template <int NF4>
-TL_D float f4_elem(const float4 (&t)[NF4], int e) {
-  const float4& x = t[e >> 2];
-  switch (e & 3) { case 0: return x.x; case 1: return x.y; case 2: return x.z; default: return x.w; }
-}
-// image row: H packed pairs of q~ and the half norm (in both lanes of hh)
-template <int H>
-TL_D void ld_image(const float* __restrict__ p, float2 (&v)[H], float2& hh) {
-  constexpr int NF4 = Img<H>::kStride / 4;
-  float4 t[NF4];
-#pragma unroll
-  for (int k = 0; k < NF4; ++k) t[k] = reinterpret_cast<const float4*>(p)[k];
-#pragma unroll
-  for (int k = 0; k < H; ++k) v[k] = make_float2(f4_elem<NF4>(t, 2 * k), f4_elem<NF4>(t, 2 * k + 1));
-  hh = make_float2(f4_elem<NF4>(t, 2 * H), f4_elem<NF4>(t, 2 * H + 1));
-}
-// d^2 by inner product and the near test.  Explicit roundings: the main loop and the second walk must agree bit for bit.
-template <int H>
-TL_D bool near_test(const float2 (&p)[H], float sp, float thr, const float2 (&q)[H], float2 hh, float& d2) {
-  float2 s = __ffma2_rn(p[0], q[0], hh);
-#pragma unroll
-  for (int k = 1; k < H; ++k) s = __ffma2_rn(p[k], q[k], s);
-  d2 = __fadd_rn(__fadd_rn(s.x, s.y), sp);
-  return d2 < thr;
-}
-// kSeries: (dist + 0.01)^-3 = (r (1 - x + x^2 - x^3))^3 (1 + O(x^4)) with r = 1 / dist (one MUFU.RSQ) and x = 0.01 r -
-// seven FMA-pipe instructions instead of three MUFU (sqrt, lg2, ex2), each of which holds the quarter's
-// special-function unit for 8 cycles.  Only pairs that pass the near test get here: the threshold is never below
-// kSeriesFloor = 0.1 (dist > 0.316, x < 0.0316, x^4 < 1e-6), the others take the exact formula in the second walk.
-constexpr float kSeriesFloor = 0.1f;
-TL_D float rsqrt_approx(float x) { float r; asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x)); return r; }
-template <int H, bool kSeries>
-TL_D bool repel_dot(const float2 (&p)[H], float sp, float thr, const float2 (&q)[H], float2 hh, float2 (&acc)[H], float& W) {
-  float d2;
-  const bool nr = near_test<H>(p, sp, thr, q, hh, d2);
-  float w;
-  if constexpr (kSeries) {
-    const float r = rsqrt_approx(d2);
-    const float a = fmaf(-0.01f, r, 1.0f);
-    const float b = (r * r) * 1e-4f;
-    const float u = r * fmaf(b, a, a);
-    w = u * u * u;
-  } else {
-    const float ds = sqrt_approx(d2) + 0.01f;
-    w = ex2_approx(-3.0f * lg2_approx(ds));
-  }
-  w = nr ? 0.f : w;                      // also swallows the NaN of a slightly negative d2
-  const float2 ww = make_float2(w, w);
-#pragma unroll
-  for (int k = 0; k < H; ++k) acc[k] = __ffma2_rn(q[k], ww, acc[k]);
-  W += w;
-  return nr;
-}
-
-template <int H>
-__global__ void __launch_bounds__(kBlockRows) image_kernel(RowDev dv, int cur, unsigned epoch) {
-  constexpr int Dp = Row<H>::kStride, Dq = Img<H>::kStride;
-  if (__ldcg(&dv.state->stop)) return;
-  if (!wait_epoch(dv, epoch)) { if (blockIdx.x == 0 && threadIdx.x == 0) peer_timeout(dv); return; }
-  const int row = blockIdx.x * kBlockRows + threadIdx.x;
-  if (row == 0) dv.hmax[cur ^ 1] = 0.f;          // the other buffer's maximum: its readers (the previous iteration) are done
-  const float* __restrict__ P = dv.pos[dv.rank] + (size_t)cur * dv.cap_rows * Dp;
-  float2 p[H];
-  ld_point<H>(P + (size_t)row * Dp, p);
-  float4 o[Dq / 4];
-  float* of = reinterpret_cast<float*>(o);
-  float2 s = make_float2(0.f, 0.f);
-#pragma unroll
-  for (int k = 0; k < H; ++k) {
-    const float2 dl = __fadd2_rn(p[k], make_float2(-dv.centre[2 * k], -dv.centre[2 * k + 1]));
-    s = __ffma2_rn(dl, dl, s);
-    of[2 * k] = -2.0f * dl.x; of[2 * k + 1] = -2.0f * dl.y;
-  }
-  float h = 0.5f * __fadd_rn(s.x, s.y);
-  if (row >= dv.n) {                              // padding rows: never partners; keep them finite
-    h = 0.f;
-#pragma unroll
-    for (int k = 0; k < 2 * H; ++k) of[k] = 0.f;
-  }
-#pragma unroll
-  for (int k = 2 * H; k < Dq; ++k) of[k] = h;
-  float4* out = reinterpret_cast<float4*>(dv.img + (size_t)row * Dq);
-#pragma unroll
-  for (int k = 0; k < Dq / 4; ++k) out[k] = o[k];
-  float m = h;
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, d));
-  if ((threadIdx.x & 31) == 0 && m > 0.f) atomicMax(reinterpret_cast<int*>(dv.hmax + cur), __float_as_int(m));   // m >= 0: integer order = float order
-}
-
-template <int H, int R, int U, int MAXR, int SJ = kStageJ, bool kSeries = false>
-__global__ void __maxnreg__(MAXR) repulse_dot_kernel(RowDev dv, int cur, unsigned epoch) {
-  extern __shared__ float4 smem4[];
-  __shared__ long long item_s;
-  float* sm = reinterpret_cast<float*>(smem4);
-  constexpr int T = kRowTile / R;
-  constexpr int Dp = Row<H>::kStride, Dq = Img<H>::kStride;
-  constexpr int kStageFloats = SJ * Dq;
-  float2* fix_s = reinterpret_cast<float2*>(sm + kStages * kStageFloats);   // [R * H][T], written by the second walk only
-  if (__ldcg(&dv.state->stop)) return;
-  (void)epoch;                                     // image_kernel of this iteration waited for the peers
-  const int tid = threadIdx.x;
-  const float* __restrict__ I = dv.img;
-  const float hmax = __ldcg(dv.hmax + cur);
-  constexpr float kTau = (float)(H + 1) / 8192.0f;
-  const int tiles = dv.rows / kRowTile;
-  const long long items = (long long)tiles * dv.chunks;
-  for (;;) {
-    if (tid == 0) item_s = (long long)atomicAdd(&dv.counters[2], 1u);
-    __syncthreads();
-    const long long item = item_s;
-    if (item >= items) break;
-    const int c = (int)(item / tiles), tile = (int)(item % tiles);
-    const int lrow0 = tile * kRowTile;
-    float2 p[R][H], acc[R][H];
-    float sp[R], thr[R], W[R];
-#pragma unroll
-    for (int r = 0; r < R; ++r) {
-      float2 qt[H], hh;
-      ld_image<H>(I + (size_t)(dv.row0 + lrow0 + tid + r * T) * Dq, qt, hh);
-#pragma unroll
-      for (int k = 0; k < H; ++k) { p[r][k] = make_float2(-0.5f * qt[k].x, -0.5f * qt[k].y); acc[r][k] = make_float2(0.f, 0.f); }
-      sp[r] = 2.0f * hh.x; thr[r] = kTau * (hh.x + hmax); W[r] = 0.f;
-      if constexpr (kSeries) thr[r] = fmaxf(thr[r], kSeriesFloor);
-    }
-    bool fixed = false;
-    const int j0 = c * kChunk;
-    const int cnt = min(kChunk, dv.n - j0);
-    const int nst = (cnt + SJ - 1) / SJ;
-    const float* __restrict__ src = I + (size_t)j0 * Dq;
-    auto prefetch = [&](int s) {
-      if (s < nst) {
-        const float4* g = reinterpret_cast<const float4*>(src + (size_t)s * kStageFloats);
-        float4* d = reinterpret_cast<float4*>(sm + (size_t)(s % kStages) * kStageFloats);
-        for (int x = tid; x < kStageFloats / 4; x += T) cp_async16(d + x, g + x);
-      }
-      cp_async_commit();
-    };
-#pragma unroll
-    for (int s = 0; s < kStages - 1; ++s) prefetch(s);
-    for (int s = 0; s < nst; ++s) {
-      cp_async_wait<kStages - 2>();
-      __syncthreads();
-      prefetch(s + kStages - 1);
-      const float* __restrict__ q_s = sm + (size_t)(s % kStages) * kStageFloats;
-      const int m = min(SJ, cnt - s * SJ);
-      bool flag = false;
-#pragma unroll U
-      for (int j = 0; j < m; ++j) {
-        float2 q[H], hh;
-        ld_image<H>(q_s + j * Dq, q, hh);
-#pragma unroll
-        for (int r = 0; r < R; ++r) flag |= repel_dot<H, kSeries>(p[r], sp[r], thr[r], q, hh, acc[r], W[r]);
-      }
-      if (flag) {                                   // rare: the near pairs of this stage, in the difference form
-        if (!fixed) {
-#pragma unroll
-          for (int x = 0; x < R * H; ++x) fix_s[x * T + tid] = make_float2(0.f, 0.f);
-          fixed = true;
-        }
-        for (int j = 0; j < m; ++j) {
-          float2 q[H], hh;
-          ld_image<H>(q_s + j * Dq, q, hh);
-#pragma unroll
-          for (int r = 0; r < R; ++r) {
-            float d2;
-            if (near_test<H>(p[r], sp[r], thr[r], q, hh, d2)) {
-              const float2 mh = make_float2(-0.5f, -0.5f);
-              float2 s2 = make_float2(0.f, 0.f);
-#pragma unroll
-              for (int k = 0; k < H; ++k) {
-                const float2 dl = __ffma2_rn(q[k], mh, make_float2(-p[r][k].x, -p[r][k].y));   // (q - centre) - (p - centre), exact halving
-                s2 = __ffma2_rn(dl, dl, s2);
-              }
-              const float ds = sqrt_approx(s2.x + s2.y) + 0.01f;
-              const float w = ex2_approx(-3.0f * lg2_approx(ds));
-              const float2 ww = make_float2(w, w);
-#pragma unroll
-              for (int k = 0; k < H; ++k) {
-                const float2 dl = __ffma2_rn(q[k], mh, make_float2(-p[r][k].x, -p[r][k].y));
-                float2* f = fix_s + (r * H + k) * T + tid;
-                *f = __ffma2_rn(dl, ww, *f);
-              }
-            }
-          }
-        }
-      }
-    }
-#pragma unroll
-    for (int r = 0; r < R; ++r) {
-      float2 o[H];
-#pragma unroll
-      for (int k = 0; k < H; ++k) {
-        // sum_j w (q_j - p) = -A / 2 - p W  (A accumulated on q~ = -2 (q - centre))
-        o[k] = make_float2(fmaf(-p[r][k].x, W[r], -0.5f * acc[r][k].x), fmaf(-p[r][k].y, W[r], -0.5f * acc[r][k].y));
-        if (fixed) o[k] = __fadd2_rn(o[k], fix_s[(r * H + k) * T + tid]);
-      }
-      st_point<H>(dv.rpart + ((size_t)c * dv.rows + lrow0 + tid + r * T) * Dp, o);
-    }
-    __syncthreads();   // the stages are refilled by the next item's prologue; item_s is rewritten
-  }
-}
-
-#include "rowblock_tc.cuh"
 #include "rowblock_tc2.cuh"
 
 // ---------------------------------------------------------------------------------------------------
@@ -1040,12 +819,9 @@ struct RowPlan {
   bool peer_ipc[kMaxShards] = {};
   // local
   float* best = nullptr; float* dp1 = nullptr; float* rpart = nullptr; float* xs = nullptr;
-  float* img = nullptr; float* hmax = nullptr;
-  float* tc_buf = nullptr;    // the five arrays of TcImage in one allocation
-  bool tc_form = false;       // distances on the tensor cores (image_tc_kernel + repulse_tc_kernel)
-  bool tc2_form = false;      // distances and accumulation on the tensor cores (+ image_t2_kernel, repulse_tc2_kernel)
+  float* tc_buf = nullptr;    // the arrays of T2Image in one allocation
+  bool tc_form = false;       // distances and accumulation on the tensor cores (image_tc_kernel, image_t2_kernel, repulse_tc2_kernel)
   int tc_cpi = 1;             // partner chunks per work item
-  bool dot_form = false;      // repulsion in the inner-product form (image_kernel + repulse_dot_kernel)
   uint2* recs = nullptr; uint2* mrecs = nullptr;
   unsigned long long* soff = nullptr; unsigned long long* moff = nullptr; int* swidth = nullptr; int* mwidth = nullptr;
   FitState* state = nullptr; double* trace = nullptr; unsigned* counters = nullptr;
@@ -1061,7 +837,7 @@ struct RowPlan {
   int64_t tensor_iters = -1;  // adaptive runs: iterations that ran the tensor form (read back by row_result; -1 = not adaptive / not read yet)
   int rep_ctas = 0;
   double near_limit = 0.0;    // adaptive runs: the tensor form while the probed near-pair fraction is at most this
-  int rep_form = 0;           // shape of the repulsion pass in use (repulse_variant / configure_repulse)
+  int rep_form = 0;           // form of the repulsion pass: 11 (two-GEMM tensor-core pass) or 5 (FP32 difference form)
   bool deep_ring = false;
   bool overlap = true;        // repulsion pass launched as programmatic dependent of the spring walk (TOPOLOW_OVERLAP=0: in order)
   int walk_ctas = 0;          // grid of the spring walk under the repulsion pass
@@ -1077,7 +853,7 @@ struct RowPlan {
     if (stream) cudaStreamSynchronize(stream);
     for (int q = 0; q < kMaxShards; ++q) if (peer_base[q] && peer_ipc[q]) cudaIpcCloseMemHandle(peer_base[q]);
     if (shared) cudaFree(shared);
-    pool_free(best); pool_free(dp1); pool_free(rpart); pool_free(xs); pool_free(img); pool_free(hmax); pool_free(tc_buf); pool_free(recs); pool_free(mrecs);
+    pool_free(best); pool_free(dp1); pool_free(rpart); pool_free(xs); pool_free(tc_buf); pool_free(recs); pool_free(mrecs);
     pool_free(soff); pool_free(moff); pool_free(swidth); pool_free(mwidth);
     pool_free(state); pool_free(trace); pool_free(counters);
     if (h_flag) cudaFreeHost((void*)h_flag);
@@ -1192,35 +968,27 @@ T2Image t2_image(const RowPlan& rp) {
 }
 template <int H>
 void launch_image_tc(RowPlan& rp, cudaStream_t s, int cur, unsigned e_prev) {
-  static_assert(H <= 8, "the tensor forms take ndim <= 16");
+  static_assert(H <= 8, "the tensor form takes ndim <= 16");
   image_tc_kernel<H><<<(unsigned)(rp.dv.cap_rows / kBlockRows), kBlockRows, 0, s>>>(rp.dv, tc_image(rp), cur, e_prev);
-  rp.launches += 1;
-  if (rp.tc2_form) {
-    image_t2_kernel<<<(unsigned)(rp.dv.cap_rows / 4 * 32 / 256), 256, 0, s>>>(rp.dv, t2_image(rp));
-    rp.launches += 1;
-  }
+  image_t2_kernel<<<(unsigned)(rp.dv.cap_rows / 4 * 32 / 256), 256, 0, s>>>(rp.dv, t2_image(rp));
+  rp.launches += 2;
 }
 template <int H>
 void launch_repulse_tc(RowPlan& rp, cudaStream_t s, int cur, bool dependent) {
-  static_assert(H <= 8, "the tensor forms take ndim <= 16");
+  static_assert(H <= 8, "the tensor form takes ndim <= 16");
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)rp.rep_ctas); cfg.blockDim = dim3(kTcThreads);
-  cfg.dynamicSmemBytes = TcSmem::kTotal; cfg.stream = s;
+  cfg.gridDim = dim3((unsigned)rp.rep_ctas); cfg.blockDim = dim3(kT2Threads);
+  cfg.dynamicSmemBytes = T2Smem::kTotal; cfg.stream = s;
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = at; cfg.numAttrs = dependent ? 1 : 0;
-  if (rp.tc2_form) {
-    cfg.blockDim = dim3(kT2Threads); cfg.dynamicSmemBytes = T2Smem::kTotal;
-    TL_CUDA(cudaLaunchKernelEx(&cfg, repulse_tc2_kernel<H>, rp.dv, t2_image(rp), cur, rp.tc_cpi));
-    return;
-  }
-  TL_CUDA(cudaLaunchKernelEx(&cfg, repulse_tc_kernel<H>, rp.dv, tc_image(rp), cur, rp.tc_cpi));
+  TL_CUDA(cudaLaunchKernelEx(&cfg, repulse_tc2_kernel<H>, rp.dv, t2_image(rp), cur, rp.tc_cpi));
 }
 
 template <int H, int kRing> constexpr size_t kWalkSmem = (size_t)(kBlockRows / 32) * Ring<H, kRing>::kWarpBytes;
 
-// The overlap of launch_iteration: two CTAs of the two-GEMM pass and one walk CTA (either ring) share an SM's 233,472 bytes
+// The overlap of launch_pass: two CTAs of the two-GEMM pass and one walk CTA (either ring) share an SM's 233,472 bytes
 // of shared memory.  The system reserves 1 KiB per CTA; kWalkStaticSmem is the walk's static shared memory with that
 // reserve, as cuobjdump -res-usage reports it (tests/test_resource_budget.py checks it and the register caps).
 constexpr size_t kSmPerSm = 233472, kSmReserved = 1024, kWalkStaticSmem = 1152;
@@ -1234,19 +1002,16 @@ void launch_spring(const RowPlan& rp, cudaStream_t s, int cur, unsigned e_spring
 template <int H>
 void launch_mae(const RowPlan& rp, cudaStream_t s, int nxt, unsigned e_spring, unsigned e_mae);
 
-// One iteration of one rank.  overlap: the spring walk runs beside the repulsion pass; otherwise the kernels run one
-// after another.
+// The pass of one rank over positions buffer `cur`: the tensor form's image, the repulsion pass (the FP32 difference form,
+// the tensor form, or both when the device picks per iteration), the spring walk, and combine_kernel, which signals the
+// next epoch.  overlap: the spring walk runs beside the repulsion pass; otherwise the kernels run one after another.
+// ev: null, or events 0..3 of row_time_kernels.
 template <int H>
-void launch_iteration(RowPlan& rp, cudaStream_t s, cudaEvent_t* ev /* 7 events or null */, bool overlap) {
+void launch_pass(RowPlan& rp, cudaStream_t s, int cur, cudaEvent_t* ev, bool overlap) {
   RowDev& dv = rp.dv;
-  const int t = rp.iter_launched;
-  const int cur = t & 1, nxt = cur ^ 1;
-  const bool check = is_check_iter(t, rp.prm), fin = ((t + 1) % 10 == 0);
-  const unsigned e_prev = rp.epoch;          // the epoch every rank reached when iteration t - 1 (and its check) ended
-  const int row_ctas = dv.rows / kBlockRows;
+  const unsigned e_prev = rp.epoch;          // the epoch every rank reached when the iteration before (and its check) ended
   if (ev) TL_CUDA(cudaEventRecord(ev[0], s));
-  if constexpr (H <= 8) {                    // the inner-product and tensor forms exist for ndim <= 16 only
-    if (rp.dot_form) { image_kernel<H><<<dv.slots / kBlockRows, kBlockRows, 0, s>>>(dv, cur, e_prev); rp.launches += 1; }
+  if constexpr (H <= 8) {                    // the tensor form exists for ndim <= 16 only
     if (rp.tc_form) launch_image_tc<H>(rp, s, cur, e_prev);
   }
   if (overlap) {
@@ -1280,11 +1045,22 @@ void launch_iteration(RowPlan& rp, cudaStream_t s, cudaEvent_t* ev /* 7 events o
     launch_spring<H>(rp, s, cur, e_prev, dv.rows / kBlockRows);
     if (ev) TL_CUDA(cudaEventRecord(ev[2], s));
   }
-  const unsigned e_iter = ++rp.epoch;
-  combine_kernel<H><<<row_ctas, kBlockRows, 0, s>>>(dv, rp.prm, cur, e_iter);
+  combine_kernel<H><<<dv.rows / kBlockRows, kBlockRows, 0, s>>>(dv, rp.prm, cur, ++rp.epoch);
   if (ev) TL_CUDA(cudaEventRecord(ev[3], s));
   rp.launches += 3;
+}
+
+// One iteration of one rank: the pass, then on check and finite-check iterations the edge MAE, the controller and the
+// best-state snapshot.
+template <int H>
+void launch_iteration(RowPlan& rp, cudaStream_t s, cudaEvent_t* ev /* 7 events or null */, bool overlap) {
+  RowDev& dv = rp.dv;
+  const int t = rp.iter_launched;
+  const int cur = t & 1, nxt = cur ^ 1;
+  const bool check = is_check_iter(t, rp.prm), fin = ((t + 1) % 10 == 0);
+  launch_pass<H>(rp, s, cur, ev, overlap);
   if (check || fin) {
+    const unsigned e_iter = rp.epoch;
     const unsigned e_mae = ++rp.epoch;
     launch_mae<H>(rp, s, nxt, e_iter, e_mae);
     if (ev) TL_CUDA(cudaEventRecord(ev[4], s));
@@ -1314,106 +1090,45 @@ void launch_one(RowPlan& rp, cudaStream_t s, cudaEvent_t* ev = nullptr) {
   dispatch_h(row_h(rp.dv.D), [&](auto h) { launch_iteration<decltype(h)::value>(rp, s, ev, rp.overlap && !ev); });
 }
 
-// Shapes of the repulsion kernel: {rows per thread, partner unroll, register cap, cube on the SFU}.
-// 0 is the production shape; the others stay selectable (TOPOLOW_REP_VARIANT) for measurements.
-// Variant 0 = policy: 11 (rowblock_tc2.cuh: distances and accumulation on the tensor cores) from ndim 5 on, 5 (the difference
-// form) below; 10 (rowblock_tc.cuh: distances only on the tensor cores) stays selectable.
-// The FP32 inner-product forms (4, 6-9) are kept selectable as the measured record of why they are not used (B200, cfg4 /
-// cfg3 repulsion pass in ms; difference form 16.8 / 0.23, tensor-core form 13.4 / 0.19):
-//   6  one partner per trip, no spill          16.6 / 0.30   issue port 79 % busy (a packed instruction holds it 2 cycles):
-//                                                            two dependency chains per warp cannot hide the MUFU chain
-//   4  two partners per trip, 128 registers    19.1 / 0.31   needs 159 registers; capped, ptxas spills W / sp / thr and shuffles p
-//   7  two partners per trip, 168 registers    18.1 / 0.30   3 warps per scheduler
-//   8  as 6, power by series (1 MUFU)          17.5 / 0.27   +6 FMA-pipe slots cost more than 2 MUFU saved
-//   9  as 4, power by series                   20.9 / 0.26
-// The difference form issues 24 packed + 8.75 other instructions per interaction (56.75 port cycles) and runs at 60.6
-// cycles: it is bound by the issue port, not by the FMA pipe's 51 cycles, and the inner-product form's 49 port cycles only
-// pay with four chains in flight, which do not fit beside 64 registers of own rows and accumulators.
-template <int H>
-void repulse_variant(int v, RepulseFn* fn, int* threads, bool* dot, int* stage) {
-  *dot = false;
-  *stage = kStageJ;
-  *threads = kRowTile / 2;
-  if constexpr (H > 8) {
-    // ndim 17..32: the difference form only, one row per thread (two rows and their accumulators alone are 4 H float2)
-    (void)v;
-    *fn = repulse_kernel<H, 1, kRepUnrollWide, kRepRegsWide, true>;
-    *threads = kRowTile;
-  } else {
-    switch (v) {
-      case 1: *fn = repulse_kernel<H, 2, 2, 128, false>; break;
-      case 2: *fn = repulse_kernel<H, 2, 2, 120, false>; break;
-      case 3: *fn = repulse_kernel<H, 2, 2, 120, true>; break;
-      case 4: *fn = repulse_dot_kernel<H, 2, 2, 128>; *dot = true; break;
-      case 6: *fn = repulse_dot_kernel<H, 2, 1, 128>; *dot = true; break;
-      case 7: *fn = repulse_dot_kernel<H, 2, 2, 168>; *dot = true; break;
-      case 8: *fn = repulse_dot_kernel<H, 2, 1, 128, kStageJ, true>; *dot = true; break;
-      case 9: *fn = repulse_dot_kernel<H, 2, 2, 128, kStageJ, true>; *dot = true; break;
-      default: *fn = repulse_kernel<H, 2, 2, 128, true>; break;
-    }
-  }
-}
+// The form of the repulsion pass.  Policy: 11, the two-GEMM tensor-core pass (rowblock_tc2.cuh), for ndim 5..16 and
+// adaptive (see below); 5, the FP32 difference form (repulse_kernel), below ndim 5 and above 16.  Measured on B200 (ms per
+// repulsion pass, forms 11 / 5): ndim 16, 100k: 7.5 / 16.8; ndim 12, 40k: 1.24 / 2.32; ndim 10, 10k: 0.16 / 0.23; ndim 6,
+// 30k: 0.69 / 0.75.  The two-GEMM form costs the same at every ndim (K is padded to 16 coordinates); the difference form's
+// cost falls with ndim and takes over below ndim 5.  TOPOLOW_REP_VARIANT=5 or 11 runs that form in every iteration.
 template <int H>
 void configure_repulse(RowPlan& rp, int sms) {
   const char* ev = std::getenv("TOPOLOW_REP_VARIANT");
-  RepulseFn fn; int threads;
-  int stage = kStageJ;
-  int variant = ev ? std::atoi(ev) : 0;
-  // policy, measured on B200 (ms per repulsion pass, forms 11 / 10 / 5): ndim 16, 100k: 7.5 / 13.4 / 16.8; ndim 12, 40k: 1.24 / 1.82 /
-  // 2.32; ndim 10, 10k: 0.16 / 0.19 / 0.23; ndim 6, 30k: 0.69 / 0.84 / 0.75.  The two-GEMM form costs the same at every ndim (K is
-  // padded to 16 coordinates); the difference form's cost falls with ndim and takes over below ndim 5.
-  if constexpr (H > 8) {
-    // ndim 17..32: the tensor forms pad K to 16 coordinates and the inner-product forms hold 2 rows per thread; only the
-    // difference form is built, and a form asked for by name that is not it is an error, not a silent substitute
-    if (variant != 0 && variant != 5) throw BadArg("ndim > 16 runs only the FP32 difference form (TOPOLOW_REP_VARIANT=5) in row-block mode");
-    variant = 5;
-  } else if (variant == 0) {
-    variant = H >= 3 ? 11 : 5;
+  int form = (H >= 3 && H <= 8) ? 11 : 5;
+  if (ev) {
+    if (std::strcmp(ev, "5") == 0) form = 5;
+    else if (std::strcmp(ev, "11") == 0) form = 11;
+    else throw BadArg("TOPOLOW_REP_VARIANT takes 5 (FP32 difference form) or 11 (two-GEMM tensor-core form) in row-block mode");
+    // ndim 17..32: the two-GEMM pass pads K to 16 coordinates; only the difference form is built, and asking for the
+    // other form is an error, not a silent substitute
+    if (H > 8 && form != 5) throw BadArg("ndim > 16 runs only the FP32 difference form (TOPOLOW_REP_VARIANT=5) in row-block mode");
   }
-  rp.rep_form = variant;
-  if constexpr (H <= 8) if (variant == 10 || variant == 11) {          // distances (10) / distances and accumulation (11) on the tensor cores
-    rp.tc_form = true;
-    rp.tc2_form = variant == 11;
-    rp.dv.rparts = (rp.tc2_form ? 3 : 2) * rp.dv.chunks;
-    if (rp.tc2_form) {
-      TL_CUDA(cudaFuncSetAttribute(repulse_tc2_kernel<H>, cudaFuncAttributeMaxDynamicSharedMemorySize, T2Smem::kTotal));
-      TL_CUDA(cudaFuncSetAttribute(repulse_tc2_kernel<H>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    }
-    TL_CUDA(cudaFuncSetAttribute(repulse_tc_kernel<H>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem::kTotal));
-    TL_CUDA(cudaFuncSetAttribute(repulse_tc_kernel<H>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    int per_sm = 0;
-    TL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, repulse_tc_kernel<H>, kTcThreads, TcSmem::kTotal));
-    if (std::getenv("TOPOLOW_DEBUG")) {
-      int sm_smem = 0, blk_smem = 0, regs_sm = 0, o0 = 0, o1 = 0, o2 = 0, o3 = 0;
-      cudaDeviceGetAttribute(&sm_smem, cudaDevAttrMaxSharedMemoryPerMultiprocessor, rp.device);
-      cudaDeviceGetAttribute(&blk_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, rp.device);
-      cudaDeviceGetAttribute(&regs_sm, cudaDevAttrMaxRegistersPerMultiprocessor, rp.device);
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o0, repulse_tc_kernel<H>, kTcThreads, 0);
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o1, repulse_tc_kernel<H>, kTcThreads, 65536);
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o2, repulse_tc_kernel<H>, 256, TcSmem::kTotal);
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o3, repulse_tc_kernel<H>, kTcThreads, 90000);
-      cudaFuncAttributes fa;
-      cudaFuncGetAttributes(&fa, repulse_tc_kernel<H>);
-      std::fprintf(stderr, "[topolow] repulse_tc: %d CTAs per SM by the occupancy API at %d bytes (0 B: %d, 64 KB: %d, 90000 B: %d, 256 threads: %d); "
-                   "SM smem %d, block optin %d, regs/SM %d; kernel regs %d static smem %d maxdyn %d carveout %d\n",
-                   per_sm, (int)TcSmem::kTotal, o0, o1, o3, o2, sm_smem, blk_smem, regs_sm, fa.numRegs, (int)fa.sharedSizeBytes,
-                   fa.maxDynamicSharedSizeBytes, fa.preferredShmemCarveout);
-    }
+  rp.rep_form = form;
+  rp.tc_form = form == 11;
+  if constexpr (H <= 8) if (rp.tc_form) {
+    rp.dv.rparts = 3 * rp.dv.chunks;
+    TL_CUDA(cudaFuncSetAttribute(repulse_tc2_kernel<H>, cudaFuncAttributeMaxDynamicSharedMemorySize, T2Smem::kTotal));
+    TL_CUDA(cudaFuncSetAttribute(repulse_tc2_kernel<H>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     // The occupancy API answers 1 for a kernel that allocates tensor memory (it cannot know how many of the 512 columns
     // tcgen05.alloc will ask for); registers, shared memory and the 256 columns a CTA takes all allow two, and the work
     // split does not depend on how many CTAs are resident at once.
-    per_sm = 2;
-    if (const char* ec = std::getenv("TOPOLOW_TC_CTAS")) per_sm = std::max(1, std::atoi(ec));
+    const int per_sm = 2;
     const long long pairs = (long long)(rp.dv.rows / kRowTile) * rp.dv.chunks;
     rp.tc_cpi = (int)std::max<long long>(1, std::min<long long>(rp.dv.chunks, pairs / (6ll * sms * per_sm)));
-    if (const char* ec = std::getenv("TOPOLOW_TC_CPI")) rp.tc_cpi = std::max(1, std::atoi(ec));
     const long long items = (long long)(rp.dv.rows / kRowTile) * ((rp.dv.chunks + rp.tc_cpi - 1) / rp.tc_cpi);
     rp.rep_ctas = (int)std::min<long long>((long long)sms * per_sm, std::max<long long>(items, 1));
-    rp.rep_fn = nullptr;
   }
-  repulse_variant<H>(rp.tc_form ? 5 : variant, &fn, &threads, &rp.dot_form, &stage);
-  const size_t smem = rp.dot_form ? (size_t)kStages * stage * Img<H>::kStride * sizeof(float) + (size_t)2 * H * threads * sizeof(float2)
-                                  : (size_t)kStages * kStageJ * Row<H>::kStride * sizeof(float);
+  // the FP32 difference form: two rows per thread, two partners per trip; ndim 17..32 one row per thread (two rows and
+  // their accumulators alone are 4 H float2)
+  RepulseFn fn;
+  int threads;
+  if constexpr (H <= 8) { fn = repulse_kernel<H, 2, 2, 128>; threads = kRowTile / 2; }
+  else { fn = repulse_kernel<H, 1, kRepUnrollWide, kRepRegsWide>; threads = kRowTile; }
+  const size_t smem = (size_t)kStages * kStageJ * Row<H>::kStride * sizeof(float);
   cudaFuncAttributes fa;
   TL_CUDA(cudaFuncGetAttributes(&fa, (const void*)fn));
   // the static shared memory counts against the same 48 KB default (ndim 32: 48 KB of stages + item_s)
@@ -1421,7 +1136,6 @@ void configure_repulse(RowPlan& rp, int sms) {
   int per_sm = 0;
   TL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, threads, smem));
   if (per_sm < 1) per_sm = 1;
-  if (const char* ec = std::getenv("TOPOLOW_REP_CTAS")) per_sm = std::max(1, std::atoi(ec));
   const long long items = (long long)(rp.dv.rows / kRowTile) * rp.dv.chunks;
   rp.f32_ctas = (int)std::min<long long>((long long)sms * per_sm, std::max<long long>(items, 1));
   rp.f32_smem = smem; rp.f32_threads = threads;
@@ -1445,8 +1159,7 @@ void configure_repulse(RowPlan& rp, int sms) {
   if (const char* eo = std::getenv("TOPOLOW_OVERLAP")) rp.overlap = std::atoi(eo) != 0;
   // spring / MAE walk: the deep ring needs more than the default 48 KB of dynamic shared memory
   rp.deep_ring = rp.dv.rows / kBlockRows <= 2 * sms;
-  rp.walk_ctas = rp.tc2_form ? std::min(rp.dv.rows / kBlockRows, sms) : rp.dv.rows / kBlockRows;
-  if (const char* er = std::getenv("TOPOLOW_DEEP_RING")) rp.deep_ring = std::atoi(er) != 0;
+  rp.walk_ctas = rp.tc_form ? std::min(rp.dv.rows / kBlockRows, sms) : rp.dv.rows / kBlockRows;
   TL_CUDA(cudaFuncSetAttribute(spring_kernel<H, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWalkSmem<H, 8>));
   TL_CUDA(cudaFuncSetAttribute(mae_kernel<H, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWalkSmem<H, 8>));
   if constexpr (kWalkSmem<H, 4> > 48 * 1024) {   // 128-byte ring rows (ndim 17..32): the 4-deep ring needs it too
@@ -1517,8 +1230,6 @@ RowPlan* row_create(const topolow_problem& pb, const topolow_params& pr, int ran
     pool_alloc(rp->rpart, (size_t)(pb.ndim <= 16 ? 3 : 1) * dv.chunks * std::max(dv.rows, 1) * dv.Dp * sizeof(float));   // 3: the two-GEMM form
     pool_alloc(rp->tc_buf, dv.cap_rows * (size_t)(16 + 16 + 4 + 4 + 16 + 32 + 16) * sizeof(float));
     pool_alloc(rp->xs, (size_t)std::max(dv.rows, 1) * dv.Dp * sizeof(float));
-    pool_alloc(rp->img, dv.cap_rows * (size_t)(((dv.D + 1) / 2 * 2 + 2 + 3) / 4 * 4) * sizeof(float));   // Img<H>::kStride floats per row
-    pool_alloc(rp->hmax, 2 * sizeof(float));
     pool_alloc(rp->state, sizeof(FitState));
     pool_alloc(rp->trace, sizeof(double) * std::max(pr.n_iter, 1));
     pool_alloc(rp->counters, 8 * sizeof(unsigned));
@@ -1529,8 +1240,7 @@ RowPlan* row_create(const topolow_problem& pb, const topolow_params& pr, int ran
     std::vector<double> tr(std::max(pr.n_iter, 1), NAN);
     TL_CUDA(cudaMemcpy(rp->trace, tr.data(), tr.size() * sizeof(double), cudaMemcpyHostToDevice));
     TL_CUDA(cudaMemset(rp->counters, 0, 8 * sizeof(unsigned)));
-    TL_CUDA(cudaMemset(rp->hmax, 0, 2 * sizeof(float)));
-    // centre of the inner-product form: the centroid of the initial positions, summed in point order (the same on
+    // centre of the tensor form's image: the centroid of the initial positions, summed in point order (the same on
     // every rank, fixed for the fit; the map stays about where it starts, and a map that wanders only makes more
     // pairs take the difference form)
     for (int d = 0; d < 16; ++d) dv.centre[d] = 0.f;
@@ -1545,7 +1255,7 @@ RowPlan* row_create(const topolow_problem& pb, const topolow_params& pr, int ran
     TL_CUDA(cudaMemcpy(rp->state, &st, sizeof st, cudaMemcpyHostToDevice));
   }
   pt.mark("rows: points");
-  dv.best = rp->best; dv.dp1 = rp->dp1; dv.rpart = rp->rpart; dv.xs = rp->xs; dv.img = rp->img; dv.hmax = rp->hmax;
+  dv.best = rp->best; dv.dp1 = rp->dp1; dv.rpart = rp->rpart; dv.xs = rp->xs;
   dv.state = rp->state; dv.trace = rp->trace;
   dv.counters = rp->counters;
   TL_CUDA(cudaHostAlloc((void**)&rp->h_flag, 2 * sizeof(int), cudaHostAllocMapped));
@@ -1670,22 +1380,8 @@ double row_run_local(RowPlan* const* plans, int n, int n_iters) {
       const bool check = is_check_iter(t, p0.prm), fin = ((t + 1) % 10 == 0);
       for (int a = 0; a < n; ++a) {
         RowPlan& rp = *plans[a];
-        dispatch_h(row_h(rp.dv.D), [&](auto h) {
-          constexpr int H = decltype(h)::value;
-          const unsigned e_prev = rp.epoch;
-          if constexpr (H <= 8) {
-            if (rp.dot_form) { image_kernel<H><<<rp.dv.slots / kBlockRows, kBlockRows, 0, s>>>(rp.dv, cur, e_prev); rp.launches += 1; }
-            if (rp.tc_form) launch_image_tc<H>(rp, s, cur, e_prev);
-          }
-          if (!rp.tc_form || rp.dv.adaptive) {
-            ((RepulseFn)rp.rep_fn)<<<rp.f32_ctas, rp.f32_threads, rp.f32_smem, s>>>(rp.dv, cur, e_prev);
-            rp.launches += rp.dv.adaptive ? 1 : 0;
-          }
-          if constexpr (H <= 8) { if (rp.tc_form) launch_repulse_tc<H>(rp, s, cur, false); }
-          launch_spring<H>(rp, s, cur, e_prev, rp.dv.rows / kBlockRows);
-          combine_kernel<H><<<rp.dv.rows / kBlockRows, kBlockRows, 0, s>>>(rp.dv, rp.prm, cur, ++rp.epoch);
-        });
-        rp.launches += 3; rp.iter_launched = t + 1;
+        dispatch_h(row_h(rp.dv.D), [&](auto h) { launch_pass<decltype(h)::value>(rp, s, cur, nullptr, false); });
+        rp.iter_launched = t + 1;
       }
       if (check || fin) {
         for (int a = 0; a < n; ++a) {

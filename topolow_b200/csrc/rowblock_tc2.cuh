@@ -1,15 +1,32 @@
-// topolow_b200/csrc/rowblock_tc2.cuh - included by rowblock.cu after rowblock_tc.cuh, inside namespace tl::{anonymous}.
+// topolow_b200/csrc/rowblock_tc2.cuh - included by rowblock.cu inside namespace tl::{anonymous}.
 //
-// Repulsion pass with BOTH contractions on the tensor cores - the structure of a fused attention kernel:
-//   GEMM 1   S = d^2 / 2 for 128 rows x 32 partners                    (as in rowblock_tc.cuh: 3-pass TF32, norms in K)
+// Repulsion pass on the 5th-generation tensor cores (tcgen05, accumulators in TMEM), built like a fused attention kernel:
+//   GEMM 1   S = d^2 / 2 for 128 rows x 32 partners
 //   FP32     w = (d + 0.01)^-3 per pair, read from and written back to the same TMEM columns (weights of near pairs 0)
 //   GEMM 2   D2[128 x 32] += w[128 x 32] Y[32 partners x 32]            A operand from TMEM, Y = (x_0..x_15, 1, 0...): columns
 //                                                                       0..15 collect sum_j w x_j, column 16 collects sum_j w
 // and per chunk of 2048 partners the rows' sums come out as D2[0..15] - x_i D2[16].  The FP32 pipes are left with 7.6
 // instructions per pair - one of them on the special-function unit when the weights can be computed by the series form
-// (all pairs of the batch farther apart than 0.1; image_tc_kernel's probe decides per iteration, rowblock_tc.cuh), two
-// (square root, reciprocal) otherwise.  Measured at cfg4 (ncu): 5.7 ms per pass, 75 % of the issue slots, FMA pipe 40 %,
+// (all pairs of the batch farther apart than 0.1; image_tc_kernel's probe decides per iteration), two (square root,
+// reciprocal) otherwise.  Measured at cfg4 (ncu): 5.7 ms per pass, 75 % of the issue slots, FMA pipe 40 %,
 // special-function unit 45 %, tensor-core unit 40 %.
+//
+// GEMM 1: d^2 / 2 = |p|^2 / 2 + |q|^2 / 2 - p.q for a block of (own row, partner) pairs is ONE small GEMM, -A B^T with K = 16
+// coordinates (zero padded) + 4 columns that add the two half norms (A: -h_i, -h_i', -1, -1; B: 1, 1, h_j, h_j') + 4 zeros,
+// in TF32 with the 3-pass split that keeps FP32 accuracy (x = hi + lo, hi = x rounded to TF32: hi.hi + hi.lo + lo.hi;
+// lo.lo is below 2^-22).
+//
+// Pairs whose inner-product distance cannot be trusted get weight 0 and are re-done from the coordinate differences (the
+// point itself, difference exactly 0, contributes nothing, as in the difference form).  The error of d^2 / 2 is about
+// 7e-7 (h_i + h_j), h = |x|^2 / 2; "near" means d^2 / 2 < tau (h_i + h_j) with tau = 1e-3 (relative error of d^2 could
+// pass 1e-3).  A near partner has |x_j| <= |x_i| + d, hence h_j <= 2 h_i + d^2, and the test d^2 / 2 < 3.01 tau h_i - a
+// per-row constant - catches every such pair whatever the rest of the map looks like.  In 16 dimensions that is the point
+// itself and hardly anything else.
+//
+// Operand layout (K-major, no swizzle; in 16-byte units ((8, n), 2) : ((1, SBO), LBO)): "chunk planes" - for every group of
+// four consecutive K values one plane [rows][4 floats]; SBO = 128 bytes (8 rows), LBO = rows x 16 bytes (next plane).
+// image_tc_kernel writes the planes for ALL points once per iteration, so a stage or an A tile is a handful of
+// contiguous copies.
 //
 // Precision of GEMM 2: w is used as TF32 (truncated by the tensor core) consistently in the sums of w x_j and of w, so
 // the difference D2[0..15] - x_i D2[16] still telescopes.  The partner coordinates enter rounded to TF32 (2^-11 relative:
@@ -28,11 +45,165 @@
 // 4 KB of shared memory each (the tensor pipe's operand fetch was its busiest part: 57 % of the cycles, and the consumers
 // waited a fifth of their time for distances).
 
+constexpr int kTcRows = 256;         // own rows per work item = two M = 128 tiles (= kRowTile)
+constexpr unsigned kTcSpinLimit = 1u << 28;
 constexpr int kT2SJ = 32;            // partners per stage
 constexpr int kT2Stages = 4;
 constexpr int kT2Threads = 320;       // 8 consumer warps + the MMA warp + the copy warp
-constexpr float kT2SeriesS = 0.005f;   // series form of the weight: pairs closer than 0.1 (d^2 / 2 < 0.005) are near pairs
-constexpr bool kT2LoPass = false;     // second pass of GEMM 2 over the TF32 remainders of the partner coordinates (see below)
+constexpr float kSeriesNearS = 0.005f;   // series form of the weight: pairs closer than 0.1 (d^2 / 2 < 0.005) are near pairs
+constexpr bool kT2LoPass = false;     // second pass of GEMM 2 over the TF32 remainders of the partner coordinates (see above)
+
+// ---- PTX wrappers -----------------------------------------------------------------------------------
+TL_D unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
+TL_D void mbar_init(unsigned bar, unsigned count) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory"); }
+TL_D void mbar_arrive(unsigned bar) { asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory"); }
+TL_D void mbar_expect_tx(unsigned bar, unsigned bytes) {
+  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
+}
+// Every calling thread polls.  A wait that does not end is a protocol bug: trap (the launch fails) instead of hanging the device.
+TL_D void mbar_wait(unsigned bar, unsigned parity) {
+  unsigned done = 0;
+  for (unsigned spin = 0; !done; ++spin) {
+    asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
+                 : "=r"(done) : "r"(bar), "r"(parity) : "memory");
+    if (spin > kTcSpinLimit) __trap();
+  }
+}
+TL_D void bulk_g2s(unsigned dst, const void* src, unsigned bytes, unsigned bar) {
+  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+               ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
+}
+TL_D void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
+TL_D void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+TL_D void tc_commit(unsigned bar) {
+  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
+}
+TL_D void tc_mma_tf32(unsigned d_tmem, unsigned long long a_desc, unsigned long long b_desc, unsigned idesc, unsigned accumulate) {
+  asm volatile("{ .reg .pred p; setp.ne.b32 p, %4, 0; tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p; }"
+               ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
+}
+TL_D void tc_ld8(unsigned taddr, unsigned (&v)[8]) {
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+               : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
+               : "r"(taddr) : "memory");
+}
+TL_D unsigned tc_ld1(unsigned taddr) {
+  unsigned v;
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x1.b32 {%0}, [%1];" : "=r"(v) : "r"(taddr) : "memory");
+  return v;
+}
+TL_D void tc_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+
+// Shared-memory matrix descriptor, K-major, no swizzle (cute::UMMA::SmemDescriptor: start >> 4 in bits [0,14), leading
+// byte offset >> 4 in [16,30), stride byte offset >> 4 in [32,46), version 1 in [46,48), layout type 0 in [61,64)).
+TL_D unsigned long long tc_desc(unsigned smem_addr, unsigned lbo_bytes, unsigned sbo_bytes) {
+  return (unsigned long long)((smem_addr >> 4) & 0x3fffu) | ((unsigned long long)((lbo_bytes >> 4) & 0x3fffu) << 16) |
+         ((unsigned long long)((sbo_bytes >> 4) & 0x3fffu) << 32) | (1ull << 46);
+}
+TL_D float tf32_round(float x) { unsigned r; asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x)); return __uint_as_float(r); }
+
+// ---- the image: chunk planes of hi / lo, the norm columns, FP32 rows ---------------------------------
+struct TcImage {
+  float* xhi;     // [4][cap_rows][4]  coordinates - centre, rounded to TF32
+  float* xlo;     // [4][cap_rows][4]  the remainder
+  float* aug_a;   // [cap_rows][4]     (-h_hi, -h_lo, -1, -1)     h = |x|^2 / 2
+  float* aug_b;   // [cap_rows][4]     (1, 1, h_hi, h_lo); padding rows: h = 1e30 (their weight underflows to 0)
+  float* rows32;  // [cap_rows][16]    coordinates - centre, FP32
+};
+
+template <int H>
+__global__ void __launch_bounds__(kBlockRows) image_tc_kernel(RowDev dv, TcImage im, int cur, unsigned epoch) {
+  constexpr int Dp = Row<H>::kStride;
+  if (__ldcg(&dv.state->stop)) return;
+  if (!wait_epoch(dv, epoch)) { if (blockIdx.x == 0 && threadIdx.x == 0) peer_timeout(dv); return; }
+  const size_t row = (size_t)blockIdx.x * kBlockRows + threadIdx.x;     // grid covers cap_rows
+  float x[16];
+#pragma unroll
+  for (int k = 0; k < 16; ++k) x[k] = 0.f;
+  const bool real = row < (size_t)dv.n;
+  if (real) {
+    float2 p[H];
+    ld_point<H>(dv.pos[dv.rank] + ((size_t)cur * dv.cap_rows + row) * Dp, p);
+#pragma unroll
+    for (int k = 0; k < H; ++k) { x[2 * k] = p[k].x - dv.centre[2 * k]; x[2 * k + 1] = p[k].y - dv.centre[2 * k + 1]; }
+  }
+  float h = 0.f;
+#pragma unroll
+  for (int k = 0; k < 16; ++k) h = fmaf(x[k], x[k], h);
+  h *= 0.5f;
+#pragma unroll
+  for (int c = 0; c < 4; ++c) {
+    float4 hi, lo;
+    hi.x = tf32_round(x[4 * c]); hi.y = tf32_round(x[4 * c + 1]); hi.z = tf32_round(x[4 * c + 2]); hi.w = tf32_round(x[4 * c + 3]);
+    lo.x = x[4 * c] - hi.x; lo.y = x[4 * c + 1] - hi.y; lo.z = x[4 * c + 2] - hi.z; lo.w = x[4 * c + 3] - hi.w;
+    reinterpret_cast<float4*>(im.xhi)[(size_t)c * dv.cap_rows + row] = hi;
+    reinterpret_cast<float4*>(im.xlo)[(size_t)c * dv.cap_rows + row] = lo;
+    reinterpret_cast<float4*>(im.rows32)[row * 4 + c] = make_float4(x[4 * c], x[4 * c + 1], x[4 * c + 2], x[4 * c + 3]);
+  }
+  const float hb = real ? h : 1e30f;
+  const float h_hi = tf32_round(h), hb_hi = tf32_round(hb);
+  reinterpret_cast<float4*>(im.aug_a)[row] = make_float4(-h_hi, -(h - h_hi), -1.f, -1.f);
+  reinterpret_cast<float4*>(im.aug_b)[row] = make_float4(1.f, 1.f, hb_hi, hb - hb_hi);
+  if (dv.adaptive) {
+    // ---- which form runs this iteration ----
+    // The tensor form re-does every pair whose distance is small against the point's distance from the centre (the
+    // cancellation in |x|^2 / 2 + |y|^2 / 2 - x.y) in the difference form, one divergent call each: cheap in a map that has
+    // spread out, ruinous in the first iterations of the reference's start (R/core.R:407-415: cumulative steps along the
+    // diagonal, 3 % of all pairs are near: 136 ms instead of 7.5 at cfg4).  Every row tests a few pseudo-random partners
+    // against the same criterion; the count is a function of the replica alone, so every rank of a sharded map decides
+    // the same way and the result still does not depend on the rank count.
+    unsigned near = 0;
+    if (real) {
+      const unsigned it = (unsigned)__ldcg(&dv.state->iter);
+      for (int k = 0; k < dv.probe_k; ++k) {
+        unsigned long long z = ((unsigned long long)row * 64ull + (unsigned long long)k) * 0x9E3779B97F4A7C15ull + (unsigned long long)it * 0xD1B54A32D192ED03ull + dv.seed;
+        z ^= z >> 30; z *= 0xBF58476D1CE4E5B9ull; z ^= z >> 27; z *= 0x94D049BB133111EBull; z ^= z >> 31;
+        const size_t j = (size_t)(z % (unsigned long long)dv.n);
+        if (j == row) continue;
+        float2 q[H];
+        ld_point<H>(dv.pos[dv.rank] + ((size_t)cur * dv.cap_rows + j) * Dp, q);
+        float d2 = 0.f;
+#pragma unroll
+        for (int c = 0; c < H; ++c) {
+          const float dx = q[c].x - dv.centre[2 * c] - x[2 * c], dy = q[c].y - dv.centre[2 * c + 1] - x[2 * c + 1];
+          d2 = fmaf(dx, dx, d2); d2 = fmaf(dy, dy, d2);
+        }
+        near += (0.5f * d2 < 3.01e-3f * h_hi) ? 1u : 0u;
+        near += (0.5f * d2 < fmaxf(3.01e-3f * h_hi, kSeriesNearS)) ? 0x10000u : 0u;   // near in the series form of the weights
+      }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) near += __shfl_xor_sync(0xffffffffu, near, o);     // <= 64 x 32 per half: no carry
+    if ((threadIdx.x & 31) == 0 && near) {
+      if (near & 0xffffu) atomicAdd(&dv.counters[4], near & 0xffffu);
+      atomicAdd(&dv.counters[3], near >> 16);
+    }
+    if (last_cta(&dv.counters[5]) && threadIdx.x == 0) {
+      const unsigned found = atomicExch(&dv.counters[4], 0u), found_series = atomicExch(&dv.counters[3], 0u);
+      // 2: tensor form, weights by the one-MUFU series; 1: tensor form, square root + reciprocal; 0: FP32 difference form
+      const unsigned form = (dv.series && found_series <= dv.probe_limit) ? 2u : (found <= dv.probe_limit ? 1u : 0u);
+      dv.counters[6] = form;
+      dv.counters[7] += form ? 1u : 0u;
+      __threadfence();
+    }
+  }
+}
+
+// A near pair, from the coordinate differences (the arithmetic of repulse_kernel).  Out of line and on accumulators in
+// local memory: it must not cost the main loop registers, and it is rare in a map that has spread out (the point
+// itself, once per row and iteration) but not in the first iterations of a tightly packed start.
+template <int H>
+__device__ __noinline__ void near_fix(const float* __restrict__ xi, const float* __restrict__ xj, float* __restrict__ facc) {
+  float d2 = 0.f;
+#pragma unroll
+  for (int k = 0; k < 2 * H; ++k) { const float dl = xj[k] - __ldg(xi + k); d2 = fmaf(dl, dl, d2); }
+  if (d2 > 0.f) {                                 // the point itself (and exact duplicates) contribute nothing
+    const float ds = sqrt_approx(d2) + 0.01f;
+    const float w = ex2_approx(-3.0f * lg2_approx(ds));
+#pragma unroll
+    for (int k = 0; k < 2 * H; ++k) facc[k] = fmaf(xj[k] - __ldg(xi + k), w, facc[k]);
+  }
+}
 
 // The only A operand GEMM 1 reads from shared memory is the remainders of tile 1 (tile 0's and both tiles' -A_hi and norm
 // columns are in tensor memory): 4 planes x 128 rows x 16 B.  At 61.6 KB per CTA two CTAs leave room on the SM for a
@@ -55,7 +226,7 @@ struct T2Smem {
 };
 
 struct T2Image {
-  TcImage a;      // the arrays of the one-GEMM form
+  TcImage a;      // the arrays image_tc_kernel writes
   float* yhi;     // [cap_rows / 4][32][4]   row n of a partner quad: n < 16 coordinate n (TF32-rounded), n = 16: 1, else 0
   float* ylo;     // [cap_rows / 4][16][4]   the remainders of the coordinates
 };
@@ -361,7 +532,7 @@ __global__ void __maxnreg__(80) repulse_tc2_kernel(RowDev dv, T2Image im, int cu
 #pragma unroll
       for (int r = 0; r < 2; ++r) {
         thr[r] = -3.01e-3f * __ldg(im.a.aug_a + (size_t)(dv.row0 + lrow[r]) * 4);
-        if (series) thr[r] = fmaxf(thr[r], kT2SeriesS);
+        if (series) thr[r] = fmaxf(thr[r], kSeriesNearS);
       }
       for (int c = c_lo; c < c_hi; ++c, ++chunk_g) {
         float facc[32];

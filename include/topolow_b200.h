@@ -256,10 +256,11 @@ TOPOLOW_API int topolow_shard_run_local(topolow_shard* const* shards, int32_t n,
 TOPOLOW_API int topolow_shard_time_kernels(topolow_shard* shard, int32_t n_iters, double* out, int32_t cap);
 TOPOLOW_API int topolow_shard_result(topolow_shard* shard, topolow_result* result);
 /* out (up to 18 values): {slots, ndim, stride, n_ranks, rank, row0, own_rows, partner_chunks, spring_records,
- * mae_records, kernel_launches, iterations_done, stopped, peer_store_bytes_per_iteration, repulsion_items,
- * repulsion_ctas, repulsion_form (5: FP32 difference form, 10: distances on tcgen05, 11: distances and accumulation on
- * tcgen05), tensor_form_iterations (forms 10 / 11 chosen by policy run adaptively: the device picks the form of every
- * iteration; the count is read back by topolow_shard_result, -1 before that or when the form is not adaptive)}. */
+ * mae_records, kernel_launches, iterations_done, stopped, peer_store_bytes_per_iteration, repulsion_items (work items
+ * of one pass of repulsion_form: 256 own rows x one chunk of 2048 partners in form 5, x a group of chunks in form 11),
+ * repulsion_ctas, repulsion_form (5: FP32 difference form, 11: distances and accumulation on tcgen05),
+ * tensor_form_iterations (form 11 chosen by the policy runs adaptively: the device picks the form of every iteration;
+ * the count is read back by topolow_shard_result, -1 before that or when the form is not adaptive)}. */
 TOPOLOW_API int topolow_shard_info(const topolow_shard* shard, int64_t* out, int32_t cap);
 /* slot_of_point of the row-block layout (a pure function of n). */
 TOPOLOW_API int topolow_shard_slot_order(int64_t n, int32_t* slot_of_point_out);

@@ -618,51 +618,29 @@ def test_tensor_form_arithmetic_emulated_in_numpy():
     differences, weights by rsqrt + cubic and truncated to TF32, sums of w x_j (x_j rounded to TF32) and of w, force =
     sum w x_j - x_i sum w.  Bars: every far pair's S within 2.5e-4 of d^2 / 2, every weight within 1.5e-3 of
     (d + 0.01)^-3, a row's repulsion sum within 1e-3 of the FP64 sum relative to its length (median 4e-4)."""
-    def tf32_rna(x):                     # cvt.rna.tf32.f32: 10 explicit mantissa bits, ties away from zero
-        u = np.asarray(x, np.float32).view(np.uint32).astype(np.uint64)
-        return (((u + 0x1000) & 0xFFFFE000) & 0xFFFFFFFF).astype(np.uint32).view(np.float32)
-
-    def tf32_trunc(x):                   # what the tensor core does to an FP32 operand
-        return (np.asarray(x, np.float32).view(np.uint32) & np.uint32(0xFFFFE000)).view(np.float32)
-
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import tc2_arith_model as model
     rng = np.random.default_rng(11)
     n, d = 1200, 16
     centres = rng.normal(size=(4, d)) * 4
     X = (centres[rng.integers(0, 4, n)] + rng.normal(size=(n, d)) + np.linspace(0, 6, n)[:, None] * rng.normal(size=d) / 4).astype(np.float32)
     X = X + np.float32(30.0)             # far from the origin: the kernel works on coordinates minus the centre
-    centre = X.astype(np.float64).mean(0).astype(np.float32)
-    x = (X - centre).astype(np.float32)
-    hi = tf32_rna(x); lo = tf32_trunc(x - hi)
-    h = (0.5 * (x.astype(np.float64) ** 2).sum(1)).astype(np.float32)
-    h_hi = tf32_rna(h); h_lo = tf32_trunc(h - h_hi)
-    hi64, lo64 = hi.astype(np.float64), lo.astype(np.float64)
-    dot = hi64 @ hi64.T + hi64 @ lo64.T + lo64 @ hi64.T
-    hh = (h_hi.astype(np.float64) + h_lo.astype(np.float64))
-    S = (hh[:, None] + hh[None, :] - dot).astype(np.float32)
+    x, xp, _ = model.image(X)
+    S, h_hi = model.distances(x, xp)
     x64 = X.astype(np.float64)
     diff = x64[None, :, :] - x64[:, None, :]                    # x_j - x_i
     d2 = (diff ** 2).sum(2)
     dist = np.sqrt(d2)
     off = ~np.eye(n, dtype=bool)
-    near = (S < np.float32(3.01e-3) * h_hi[:, None]) | (S < np.float32(0.005))
+    near = model.near_mask(S, h_hi, series=True)
     far = off & ~near
     assert far.sum() > 0.99 * off.sum()                         # a spread-out map: near pairs are rare
     assert np.abs(S[far] / (0.5 * d2[far]) - 1).max() < 2.5e-4
-    q = (1.0 / np.sqrt(np.abs(S.astype(np.float64)) + 1e-300)).astype(np.float32)
-    pl = np.float32(-9.3722616e-07) * q + np.float32(1.0345994e-4)
-    pl = pl * q + np.float32(-7.492801e-3)
-    pl = pl * q + np.float32(0.35355023)
-    w = tf32_trunc((q * q * q * pl).astype(np.float32)).astype(np.float64)
+    w = model.weights(S, series=True)
     want_w = (dist + 0.01) ** -3
     assert np.abs(w[far] / want_w[far] - 1).max() < 1.5e-3
-    w[~far] = 0.0
-    y = tf32_rna(x).astype(np.float64)
-    sum_wx = (w @ y).astype(np.float32).astype(np.float64)
-    sum_w = w.sum(1).astype(np.float32).astype(np.float64)
-    force = sum_wx - x.astype(np.float64) * sum_w[:, None]
-    # near pairs: FP32 differences, exactly the FP32 form's arithmetic (here in FP64: they are not what is being tested)
-    wn = np.where(near & off, want_w, 0.0)
-    force += (wn[:, :, None] * diff).sum(1)
+    # near pairs: FP32 differences, exactly the FP32 form's arithmetic (in FP64 in the model: they are not what is being tested)
+    force = model.tensor_pass(X, series=True)
     want = (np.where(off, want_w, 0.0)[:, :, None] * diff).sum(1)
     rel = np.linalg.norm(force - want, axis=1) / np.linalg.norm(want, axis=1)
     assert np.median(rel) < 4e-4 and rel.max() < 1e-3, (np.median(rel), rel.max())

@@ -836,6 +836,7 @@ struct RowPlan {
   int64_t n_recs = 0, n_mrecs = 0;
   int64_t tensor_iters = -1;  // adaptive runs: iterations that ran the tensor form (read back by row_result; -1 = not adaptive / not read yet)
   int rep_ctas = 0;
+  int64_t rep_items = 0;      // work items of one pass of the form rep_form names (the tensor form groups tc_cpi chunks per item)
   double near_limit = 0.0;    // adaptive runs: the tensor form while the probed near-pair fraction is at most this
   int rep_form = 0;           // form of the repulsion pass: 11 (two-GEMM tensor-core pass) or 5 (FP32 difference form)
   bool deep_ring = false;
@@ -1121,6 +1122,7 @@ void configure_repulse(RowPlan& rp, int sms) {
     rp.tc_cpi = (int)std::max<long long>(1, std::min<long long>(rp.dv.chunks, pairs / (6ll * sms * per_sm)));
     const long long items = (long long)(rp.dv.rows / kRowTile) * ((rp.dv.chunks + rp.tc_cpi - 1) / rp.tc_cpi);
     rp.rep_ctas = (int)std::min<long long>((long long)sms * per_sm, std::max<long long>(items, 1));
+    rp.rep_items = items;
   }
   // the FP32 difference form: two rows per thread, two partners per trip; ndim 17..32 one row per thread (two rows and
   // their accumulators alone are 4 H float2)
@@ -1140,7 +1142,7 @@ void configure_repulse(RowPlan& rp, int sms) {
   rp.f32_ctas = (int)std::min<long long>((long long)sms * per_sm, std::max<long long>(items, 1));
   rp.f32_smem = smem; rp.f32_threads = threads;
   rp.rep_fn = (void*)fn;
-  if (!rp.tc_form) rp.rep_ctas = rp.f32_ctas;
+  if (!rp.tc_form) { rp.rep_ctas = rp.f32_ctas; rp.rep_items = items; }
   // The policy's tensor form is adaptive: the device picks the form of every iteration (image_tc_kernel's probe) and
   // the host launches both kernels.  A form asked for by name (TOPOLOW_REP_VARIANT) runs unconditionally.
   rp.dv.adaptive = (rp.tc_form && !ev) ? 1 : 0;
@@ -1513,7 +1515,7 @@ void row_info(const RowPlan& rp, int64_t* out, int cap) {
   const int64_t v[18] = {dv.slots, dv.D, dv.Dp, dv.G, dv.rank, dv.row0, dv.rows, dv.chunks, rp.n_recs, rp.n_mrecs, rp.launches,
                          rp.h_flag ? rp.h_flag[1] : 0, rp.h_flag ? rp.h_flag[0] : 0,
                          (int64_t)(dv.G - 1) * dv.rows * dv.Dp * 4,   // position bytes this rank stores into its peers per iteration
-                         (int64_t)(dv.rows / kRowTile) * dv.chunks, rp.rep_ctas, rp.rep_form, rp.tensor_iters};
+                         rp.rep_items, rp.rep_ctas, rp.rep_form, rp.tensor_iters};
   for (int i = 0; i < cap && i < 18; ++i) out[i] = v[i];
 }
 

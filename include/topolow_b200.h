@@ -188,6 +188,32 @@ TOPOLOW_API int topolow_fit_batch_interruptible(int32_t n_jobs, const topolow_pr
                                                 const topolow_params* params, topolow_result* results, int32_t device,
                                                 topolow_interrupt_fn poll, void* user);
 
+/* The same batch spread over several GPUs from one process (R runs in one process, and a forked child cannot use a
+ * CUDA context its parent holds).  `devices` holds n_devices >= 1 CUDA ordinals; one host thread runs the share of
+ * each entry.  An ordinal may repeat: its shares then run on the same device from separate host threads (how one GPU
+ * runs this path).
+ *   - Results: every job's result (positions, MAE, k, iterations, iterations_run, pair_updates, hold-out sums,
+ *     trace, status, message) is bit for bit what topolow_fit_batch_interruptible(..., devices[0], ...) returns for
+ *     the same arrays, whatever the list.  The one-CTA rule above (16 or more jobs) is taken on n_jobs of the whole
+ *     call, never on one share.  params[j].device is ignored.
+ *   - Arguments: a null `devices`, n_devices < 1 or an ordinal outside [0, cudaGetDeviceCount()) returns
+ *     TOPOLOW_ERR_BAD_ARG before anything is allocated, with the reason in results[0].message when n_jobs > 0
+ *     (TOPOLOW_ERR_CUDA when the device count cannot be read).  n_devices == 1 is
+ *     topolow_fit_batch_interruptible on devices[0].
+ *   - Placement: jobs are dealt longest first by n(n-1)/2 x n_iter to the entry with the least work so far; ties go
+ *     to the lower job index, then to the lower list position.  The placement is a pure function of the inputs.
+ *     Jobs that share edge arrays share one set of device records per device.
+ *   - Interrupt: `poll` is called from the calling thread only (never from a worker thread): once before set-up,
+ *     once after the set-up of every share and before the first launch on any device, then at least every 100 ms
+ *     while any fit on any device runs.  When it fires, the abort word of every share is raised, no device issues
+ *     another launch, and every result is filled in by the rules of topolow_fit_batch_interruptible.
+ *   - Errors: a CUDA error in one share marks that share's jobs TOPOLOW_ERR_CUDA and the call returns
+ *     TOPOLOW_ERR_CUDA (also when the batch was interrupted); jobs of the other shares keep their full results.
+ *     Everything allocated on every device, and every mapped host block, is released before the call returns. */
+TOPOLOW_API int topolow_fit_batch_devices(int32_t n_jobs, const topolow_problem* problems, const topolow_params* params,
+                                          topolow_result* results, const int32_t* devices, int32_t n_devices,
+                                          topolow_interrupt_fn poll, void* user);
+
 /* ---- device-resident plan ----------------------------------------------- */
 typedef struct topolow_plan topolow_plan;
 

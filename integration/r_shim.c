@@ -99,11 +99,20 @@ SEXP _topolow_optimize_layout_b200(SEXP init, SEXP dmat, SEXP tmat, SEXP degrees
  * positions (only when keep_positions)}: a failed fit is a status + message, never an R error
  * (R/adaptive_sampling.R:2657-2666 turns failures into NA rows).  Ctrl-C stops the batch as it stops a single fit: the
  * library is polled while the fits run, stops them, releases what it holds and returns TOPOLOW_ERR_INTERRUPTED, and
- * the R condition is raised from this frame. */
+ * the R condition is raised from this frame.
+ * `device` is one CUDA ordinal, or an integer or double vector of them (e.g. 0:7): the batch is then dealt over those
+ * GPUs from this one process (topolow_fit_batch_devices), with the same results as on the first of them. */
 SEXP _topolow_fit_batch_b200(SEXP jobs, SEXP keep_positions, SEXP device) {
   if (TYPEOF(jobs) != VECSXP) Rf_error("jobs must be a list");
   const R_xlen_t nj = XLENGTH(jobs);
-  const int keep = Rf_asLogical(keep_positions) == TRUE, dev = Rf_asInteger(device);
+  const int keep = Rf_asLogical(keep_positions) == TRUE;
+  const R_xlen_t n_dev = XLENGTH(device);
+  if (n_dev < 1) Rf_error("device must name at least one CUDA ordinal");
+  if (n_dev > 1024) Rf_error("device: too many ordinals");   /* (the count crosses the C ABI as int32) */
+  SEXP dev_int = PROTECT(Rf_coerceVector(device, INTSXP));   /* (device itself when it is already integer) */
+  for (R_xlen_t i = 0; i < n_dev; ++i)
+    if (INTEGER(dev_int)[i] == NA_INTEGER) { UNPROTECT(1); Rf_error("device must not be NA"); }
+  const int dev = INTEGER(dev_int)[0];
   topolow_problem* pb = (topolow_problem*)R_alloc((size_t)(nj > 0 ? nj : 1), sizeof(topolow_problem));   /* freed by R at .Call exit */
   topolow_params* pr = (topolow_params*)R_alloc((size_t)(nj > 0 ? nj : 1), sizeof(topolow_params));
   topolow_result* rs = (topolow_result*)R_alloc((size_t)(nj > 0 ? nj : 1), sizeof(topolow_result));
@@ -141,9 +150,11 @@ SEXP _topolow_fit_batch_b200(SEXP jobs, SEXP keep_positions, SEXP device) {
     SET_VECTOR_ELT(res, 8, pos);
     rs[j].positions = keep ? REAL(pos) : NULL;
   }
-  const int rc = topolow_fit_batch_interruptible((int32_t)nj, pb, pr, rs, dev, poll_interrupt, NULL);
-  if (rc == TOPOLOW_ERR_INTERRUPTED) { UNPROTECT(1); Rf_onintr(); Rf_error("interrupted"); }   /* the library has unwound */
-  if (rc != TOPOLOW_OK) { UNPROTECT(1); Rf_error("topolow_fit_batch failed with status %d%s%s", rc, nj > 0 ? ": " : "", nj > 0 ? rs[0].message : ""); }
+  const int rc = n_dev == 1 ? topolow_fit_batch_interruptible((int32_t)nj, pb, pr, rs, dev, poll_interrupt, NULL)
+                            : topolow_fit_batch_devices((int32_t)nj, pb, pr, rs, INTEGER(dev_int), (int32_t)n_dev,
+                                                        poll_interrupt, NULL);
+  if (rc == TOPOLOW_ERR_INTERRUPTED) { UNPROTECT(2); Rf_onintr(); Rf_error("interrupted"); }   /* the library has unwound */
+  if (rc != TOPOLOW_OK) { UNPROTECT(2); Rf_error("topolow_fit_batch failed with status %d%s%s", rc, nj > 0 ? ": " : "", nj > 0 ? rs[0].message : ""); }
   for (R_xlen_t j = 0; j < nj; ++j) {
     SEXP res = VECTOR_ELT(out, j);
     SET_VECTOR_ELT(res, 0, Rf_ScalarLogical(rs[j].converged));
@@ -155,7 +166,7 @@ SEXP _topolow_fit_batch_b200(SEXP jobs, SEXP keep_positions, SEXP device) {
     SET_VECTOR_ELT(res, 6, Rf_ScalarInteger(rs[j].status));
     SET_VECTOR_ELT(res, 7, Rf_mkString(rs[j].message));
   }
-  UNPROTECT(1);
+  UNPROTECT(2);
   return out;
 }
 

@@ -12,6 +12,7 @@ typedef enum { FALSE = 0, TRUE = 1 } Rboolean;
 typedef struct SEXPREC* SEXP;
 enum { NILSXP = 0, SYMSXP = 1, CHARSXP = 9, LGLSXP = 10, INTSXP = 13, REALSXP = 14, STRSXP = 16, VECSXP = 19 };
 extern SEXP R_NilValue;
+#define NA_INTEGER (-2147483647 - 1)   /* R_NaInt */
 int TYPEOF(SEXP x);
 R_xlen_t XLENGTH(SEXP x);
 int Rf_nrows(SEXP x);
@@ -26,6 +27,7 @@ SEXP SET_VECTOR_ELT(SEXP x, R_xlen_t i, SEXP v);
 int Rf_asInteger(SEXP x);
 int Rf_asLogical(SEXP x);
 double Rf_asReal(SEXP x);
+SEXP Rf_coerceVector(SEXP x, unsigned type);
 SEXP Rf_allocVector(unsigned type, R_xlen_t n);
 SEXP Rf_allocMatrix(unsigned type, int nrow, int ncol);
 SEXP Rf_mkNamed(unsigned type, const char** names);

@@ -67,3 +67,20 @@ int topolow_fit_batch_interruptible(int32_t n_jobs, const topolow_problem* pb, c
     }
   return topolow_fit_batch(n_jobs, pb, pr, rs, device);
 }
+
+/* Records the device list it was handed at the end of the first job's message (" devices=0,0"); polls and answers
+ * as topolow_fit_batch_interruptible does. */
+int topolow_fit_batch_devices(int32_t n_jobs, const topolow_problem* pb, const topolow_params* pr, topolow_result* rs,
+                              const int32_t* devices, int32_t n_devices, topolow_interrupt_fn poll, void* user) {
+  if (!devices || n_devices < 1) return TOPOLOW_ERR_BAD_ARG;
+  for (int32_t i = 0; i < n_devices; ++i)
+    if (devices[i] < 0) return TOPOLOW_ERR_BAD_ARG;
+  const int rc = topolow_fit_batch_interruptible(n_jobs, pb, pr, rs, devices[0], poll, user);
+  if (rc == TOPOLOW_OK && n_jobs > 0) {
+    size_t at = strlen(rs[0].message);
+    at += (size_t)snprintf(rs[0].message + at, sizeof rs[0].message - at, " devices=");
+    for (int32_t i = 0; i < n_devices && at < sizeof rs[0].message; ++i)
+      at += (size_t)snprintf(rs[0].message + at, sizeof rs[0].message - at, "%s%d", i ? "," : "", devices[i]);
+  }
+  return rc;
+}

@@ -9,10 +9,14 @@
  *   harness batch     problem.bin out.bin n_jobs n_iter k0 cooling c_rep rel_eps window freq keep
  *   harness batch_interrupt problem.bin out.bin n_jobs n_iter k0 cooling c_rep rel_eps window freq keep at_check
  *                     (the batch call with R_CheckUserInterrupt firing at its at_check-th call; 0 = never)
+ *   harness batch_devices problem.bin out.bin n_jobs n_iter k0 cooling c_rep rel_eps window freq keep int|double d...
+ *                     (the batch call with `device` an integer or double vector of the ordinals d...; NA = NA, none =
+ *                     a vector of length 0)
  *
  * problem.bin: int64 n, d, E, H | init[n*d] f64 (column-major) | degrees[n] i32 | edge_i[E] edge_j[E] i32 | edge_dist[E]
  * f64 | edge_thresh[E] i32 | holdout_i[H] holdout_j[H] i32 | holdout_truth[H] f64.  out.bin: the doubles named in the
  * JSON line, in order.  Test infrastructure only. */
+#include <math.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -123,10 +127,23 @@ int main(int argc, char** argv) {
     printf("}\n");
     return 0;
   }
-  const int batch_interrupt = !strcmp(what, "batch_interrupt");
-  if ((!strcmp(what, "batch") && argc >= 13) || (batch_interrupt && argc >= 14)) {
+  const int batch_interrupt = !strcmp(what, "batch_interrupt"), batch_devices = !strcmp(what, "batch_devices");
+  if ((!strcmp(what, "batch") && argc >= 13) || ((batch_interrupt || batch_devices) && argc >= 14)) {
     struct problem p = load(argv[2]);
     if (batch_interrupt) stub.interrupt_after = atoi(argv[13]);
+    SEXP device;
+    if (batch_devices) {
+      const int nd = argc - 14, as_double = !strcmp(argv[13], "double");
+      device = as_double ? stub_real(nd, NULL) : stub_int(nd, NULL);
+      for (int i = 0; i < nd; ++i) {
+        const int na = !strcmp(argv[14 + i], "NA");
+        if (as_double) REAL(device)[i] = na ? NAN : atof(argv[14 + i]);
+        else INTEGER(device)[i] = na ? NA_INTEGER : atoi(argv[14 + i]);
+      }
+    } else {
+      int dev = 0;
+      device = stub_int(1, &dev);
+    }
     const int nj = atoi(argv[4]), keep = atoi(argv[12]);
     SEXP jobs = stub_list(nj);
     for (int j = 0; j < nj; ++j) {
@@ -138,8 +155,7 @@ int main(int argc, char** argv) {
       SET_VECTOR_ELT(job, 9, stub_real(7, hp));
       SET_VECTOR_ELT(jobs, j, job);
     }
-    int dev = 0;
-    SEXP r = _topolow_fit_batch_b200(jobs, Rf_ScalarLogical(keep), stub_int(1, &dev));
+    SEXP r = _topolow_fit_batch_b200(jobs, Rf_ScalarLogical(keep), device);
     FILE* o = fopen(argv[3], "wb");
     printf("{\"scenario\": \"%s\", \"left_by\": \"return\", \"n\": %d, \"names\": [", what, (int)XLENGTH(r));
     for (int i = 0; nj > 0 && i < (int)XLENGTH(VECTOR_ELT(r, 0)); ++i) printf("%s\"%s\"", i ? ", " : "", stub_name(VECTOR_ELT(r, 0), i));

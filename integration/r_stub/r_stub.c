@@ -63,6 +63,18 @@ SEXP Rf_allocVector(unsigned type, R_xlen_t n) {
     default: stub.type_errors++; return R_NilValue;
   }
 }
+/* INTSXP only (what the shim asks for): x itself when it is already integer, NA for NaN or out of range doubles */
+SEXP Rf_coerceVector(SEXP x, unsigned type) {
+  if (type != INTSXP || (x->type != INTSXP && x->type != LGLSXP && x->type != REALSXP)) { stub.type_errors++; return R_NilValue; }
+  if (x->type == INTSXP) return x;
+  SEXP y = Rf_allocVector(INTSXP, x->len);
+  for (R_xlen_t i = 0; i < x->len; ++i) {
+    if (x->type == LGLSXP) { ((int*)y->data)[i] = ((int*)x->data)[i]; continue; }
+    const double v = ((double*)x->data)[i];
+    ((int*)y->data)[i] = (v != v || v >= 2147483648.0 || v <= -2147483649.0) ? NA_INTEGER : (int)v;
+  }
+  return y;
+}
 SEXP Rf_allocMatrix(unsigned type, int nrow, int ncol) {
   SEXP x = Rf_allocVector(type, (R_xlen_t)nrow * ncol);
   x->nrow = nrow; x->ncol = ncol;

@@ -51,7 +51,7 @@ INTERRUPT_FN = C.CFUNCTYPE(C.c_int, C.c_void_p)
 
 EXPORTS = [
     "topolow_fit", "topolow_fit_interruptible", "topolow_optimize_layout_exact", "topolow_fit_batch",
-    "topolow_fit_batch_interruptible",
+    "topolow_fit_batch_interruptible", "topolow_fit_batch_devices",
     "topolow_plan_create", "topolow_plan_run", "topolow_plan_result", "topolow_plan_info",
     "topolow_plan_destroy", "topolow_plan_enumerate", "topolow_schedule_enumerate", "topolow_plan_run_job",
     "topolow_plan_end_iteration", "topolow_plan_layout", "topolow_plan_positions", "topolow_plan_enumerate_job",
@@ -94,6 +94,9 @@ def lib() -> C.CDLL:
     L.topolow_fit_batch_interruptible.restype = C.c_int
     L.topolow_fit_batch_interruptible.argtypes = [C.c_int32, C.POINTER(Problem), C.POINTER(Params), C.POINTER(Result),
                                                   C.c_int32, INTERRUPT_FN, C.c_void_p]
+    L.topolow_fit_batch_devices.restype = C.c_int
+    L.topolow_fit_batch_devices.argtypes = [C.c_int32, C.POINTER(Problem), C.POINTER(Params), C.POINTER(Result), _i32p,
+                                            C.c_int32, INTERRUPT_FN, C.c_void_p]
     L.topolow_plan_create.restype = C.c_int
     L.topolow_plan_create.argtypes = [C.POINTER(Problem), C.POINTER(Params), C.POINTER(C.c_void_p), C.c_char_p,
                                       C.c_int32]
@@ -280,11 +283,19 @@ def fit_batch(jobs, device=0, interrupt=None):
     result dicts; a failed job yields {'status': code, 'message': ...} instead of raising
     (R/adaptive_sampling.R:2657-2666 turns fit errors into NA rows).
 
+    device: a CUDA ordinal, or a sequence of ordinals (topolow_fit_batch_devices): the jobs are dealt over the
+    devices of the list, one host thread each, and every result is bit for bit what the batch returns on the first
+    device of the list.  An ordinal may repeat.
+
     interrupt: a callable polled while the batch runs (topolow_fit_batch_interruptible); when it returns True the
     fits stop and TopolowError(ERR_INTERRUPTED) is raised with the per-job list attached as `.results`.  There a job
     that was stopped is a full result dict with status ERR_INTERRUPTED and a 'message' (its best state as of its last
     completed iteration); jobs that had already ended are what the uninterrupted call returns."""
     L = lib()
+    devices = None
+    if not isinstance(device, (int, np.integer)):
+        devices = np.ascontiguousarray([int(d) for d in device], dtype=np.int32)
+        device = int(devices[0]) if len(devices) else 0     # Params.device (ignored by the batch) stays an int
     n = len(jobs)
     probs, pars, ress = (Problem * n)(), (Params * n)(), (Result * n)()
     keep, outs = [], []
@@ -299,10 +310,15 @@ def fit_batch(jobs, device=0, interrupt=None):
         ress[j].positions = out.ctypes.data_as(_dp)
         keep.append((pa, k2))
         outs.append(out)
-    if interrupt is None:
+    cb = INTERRUPT_FN() if interrupt is None else INTERRUPT_FN(lambda _u: int(bool(interrupt())))   # (null: no poll)
+    if devices is not None:
+        rc = L.topolow_fit_batch_devices(n, probs, pars, ress, devices.ctypes.data_as(_i32p), len(devices), cb, None)
+        if rc not in (OK, ERR_INTERRUPTED):
+            why = ress[0].message.decode() if n else ""
+            raise TopolowError(rc, why or f"topolow_fit_batch_devices failed with status {rc}")
+    elif interrupt is None:
         rc = L.topolow_fit_batch(n, probs, pars, ress, device)
     else:
-        cb = INTERRUPT_FN(lambda _u: int(bool(interrupt())))
         rc = L.topolow_fit_batch_interruptible(n, probs, pars, ress, device, cb, None)
     if rc not in (OK, ERR_INTERRUPTED):
         raise TopolowError(rc, f"topolow_fit_batch failed with status {rc}")

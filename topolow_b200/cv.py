@@ -214,6 +214,9 @@ def likelihood_batch(dissimilarity_matrix, samples, mapping_max_iter, relative_e
     preserve_order defaults to True here because fold residuals are aligned by position; the
     reference re-aligns by row names (R/error_metrics.R:76-87) which an unnamed matrix lacks.
 
+    device: a CUDA ordinal, or a sequence of ordinals over which the batch is dealt (_lib.fit_batch); the scores do
+    not depend on it.
+
     interrupt: a callable polled while the fits run (see _lib.fit_batch); when it returns True the batch stops and
     TopolowError(ERR_INTERRUPTED) is raised."""
     rng = rng or np.random.default_rng(seed)

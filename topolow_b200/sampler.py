@@ -195,7 +195,7 @@ def adaptive_mc_batch(samples, dissimilarity_matrix, iterations, chains, mapping
     The reference's chains are separate processes that append to one CSV whenever they finish; here a round's draws
     all see the table as it was when the round began.
     `interrupt` is polled while a round's batch runs (cv.likelihood_batch); when it returns True the batch stops and
-    TopolowError(ERR_INTERRUPTED) is raised."""
+    TopolowError(ERR_INTERRUPTED) is raised.  `device` may be a sequence of ordinals (cv.likelihood_batch)."""
     rng = rng or np.random.default_rng()
     table = {k: np.array(v, copy=True) for k, v in _as_table(samples).items()}
     required = list(PAR_NAMES) + ["NLL", "Holdout_MAE"]

@@ -162,16 +162,26 @@ TOPOLOW_API int topolow_optimize_layout_exact(
 /* ---- batch of independent fits ----------------------------------------- */
 /* Jobs run concurrently on `device` (params[j].device is ignored); results[j].status is
  * per job and the call itself only fails for argument / CUDA set-up errors.
- * With 16 or more jobs every fit runs on one CTA (64-point tiles unless tile_points is set) and the fits
- * are launched many per kernel.  Jobs whose edge_i / edge_j / edge_dist / edge_thresh POINTERS (and n,
- * n_edges) are equal share one set of device records: hand the parameter samples of a CV grid the same
- * arrays per fold.  topolow_fit_batch is topolow_fit_batch_interruptible with poll = NULL. */
+ * Modes: params[j].mode is TOPOLOW_MODE_COLOURED or TOPOLOW_MODE_ROWBLOCK; a TOPOLOW_MODE_REPLAY job fails alone with
+ * TOPOLOW_ERR_BAD_ARG.
+ *   - Coloured jobs run first.  With 16 or more coloured jobs in the call (every job that is not a row-block job
+ *     counts) every coloured fit runs on one CTA (64-point tiles unless tile_points is set) and the fits are launched
+ *     many per kernel.  Jobs whose edge_i / edge_j / edge_dist / edge_thresh POINTERS (and n, n_edges) are equal share
+ *     one set of device records: hand the parameter samples of a CV grid the same arrays per fold.
+ *   - Row-block jobs (large maps, ndim 1..32) run after the coloured fits of the call (of the share, for
+ *     topolow_fit_batch_devices) have ended, one at a time in job order, each created, run, read back and destroyed before the next: device memory is bounded by the largest job.
+ *     Each result is bit for bit what topolow_fit returns for the same problem and params on `device` (positions,
+ *     MAE, k, iterations, iterations_run, pair_updates, hold-out sums, trace, status and message, including the
+ *     single fit's argument checks); device_ms is the job's own CUDA-event time.  No records are shared between them.
+ *   - results[j].positions may be NULL (not topolow_fit's): the positions are then not returned, and the hold-out
+ *     sums are the same as with positions.
+ * topolow_fit_batch is topolow_fit_batch_interruptible with poll = NULL. */
 TOPOLOW_API int topolow_fit_batch(int32_t n_jobs, const topolow_problem* problems, const topolow_params* params,
                       topolow_result* results, int32_t device);
 
 /* The same batch, stoppable.  `poll` is called from the calling thread only: once before set-up, once after set-up
- * (before the first launch), then at least every 100 ms (every 20 ms today) while any fit of the batch is on the
- * device, and not again once every fit has ended.  When it returns non-zero the library raises the batch's abort
+ * (before the first launch), before and after the set-up of each row-block job, then at least every 100 ms (every
+ * 20 ms today) while any fit of the batch is on the device, and not again once every fit has ended.  When it returns non-zero the library raises the batch's abort
  * word (mapped host memory the kernels read), issues no further launch, waits for every stream and returns
  * TOPOLOW_ERR_INTERRUPTED with every result filled in:
  *   - a job that had already ended (converged, ran all its iterations, non-finite) keeps the result it has without
@@ -182,7 +192,9 @@ TOPOLOW_API int topolow_fit_batch(int32_t n_jobs, const topolow_problem* problem
  *   - a job that failed set-up (or has n < 2) keeps its status.
  * How soon a fit stops: a fit on one CTA (every fit of a batch of 16 or more jobs) at the end of the iteration
  * it is running; a fit on several CTAs at its next convergence check or finite check, i.e. after at most
- * min(convergence_check_freq, 10) more iterations; a fit or chunk that had not started yet does not start.
+ * min(convergence_check_freq, 10) more iterations; a row-block job at an iteration boundary within 10 iterations (the
+ * host keeps at most 10 of its iterations queued); a fit or chunk that had not started yet does not start.  The
+ * set-up of a row-block job (record build and uploads) is not interrupted mid-way.
  * Everything the batch allocated is released before the call returns, the abort word included. */
 TOPOLOW_API int topolow_fit_batch_interruptible(int32_t n_jobs, const topolow_problem* problems,
                                                 const topolow_params* params, topolow_result* results, int32_t device,
@@ -194,8 +206,10 @@ TOPOLOW_API int topolow_fit_batch_interruptible(int32_t n_jobs, const topolow_pr
  * runs this path).
  *   - Results: every job's result (positions, MAE, k, iterations, iterations_run, pair_updates, hold-out sums,
  *     trace, status, message) is bit for bit what topolow_fit_batch_interruptible(..., devices[0], ...) returns for
- *     the same arrays, whatever the list.  The one-CTA rule above (16 or more jobs) is taken on n_jobs of the whole
- *     call, never on one share.  params[j].device is ignored.
+ *     the same arrays, whatever the list.  The one-CTA rule above (16 or more coloured jobs) is taken on the jobs of the
+ *     whole call, never on one share.  params[j].device is ignored.  Row-block jobs are dealt like the others; a share
+ *     runs its own one at a time, and a single-rank row-block fit waits on no peer, so the shares of one device (an
+ *     ordinal that repeats) run their row-block fits side by side.
  *   - Arguments: a null `devices`, n_devices < 1 or an ordinal outside [0, cudaGetDeviceCount()) returns
  *     TOPOLOW_ERR_BAD_ARG before anything is allocated, with the reason in results[0].message when n_jobs > 0
  *     (TOPOLOW_ERR_CUDA when the device count cannot be read).  n_devices == 1 is

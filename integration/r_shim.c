@@ -88,18 +88,34 @@ SEXP _topolow_optimize_layout_b200(SEXP init, SEXP dmat, SEXP tmat, SEXP degrees
   return out;
 }
 
+/* The optional 11th element of a batch job: "coloured" or "rowblock" (a character scalar). */
+static int job_mode(SEXP job, int number) {
+  if (XLENGTH(job) < 11) return TOPOLOW_MODE_COLOURED;
+  SEXP m = VECTOR_ELT(job, 10);
+  if (TYPEOF(m) == STRSXP && XLENGTH(m) == 1) {   /* (NA_character_ is the string "NA" here: refused below) */
+    const char* s = CHAR(STRING_ELT(m, 0));
+    if (strcmp(s, "coloured") == 0) return TOPOLOW_MODE_COLOURED;
+    if (strcmp(s, "rowblock") == 0) return TOPOLOW_MODE_ROWBLOCK;
+  }
+  Rf_error("job %d: element 11 (mode) must be 'coloured' or 'rowblock'", number);
+}
+
 /* One batch of independent fits.  `jobs` is a list; job j is a named-by-position list of
  *   [[1]] initial_positions (n x ndim double)   [[2]] degrees (int)   [[3]] edge_i  [[4]] edge_j (int, 0-based)
  *   [[5]] edge_dist (double)  [[6]] edge_thresh (int)   [[7]] holdout_i  [[8]] holdout_j (int, 0-based; may be
  *   length 0)  [[9]] holdout_truth (double)   [[10]] c(mapping_max_iter, k0, cooling_rate, c_repulsion,
- *   relative_epsilon, convergence_counter, convergence_check_freq) (double)
+ *   relative_epsilon, convergence_counter, convergence_check_freq) (double)   [[11]] optional: the mode, "coloured"
+ *   (the default when the job has 10 elements) or "rowblock" (large maps, ndim up to 32; the fit is exactly the
+ *   single row-block fit); anything else is an R error raised before the library is called
  * Jobs that carry the SAME R vectors for [[3]]..[[6]] (the parameter samples evaluated on one fold) share one set
  * of device records - R lists hold references, so `job$edge_i <- fold$edge_i` is enough.  Returns a list of
  * per-job lists {converged, iterations, final_mae, final_k, holdout_sum_abs, holdout_count, status, message,
- * positions (only when keep_positions)}: a failed fit is a status + message, never an R error
+ * positions (only when keep_positions; a 0 x 0 matrix otherwise)}: a failed fit is a status + message, never an R error
  * (R/adaptive_sampling.R:2657-2666 turns failures into NA rows).  Ctrl-C stops the batch as it stops a single fit: the
  * library is polled while the fits run, stops them, releases what it holds and returns TOPOLOW_ERR_INTERRUPTED, and
  * the R condition is raised from this frame.
+ * keep_positions = FALSE is the call for a CV grid: only the hold-out sums are needed, and they are the same as with
+ * TRUE; no positions cross back (a 100 000-point map would be 12.8 MB per fold fit).
  * `device` is one CUDA ordinal, or an integer or double vector of them (e.g. 0:7): the batch is then dealt over those
  * GPUs from this one process (topolow_fit_batch_devices), with the same results as on the first of them. */
 SEXP _topolow_fit_batch_b200(SEXP jobs, SEXP keep_positions, SEXP device) {
@@ -123,6 +139,7 @@ SEXP _topolow_fit_batch_b200(SEXP jobs, SEXP keep_positions, SEXP device) {
   for (R_xlen_t j = 0; j < nj; ++j) {
     SEXP job = VECTOR_ELT(jobs, j);
     if (TYPEOF(job) != VECSXP || XLENGTH(job) < 10) Rf_error("job %d: expected a list of 10 elements", (int)j + 1);
+    const int mode = job_mode(job, (int)j + 1);
     SEXP init = VECTOR_ELT(job, 0), hp = VECTOR_ELT(job, 9);
     if (TYPEOF(init) != REALSXP || TYPEOF(hp) != REALSXP || XLENGTH(hp) < 7) Rf_error("job %d: malformed", (int)j + 1);
     const R_xlen_t E = XLENGTH(VECTOR_ELT(job, 2)), Hn = XLENGTH(VECTOR_ELT(job, 6));
@@ -141,6 +158,7 @@ SEXP _topolow_fit_batch_b200(SEXP jobs, SEXP keep_positions, SEXP device) {
     }
     const double* h = REAL(hp);
     fill_params(&pr[j], (int)h[0], h[1], h[2], h[3], h[4], (int)h[5], (int)h[6], 0);
+    pr[j].mode = mode;
     pr[j].seed = seed + (uint64_t)j;
     memset(&rs[j], 0, sizeof rs[j]);
     SEXP res = PROTECT(Rf_mkNamed(VECSXP, names));

@@ -12,6 +12,9 @@
  *   harness batch_devices problem.bin out.bin n_jobs n_iter k0 cooling c_rep rel_eps window freq keep int|double d...
  *                     (the batch call with `device` an integer or double vector of the ordinals d...; NA = NA, none =
  *                     a vector of length 0)
+ *   harness batch_modes problem.bin out.bin n_jobs n_iter k0 cooling c_rep rel_eps window freq keep m...
+ *                     (the batch call with one mode token per job: "-" = a job of 10 elements, "@int" / "@real" = an
+ *                     11th element of that type, anything else = that string as the 11th element)
  *
  * problem.bin: int64 n, d, E, H | init[n*d] f64 (column-major) | degrees[n] i32 | edge_i[E] edge_j[E] i32 | edge_dist[E]
  * f64 | edge_thresh[E] i32 | holdout_i[H] holdout_j[H] i32 | holdout_truth[H] f64.  out.bin: the doubles named in the
@@ -128,7 +131,9 @@ int main(int argc, char** argv) {
     return 0;
   }
   const int batch_interrupt = !strcmp(what, "batch_interrupt"), batch_devices = !strcmp(what, "batch_devices");
-  if ((!strcmp(what, "batch") && argc >= 13) || ((batch_interrupt || batch_devices) && argc >= 14)) {
+  const int batch_modes = !strcmp(what, "batch_modes");
+  if ((!strcmp(what, "batch") && argc >= 13) || ((batch_interrupt || batch_devices) && argc >= 14) ||
+      (batch_modes && argc >= 13 + atoi(argv[4]))) {
     struct problem p = load(argv[2]);
     if (batch_interrupt) stub.interrupt_after = atoi(argv[13]);
     SEXP device;
@@ -147,7 +152,12 @@ int main(int argc, char** argv) {
     const int nj = atoi(argv[4]), keep = atoi(argv[12]);
     SEXP jobs = stub_list(nj);
     for (int j = 0; j < nj; ++j) {
-      SEXP job = stub_list(10);
+      const char* m = batch_modes ? argv[13 + j] : "-";
+      SEXP job = stub_list(strcmp(m, "-") ? 11 : 10);
+      if (strcmp(m, "-")) {
+        int one = 1; double half = 0.5;
+        SET_VECTOR_ELT(job, 10, !strcmp(m, "@int") ? stub_int(1, &one) : !strcmp(m, "@real") ? stub_real(1, &half) : Rf_mkString(m));
+      }
       double hp[7] = {atof(argv[5]), atof(argv[6]) * (1.0 + 0.25 * j), atof(argv[7]), atof(argv[8]), atof(argv[9]), atof(argv[10]), atof(argv[11])};
       SET_VECTOR_ELT(job, 0, p.init); SET_VECTOR_ELT(job, 1, p.deg);
       SET_VECTOR_ELT(job, 2, p.ei); SET_VECTOR_ELT(job, 3, p.ej); SET_VECTOR_ELT(job, 4, p.ed); SET_VECTOR_ELT(job, 5, p.et);   /* the same vectors in every job */

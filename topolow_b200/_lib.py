@@ -239,12 +239,14 @@ def make_params(n_iter, k0, cooling_rate, c_repulsion, relative_epsilon=1e-4, co
     return p, keep
 
 
-def result_dict(res: Result, positions: np.ndarray, trace=None):
-    out = dict(positions=np.ascontiguousarray(positions), converged=bool(res.converged),
+def result_dict(res: Result, positions, trace=None):
+    out = dict(converged=bool(res.converged),
                iterations=int(res.iterations), final_mae=float(res.final_mae), final_k=float(res.final_k),
                iterations_run=int(res.iterations_run), pair_updates=int(res.pair_updates),
                device_ms=float(res.device_ms), status=int(res.status),
                holdout_sum_abs=float(res.holdout_sum_abs), holdout_count=int(res.holdout_count))
+    if positions is not None:
+        out["positions"] = np.ascontiguousarray(positions)
     if trace is not None:
         out["trace_mae"] = trace
     return out
@@ -278,10 +280,14 @@ def fit(initial_positions, degrees, edge_i, edge_j, edge_dist, edge_thresh, n_it
     return result_dict(res, out, tr)
 
 
-def fit_batch(jobs, device=0, interrupt=None):
-    """jobs: list of dicts with the keyword arguments of `fit` (coloured mode).  Returns a list of
-    result dicts; a failed job yields {'status': code, 'message': ...} instead of raising
+def fit_batch(jobs, device=0, interrupt=None, keep_positions=True):
+    """jobs: list of dicts with the keyword arguments of `fit`; `mode` is MODE_COLOURED (the default) or MODE_ROWBLOCK
+    (large maps and ndim 17..32: each such job is exactly `fit(..., mode=MODE_ROWBLOCK)`), and `trace=True` adds
+    'trace_mae'.  Returns a list of result dicts; a failed job yields {'status': code, 'message': ...} instead of raising
     (R/adaptive_sampling.R:2657-2666 turns fit errors into NA rows).
+
+    keep_positions=False: the positions do not come back (a CV grid needs only the hold-out sums, which are the same
+    either way) and the result dicts have no 'positions'.
 
     device: a CUDA ordinal, or a sequence of ordinals (topolow_fit_batch_devices): the jobs are dealt over the
     devices of the list, one host thread each, and every result is bit for bit what the batch returns on the first
@@ -298,18 +304,23 @@ def fit_batch(jobs, device=0, interrupt=None):
         device = int(devices[0]) if len(devices) else 0     # Params.device (ignored by the batch) stays an int
     n = len(jobs)
     probs, pars, ress = (Problem * n)(), (Params * n)(), (Result * n)()
-    keep, outs = [], []
+    keep, outs, traces = [], [], []
     for j, job in enumerate(jobs):
         job = dict(job)
         pa = ProblemArrays(job.pop("initial_positions"), job.pop("degrees"), job.pop("edge_i"), job.pop("edge_j"),
                            job.pop("edge_dist"), job.pop("edge_thresh"), job.pop("holdout", None))
+        tr = np.full(max(int(job["n_iter"]), 1), np.nan) if job.pop("trace", False) else None
         pr, k2 = make_params(job.pop("n_iter"), job.pop("k0"), job.pop("cooling_rate"), job.pop("c_repulsion"),
                              device=device, **job)
-        out = np.empty((pa.n, pa.ndim), dtype=np.float64, order="F")
+        out = np.empty((pa.n, pa.ndim), dtype=np.float64, order="F") if keep_positions else None
         probs[j], pars[j] = pa.struct, pr
-        ress[j].positions = out.ctypes.data_as(_dp)
+        if out is not None:
+            ress[j].positions = out.ctypes.data_as(_dp)
+        if tr is not None:
+            ress[j].trace_mae = tr.ctypes.data_as(_dp)
         keep.append((pa, k2))
         outs.append(out)
+        traces.append(tr)
     cb = INTERRUPT_FN() if interrupt is None else INTERRUPT_FN(lambda _u: int(bool(interrupt())))   # (null: no poll)
     if devices is not None:
         rc = L.topolow_fit_batch_devices(n, probs, pars, ress, devices.ctypes.data_as(_i32p), len(devices), cb, None)
@@ -325,11 +336,11 @@ def fit_batch(jobs, device=0, interrupt=None):
     results = []
     for j in range(n):
         if ress[j].status == ERR_INTERRUPTED:
-            results.append(dict(result_dict(ress[j], outs[j]), message=ress[j].message.decode()))
+            results.append(dict(result_dict(ress[j], outs[j], traces[j]), message=ress[j].message.decode()))
         elif ress[j].status != OK:
             results.append(dict(status=int(ress[j].status), message=ress[j].message.decode()))
         else:
-            results.append(result_dict(ress[j], outs[j]))
+            results.append(result_dict(ress[j], outs[j], traces[j]))
     if rc == ERR_INTERRUPTED:
         err = TopolowError(rc, "interrupted")
         err.results = results

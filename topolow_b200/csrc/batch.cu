@@ -5,7 +5,8 @@
 // :2670-2693) as ONE call.  Jobs that point at the same edge arrays share one EdgeStore; fits that run
 // on one CTA are launched many per kernel (tile_batch_kernel), grouped by (ndim, precision, warps, tile).
 // topolow_fit_batch_devices deals the jobs over several devices and runs each device's share on a host thread of
-// its own with the same code (run_share).
+// its own with the same code (run_share).  Row-block jobs (large maps, ndim up to 32) run after a share's coloured
+// fits have ended, one at a time, each exactly the single fit of topolow_fit.
 #include <algorithm>
 #include <atomic>
 #include <chrono>
@@ -21,6 +22,7 @@
 #include <vector>
 
 #include "plan.h"
+#include "rowblock.h"
 
 using namespace tl;
 
@@ -162,10 +164,19 @@ struct AbortAttach {
   ~AbortAttach() { if (word) stop.detach(word); }
 };
 
-// One device's share of a batch: jobs `ids` (indices into the caller's arrays) of a call of n_total jobs, run on
-// `device` from the current host thread; `shares` host threads run shares at the same time (they split the set-up
-// threads).  Returns TOPOLOW_OK, TOPOLOW_ERR_INTERRUPTED when this share saw the stop request, or TOPOLOW_ERR_CUDA.
-int run_share(const std::vector<int>& ids, int n_total, const topolow_problem* problems_in,
+// Jobs of a call that are not row-block jobs: the count the one-CTA rule is taken on, so that adding or removing
+// row-block jobs never changes a coloured job's result.
+int coloured_count(int n_jobs, const topolow_params* params) {
+  int c = 0;
+  for (int j = 0; j < n_jobs; ++j) c += params[j].mode != TOPOLOW_MODE_ROWBLOCK;
+  return c;
+}
+
+// One device's share of a batch: jobs `ids` (indices into the caller's arrays) of a call with n_coloured jobs that are
+// not row-block jobs, run on `device` from the current host thread; `shares` host threads run shares at the same time
+// (they split the set-up threads).  Returns TOPOLOW_OK, TOPOLOW_ERR_INTERRUPTED when this share saw the stop request,
+// or TOPOLOW_ERR_CUDA.
+int run_share(const std::vector<int>& ids, int n_coloured, const topolow_problem* problems_in,
               const topolow_params* params_in, topolow_result* results_in, int device, int share, int shares,
               StopSource& stop) {
   const int n_jobs = (int)ids.size();
@@ -187,16 +198,18 @@ int run_share(const std::vector<int>& ids, int n_total, const topolow_problem* p
   const int* d_abort = nullptr;            // its device address
   std::vector<std::unique_ptr<topolow_plan>> plans(n_jobs);
   std::vector<int> left(n_jobs, 0);
+  std::vector<char> rowblock(n_jobs, 0);   // row-block jobs still to run (one at a time, after the coloured launches)
+  int rowblock_running = -1;
   const bool dbg = std::getenv("TOPOLOW_DEBUG") != nullptr;
   const auto t_begin = std::chrono::steady_clock::now();
   auto since = [&]() { return std::chrono::duration<double>(std::chrono::steady_clock::now() - t_begin).count(); };
   // Many independent fits: one CTA per fit (no grid barrier, plain launches that run side by side on
-  // different SMs) keeps every SM busy; a lone large fit still gets the whole chip.  Decided on the job count of the
-  // whole call, so that a job's result does not depend on how the call was split over devices.
+  // different SMs) keeps every SM busy; a lone large fit still gets the whole chip.  Decided on the coloured job count
+  // of the whole call, so that a job's result does not depend on how the call was split over devices.
   auto job_params = [&](int j) {
     topolow_params pr = params[j];
     pr.device = device;
-    if (n_total >= 16 && pr.max_ctas == 0) {
+    if (n_coloured >= 16 && pr.max_ctas == 0) {
       pr.max_ctas = 1;
       if (pr.tile_points == 0) pr.tile_points = batch_tile_points();
     }
@@ -265,8 +278,8 @@ int run_share(const std::vector<int>& ids, int n_total, const topolow_problem* p
         set_msg(r.message, sizeof r.message, "Need at least 2 points for embedding");
         return;
       }
-      if (!r.positions) throw BadArg("result->positions must be caller-allocated");
-      if (params[j].mode != TOPOLOW_MODE_COLOURED) throw BadArg("batch supports the coloured mode only");
+      if (params[j].mode == TOPOLOW_MODE_ROWBLOCK) { rowblock[j] = 1; return; }   // set up when its turn comes
+      if (params[j].mode != TOPOLOW_MODE_COLOURED) throw BadArg("batch supports the coloured and row-block modes only");
       const topolow_params pr = job_params(j);
       std::shared_ptr<EdgeStore> store;
       if (slot_of_job[j] >= 0) {
@@ -396,6 +409,54 @@ int run_share(const std::vector<int>& ids, int n_total, const topolow_problem* p
       if (cudaPeekAtLastError() == cudaErrorNotReady) cudaGetLastError();
       if (dbg) std::fprintf(stderr, "[topolow] batch %s (device %d): %.3f s\n", aborted ? "interrupted" : "fits ended", device, since());
     }
+    // Row-block jobs, once the coloured fits have ended (waited for above with the poll running: row_create
+    // synchronises the device, which would otherwise wait for them without a poll): one at a time in job-index order,
+    // each created, run, read back and destroyed before the next (device memory is bounded by the largest job), each
+    // exactly what topolow_fit returns.  The poll runs before and after each set-up; the set-up itself is not
+    // interrupted.
+    auto stop_requested = [&]() {
+      if (!stop.armed()) return false;
+      if (aborted || stop.fired()) return aborted = true;
+      return std::chrono::steady_clock::now() - last_poll >= kPollPeriod && poll_now();
+    };
+    for (int j = 0; j < n_jobs; ++j) {
+      if (!rowblock[j]) continue;
+      topolow_result& r = *results[j];
+      rowblock[j] = 0;
+      if (stop.armed() && (aborted || poll_now())) { result_not_run(problems[j], r); continue; }
+      std::unique_ptr<RowPlan, void (*)(RowPlan*)> rp(nullptr, row_destroy);
+      try {
+        topolow_params pr = params[j];
+        pr.device = device;
+        rp.reset(row_create(problems[j], pr, 0, 1));
+      } catch (const CudaError& e) {   // (out of device memory): this job fails, the share goes on
+        r.status = TOPOLOW_ERR_CUDA; set_msg(r.message, sizeof r.message, e.what()); cudaGetLastError();
+        continue;
+      } catch (const std::exception& e) {
+        r.status = TOPOLOW_ERR_BAD_ARG; set_msg(r.message, sizeof r.message, e.what());
+        continue;
+      }
+      if (stop.armed() && poll_now()) { rp.reset(); result_not_run(problems[j], r); continue; }
+      rowblock_running = j;
+      const bool cut = row_run_windows(*rp, stop_requested);
+      // without positions to return, the hold-out cells are scored on a host copy of them
+      double* const pos = r.positions;
+      std::vector<double> scratch;
+      if (!pos && problems[j].n_holdout > 0) {
+        scratch.resize((size_t)problems[j].n * (size_t)problems[j].ndim);
+        r.positions = scratch.data();
+      }
+      try {
+        row_result(*rp, r, cut);
+      } catch (const BadArg& e) {   // (hold-out cells out of range: what topolow_fit reports)
+        r.status = TOPOLOW_ERR_BAD_ARG; set_msg(r.message, sizeof r.message, e.what());
+      } catch (...) {
+        r.positions = pos;
+        throw;
+      }
+      r.positions = pos;
+      rowblock_running = -1;
+    }
     for (auto& kv : groups) {
       Group& g = kv.second;
       TL_CUDA(cudaEventSynchronize(*g.ev1));
@@ -421,7 +482,9 @@ int run_share(const std::vector<int>& ids, int n_total, const topolow_problem* p
     if (dbg) std::fprintf(stderr, "[topolow] batch plans destroyed (device %d): %.3f s\n", device, since());
   } catch (const CudaError& e) {
     for (int j = 0; j < n_jobs; ++j)
-      if (plans[j]) { results[j]->status = TOPOLOW_ERR_CUDA; set_msg(results[j]->message, sizeof results[j]->message, e.what()); }
+      if (plans[j] || rowblock[j] || j == rowblock_running) {
+        results[j]->status = TOPOLOW_ERR_CUDA; set_msg(results[j]->message, sizeof results[j]->message, e.what());
+      }
     cudaGetLastError();
     return TOPOLOW_ERR_CUDA;
   }
@@ -467,7 +530,7 @@ extern "C" int topolow_fit_batch_interruptible(int32_t n_jobs, const topolow_pro
   std::vector<int> all(n_jobs);
   for (int j = 0; j < n_jobs; ++j) all[j] = j;
   StopSource stop(poll, user, 0);
-  return run_share(all, n_jobs, problems, params, results, device, 0, 1, stop);
+  return run_share(all, coloured_count(n_jobs, params), problems, params, results, device, 0, 1, stop);
 }
 
 extern "C" int topolow_fit_batch_devices(int32_t n_jobs, const topolow_problem* problems, const topolow_params* params,
@@ -495,13 +558,14 @@ extern "C" int topolow_fit_batch_devices(int32_t n_jobs, const topolow_problem* 
     return TOPOLOW_ERR_INTERRUPTED;
   }
   const std::vector<std::vector<int>> parts = deal_jobs(n_jobs, problems, params, n_devices);
+  const int n_coloured = coloured_count(n_jobs, params);
   StopSource stop(poll, user, n_devices);
   std::vector<int> status(n_devices, TOPOLOW_OK);
   std::vector<std::thread> workers;
   for (int s = 0; s < n_devices; ++s)
     workers.emplace_back([&, s] {
       try {
-        status[s] = run_share(parts[s], n_jobs, problems, params, results, devices[s], s, n_devices, stop);
+        status[s] = run_share(parts[s], n_coloured, problems, params, results, devices[s], s, n_devices, stop);
       } catch (const std::exception& ex) {   // (host memory exhausted): the share's jobs fail, the others do not
         for (int j : parts[s]) { results[j].status = TOPOLOW_ERR_CUDA; set_msg(results[j].message, sizeof results[j].message, ex.what()); }
         status[s] = TOPOLOW_ERR_CUDA;

@@ -30,8 +30,12 @@
 // sequential loop statistically (tests/test_gpu_rowblock.py) and with its own CPU restatement
 // (oracle/relaxed_oracle.cpp) numerically.
 #include <algorithm>
+#include <chrono>
+#include <cstddef>
 #include <cstring>
+#include <functional>
 #include <memory>
+#include <thread>
 #include <vector>
 
 #include "plan.h"
@@ -1051,6 +1055,16 @@ void launch_pass(RowPlan& rp, cudaStream_t s, int cur, cudaEvent_t* ev, bool ove
   rp.launches += 3;
 }
 
+// ctl_kernel raises FitState::snapshot when its check improved the best state, and snap_kernel copies the positions
+// while it is raised.  The flag is cleared after every snap launch: once a fit has stopped, ctl_kernel returns at
+// once and a raised flag would stay raised, so the snap launches of the iterations the host had already enqueued
+// would copy the position buffer of their own parity over the best state - for every second of them the positions of
+// the iteration before the last one.  How many such launches there are depends on host timing, so the best positions
+// (and the hold-out sums scored on them) of a fit that stopped early depended on it.
+void clear_snapshot(const RowPlan& rp, cudaStream_t s) {
+  TL_CUDA(cudaMemsetAsync(reinterpret_cast<char*>(rp.state) + offsetof(FitState, snapshot), 0, sizeof(int), s));
+}
+
 // One iteration of one rank: the pass, then on check and finite-check iterations the edge MAE, the controller and the
 // best-state snapshot.
 template <int H>
@@ -1069,6 +1083,7 @@ void launch_iteration(RowPlan& rp, cudaStream_t s, cudaEvent_t* ev /* 7 events o
     if (ev) TL_CUDA(cudaEventRecord(ev[5], s));
     snap_kernel<<<148, 256, 0, s>>>(dv, nxt);
     if (ev) TL_CUDA(cudaEventRecord(ev[6], s));
+    clear_snapshot(rp, s);
     rp.launches += 3;
   }
   TL_CUDA(cudaGetLastError());
@@ -1363,6 +1378,42 @@ double row_run(RowPlan& rp, int n_iters, cudaStream_t stream_in, topolow_interru
   return ms;
 }
 
+bool row_run_windows(RowPlan& rp, const std::function<bool()>& stop) {
+  check_runnable(rp);
+  TL_CUDA(cudaSetDevice(rp.device));
+  constexpr int kWindow = 5;                  // iterations per window; two windows in flight
+  cudaStream_t s = rp.stream;
+  EventGuard win[2];
+  // (returns true when `stop` fired before `e` completed)
+  auto wait = [&](cudaEvent_t e) {
+    while (true) {
+      const cudaError_t q = cudaEventQuery(e);
+      if (q == cudaSuccess) return false;
+      if (q != cudaErrorNotReady) TL_CUDA(q);
+      if (stop()) return true;
+      std::this_thread::sleep_for(std::chrono::microseconds(200));
+    }
+  };
+  TL_CUDA(cudaEventRecord(rp.ev0, s));
+  int left = std::max(0, rp.prm.n_iter - rp.iter_launched);
+  bool cut = false;
+  for (int w = 0; left > 0 && !rp.h_flag[0]; ++w) {
+    if (w >= 2 ? wait(win[w & 1]) : (w == 1 && stop())) { cut = true; break; }   // window w - 2 has ended
+    const int c = std::min(left, kWindow);
+    for (int i = 0; i < c; ++i) launch_one(rp, s);
+    left -= c;
+    TL_CUDA(cudaEventRecord(win[w & 1], s));
+  }
+  TL_CUDA(cudaEventRecord(rp.ev1, s));
+  if (!cut) wait(rp.ev1);                     // a stop request now lets the queued iterations finish the fit
+  if (cudaPeekAtLastError() == cudaErrorNotReady) cudaGetLastError();
+  TL_CUDA(cudaEventSynchronize(rp.ev1));
+  float ms = 0.f;
+  TL_CUDA(cudaEventElapsedTime(&ms, rp.ev0, rp.ev1));
+  rp.total_ms += ms;
+  return cut && !rp.h_flag[0];                // a fit that converged or failed on its own was not cut short
+}
+
 double row_run_local(RowPlan* const* plans, int n, int n_iters) {
   for (int a = 0; a < n; ++a) check_runnable(*plans[a]);
   bool same_device = true;
@@ -1399,6 +1450,7 @@ double row_run_local(RowPlan* const* plans, int n, int n_iters) {
           RowPlan& rp = *plans[a];
           ctl_kernel<<<1, 256, 0, s>>>(rp.dv, rp.prm, check ? 1 : 0, fin ? 1 : 0, rp.epoch);
           snap_kernel<<<148, 256, 0, s>>>(rp.dv, nxt);
+          clear_snapshot(rp, s);
           rp.launches += 2;
         }
       }

@@ -1,6 +1,7 @@
 // topolow_b200/csrc/rowblock.h - host interface of the row-block ("owner computes") mode, rowblock.cu.
 #pragma once
 #include <cstdint>
+#include <functional>
 #include <vector>
 
 #include "../../include/topolow_b200.h"
@@ -20,6 +21,12 @@ RowPlan* row_create(const topolow_problem& pb, const topolow_params& pr, int ran
 void row_destroy(RowPlan* rp);
 // Up to n_iters further iterations (stops on convergence); returns CUDA-event milliseconds.
 double row_run(RowPlan& rp, int n_iters, cudaStream_t stream, topolow_interrupt_fn poll, void* user, bool* interrupted);
+// The loop of a row-block job of a fit batch (single rank): every remaining iteration, in windows of 5 on the plan's
+// stream with an event after each and at most two windows queued; waits with event queries, calling `stop` (the
+// batch's stop check, which rate-limits its own poll) every 200 us.  When `stop` returns true no further window is
+// issued and the queued ones finish (at most 10 iterations).  Returns true when that cut the fit short (it had not
+// converged, failed or issued all its iterations); the CUDA-event time is added to the plan's device time.
+bool row_run_windows(RowPlan& rp, const std::function<bool()>& stop);
 // All replicas of a map that live in this process: same device = lock-step emulation on one stream (every
 // wait is already satisfied when its kernel starts), distinct devices = concurrent.
 double row_run_local(RowPlan* const* plans, int n, int n_iters);

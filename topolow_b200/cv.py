@@ -16,6 +16,9 @@ import numpy as np
 from . import _lib
 from .core import build_problem, build_problem_coo, parse_dissimilarity, random_initial_positions
 
+# the modes a fit batch runs (core.euclidean_embedding's names); replay fits are single fits only
+_BATCH_MODES = {"coloured": _lib.MODE_COLOURED, "rowblock": _lib.MODE_ROWBLOCK}
+
 
 def error_calculator_comparison(predicted_dissimilarities, true_dissimilarities, input_dissimilarities=None):
     """R/error_metrics.R:55-144.  Returns report_df columns (flattened column-major, NaN = NA)
@@ -199,7 +202,7 @@ def _fold_job(value, code, is_na, holdout, preserve_order):
 
 def likelihood_batch(dissimilarity_matrix, samples, mapping_max_iter, relative_epsilon, folds=20,
                      preserve_order=True, *, fold_indices=None, init_list=None, rng=None, seed=0, device=0,
-                     precision="f32", interrupt=None):
+                     precision="f32", interrupt=None, mode="coloured"):
     """Evaluate many parameter samples at once.  `samples` is a list of dicts with keys N, k0,
     cooling_rate, c_repulsion; returns one likelihood_function() result per sample.  All
     len(samples) x folds fits run in a single topolow_fit_batch call.
@@ -218,22 +221,27 @@ def likelihood_batch(dissimilarity_matrix, samples, mapping_max_iter, relative_e
     not depend on it.
 
     interrupt: a callable polled while the fits run (see _lib.fit_batch); when it returns True the batch stops and
-    TopolowError(ERR_INTERRUPTED) is raised."""
+    TopolowError(ERR_INTERRUPTED) is raised.
+
+    mode: "coloured" (the default) or "rowblock", the names core.euclidean_embedding takes, for every fit of the batch.
+    "rowblock" is the mode for large maps and for N of 17 to 32 (the coloured mode takes N up to 16); each fold fit is
+    then exactly the single row-block fit."""
     rng = rng or np.random.default_rng(seed)
     value, code, is_na = parse_dissimilarity(dissimilarity_matrix)
     if fold_indices is None:
         fold_indices = make_folds(dissimilarity_matrix, folds, rng)
     fold_jobs = [_fold_job(value, code, is_na, np.asarray(h), preserve_order) for h in fold_indices]
     return _run_folds(fold_jobs, samples, mapping_max_iter, relative_epsilon, init_list, rng, seed, device, precision,
-                      interrupt)
+                      interrupt, mode)
 
 
 def likelihood_batch_coo(n, rows, cols, values, samples, mapping_max_iter, relative_epsilon, folds=20, *, diagonal=True,
-                         fold_cells=None, init_list=None, rng=None, seed=0, device=0, precision="f32", interrupt=None):
+                         fold_cells=None, init_list=None, rng=None, seed=0, device=0, precision="f32", interrupt=None,
+                         mode="coloured"):
     """likelihood_batch for a dissimilarity table (0-based rows / cols, values numbers or threshold strings): the folds
     are drawn and masked on the cell list (make_folds_cells / fold_problem_cells), nothing n x n is built, and the
     hold-out cells are scored on the device inside each fit.  Row order is the table's (preserve_order = TRUE).
-    `fold_cells` injects the drawn cell ids (see make_folds_cells); `interrupt` as in likelihood_batch."""
+    `fold_cells` injects the drawn cell ids (see make_folds_cells); `interrupt` and `mode` as in likelihood_batch."""
     rng = rng or np.random.default_rng(seed)
     full = build_problem_coo(n, rows, cols, values, preserve_order=True, diagonal=diagonal)
     base = n if diagonal else 0
@@ -246,7 +254,7 @@ def likelihood_batch_coo(n, rows, cols, values, samples, mapping_max_iter, relat
         prob["init_step"] = (max(float(prob["edge_dist"][kept].max()), 0.0) if kept.any() else 0.0) / n
         fold_jobs.append((prob, hi, hj, ht))
     return _run_folds(fold_jobs, samples, mapping_max_iter, relative_epsilon, init_list, rng, seed, device, precision,
-                      interrupt)
+                      interrupt, mode)
 
 
 def _initial_positions(prob, ndim, rng):
@@ -257,9 +265,11 @@ def _initial_positions(prob, ndim, rng):
 
 
 def _run_folds(fold_jobs, samples, mapping_max_iter, relative_epsilon, init_list, rng, seed, device, precision,
-               interrupt=None):
+               interrupt=None, mode="coloured"):
     """All len(samples) x len(fold_jobs) fits in one topolow_fit_batch call, pooled as R/adaptive_sampling.R:2695-2725."""
     prec_c = {"f32": _lib.PREC_F32, "f64": _lib.PREC_F64_EXACT}[precision]
+    if mode not in _BATCH_MODES:
+        raise ValueError(f"mode must be one of {sorted(_BATCH_MODES)}, not {mode!r}")
     # hold-out cells in the row numbering of the fold's training problem: they are scored on the device
     # at the end of each fit (topolow_problem.holdout_*), the positions need not come back for that
     fold_holdout = []
@@ -285,7 +295,8 @@ def _run_folds(fold_jobs, samples, mapping_max_iter, relative_epsilon, init_list
                              edge_j=prob["edge_j"], edge_dist=prob["edge_dist"], edge_thresh=prob["edge_thresh"],
                              n_iter=int(mapping_max_iter), k0=s["k0"], cooling_rate=s["cooling_rate"],
                              c_repulsion=s["c_repulsion"], relative_epsilon=relative_epsilon, convergence_window=5,
-                             precision=prec_c, seed=seed + 1000003 * s_idx + f_idx, holdout=fold_holdout[f_idx]))
+                             precision=prec_c, seed=seed + 1000003 * s_idx + f_idx, holdout=fold_holdout[f_idx],
+                             mode=_BATCH_MODES[mode]))
             meta.append((s_idx, f_idx, len(jobs) - 1))
     extra = {} if interrupt is None else {"interrupt": interrupt}
     results = _lib.fit_batch(jobs, device=device, **extra) if jobs else []
@@ -316,10 +327,10 @@ def _run_folds(fold_jobs, samples, mapping_max_iter, relative_epsilon, init_list
 
 
 def likelihood_function(dissimilarity_matrix, mapping_max_iter, relative_epsilon, N, k0, cooling_rate, c_repulsion,
-                        folds=20, num_cores=1, preserve_order=True, *, interrupt=None, **kw):
+                        folds=20, num_cores=1, preserve_order=True, *, interrupt=None, mode="coloured", **kw):
     """Single-sample form with the reference's signature (R/adaptive_sampling.R:2552-2555);
     num_cores is accepted and ignored (the folds already run concurrently on the device).
-    `interrupt` as in likelihood_batch."""
+    `interrupt` and `mode` as in likelihood_batch."""
     return likelihood_batch(dissimilarity_matrix, [dict(N=N, k0=k0, cooling_rate=cooling_rate,
                                                         c_repulsion=c_repulsion)], mapping_max_iter,
-                            relative_epsilon, folds, preserve_order, interrupt=interrupt, **kw)[0]
+                            relative_epsilon, folds, preserve_order, interrupt=interrupt, mode=mode, **kw)[0]

@@ -187,7 +187,8 @@ def draw_from_marginals(marginals, rng, size=1):
 
 
 def adaptive_mc_batch(samples, dissimilarity_matrix, iterations, chains, mapping_max_iter, relative_epsilon, folds=20,
-                      preserve_order=True, *, rng=None, evaluate=None, device=0, verbose=False, interrupt=None):
+                      preserve_order=True, *, rng=None, evaluate=None, device=0, verbose=False, interrupt=None,
+                      mode="coloured"):
     """`chains` chains of adaptive_MC_sampling (R/adaptive_sampling.R:1593-1790) advanced together: per round the
     weighted marginals of the shared table are computed once, every chain draws one parameter set, all chains x folds
     fits run as one device batch, valid rows are appended (invalid evaluations are skipped, :1683-1686).  Returns the
@@ -195,7 +196,9 @@ def adaptive_mc_batch(samples, dissimilarity_matrix, iterations, chains, mapping
     The reference's chains are separate processes that append to one CSV whenever they finish; here a round's draws
     all see the table as it was when the round began.
     `interrupt` is polled while a round's batch runs (cv.likelihood_batch); when it returns True the batch stops and
-    TopolowError(ERR_INTERRUPTED) is raised.  `device` may be a sequence of ordinals (cv.likelihood_batch)."""
+    TopolowError(ERR_INTERRUPTED) is raised.  `device` may be a sequence of ordinals (cv.likelihood_batch).  `mode`
+    ("coloured" or "rowblock", as in cv.likelihood_batch) is the mode of every fit: "rowblock" for large maps and for
+    N above 16."""
     rng = rng or np.random.default_rng()
     table = {k: np.array(v, copy=True) for k, v in _as_table(samples).items()}
     required = list(PAR_NAMES) + ["NLL", "Holdout_MAE"]
@@ -207,7 +210,7 @@ def adaptive_mc_batch(samples, dissimilarity_matrix, iterations, chains, mapping
 
         def evaluate(matrix, sets):
             return cv.likelihood_batch(matrix, sets, mapping_max_iter, relative_epsilon, folds, preserve_order,
-                                       rng=rng, device=device, interrupt=interrupt)
+                                       rng=rng, device=device, interrupt=interrupt, mode=mode)
     for it in range(int(iterations)):
         try:
             with warnings.catch_warnings():

@@ -82,7 +82,7 @@ typedef struct {
   const int32_t* edge_i;            /* 0-based */
   const int32_t* edge_j;            /* 0-based, edge_i[e] != edge_j[e] */
   const double* edge_dist;          /* target distance */
-  const int32_t* edge_thresh;       /* 0 exact, +1 '>' , -1 '<'  (R/core.R:346,358-359) */
+  const int32_t* edge_thresh;       /* 0 exact, +1 '>' , -1 '<'  (R/core.R:346,358-359); any other code is refused */
   const int32_t* degrees;           /* rowSums(!is.na), diagonal included (R/core.R:340-341) */
   const double* initial_positions;  /* n x ndim, column-major like an R matrix */
   /* ---- optional: cells held out of this fit, scored on the final (best) positions before they leave
@@ -295,12 +295,14 @@ TOPOLOW_API int topolow_shard_run_local(topolow_shard* const* shards, int32_t n,
  * of {repulsion, springs, edge MAE, controller, snapshot}, the number of MAE launches seen, {combine}. */
 TOPOLOW_API int topolow_shard_time_kernels(topolow_shard* shard, int32_t n_iters, double* out, int32_t cap);
 TOPOLOW_API int topolow_shard_result(topolow_shard* shard, topolow_result* result);
-/* out (up to 18 values): {slots, ndim, stride, n_ranks, rank, row0, own_rows, partner_chunks, spring_records,
+/* out (up to 20 values): {slots, ndim, stride, n_ranks, rank, row0, own_rows, partner_chunks, spring_records,
  * mae_records, kernel_launches, iterations_done, stopped, peer_store_bytes_per_iteration, repulsion_items (work items
  * of one pass of repulsion_form: 256 own rows x one chunk of 2048 partners in form 5, x a group of chunks in form 11),
  * repulsion_ctas, repulsion_form (5: FP32 difference form, 11: distances and accumulation on tcgen05),
  * tensor_form_iterations (form 11 chosen by the policy runs adaptively: the device picks the form of every iteration;
- * the count is read back by topolow_shard_result, -1 before that or when the form is not adaptive)}. */
+ * the count is read back by topolow_shard_result, -1 before that or when the form is not adaptive), walk_ring (partner rows
+ * in flight per warp of the spring and MAE walks: 8 when the rank owns at most 2 x SMs row blocks of 128, else 4),
+ * walk_ctas (grid of the spring walk beside the repulsion pass: under form 11 one CTA per SM walks several row blocks)}. */
 TOPOLOW_API int topolow_shard_info(const topolow_shard* shard, int64_t* out, int32_t cap);
 /* slot_of_point of the row-block layout (a pure function of n). */
 TOPOLOW_API int topolow_shard_slot_order(int64_t n, int32_t* slot_of_point_out);

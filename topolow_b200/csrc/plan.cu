@@ -37,6 +37,11 @@ void validate(const topolow_problem& pb, const topolow_params& pr) {
   if (pb.n_edges > 0 && (!pb.edge_i || !pb.edge_j || !pb.edge_dist || !pb.edge_thresh))
     throw BadArg("edge arrays are required when n_edges > 0");
   if (pb.n_edges < 0 || pb.n_edges >= (1ll << 32)) throw BadArg("n_edges out of range");
+  // The kernels read 1 as '>' and any other non-zero code as '<'; the oracles read them otherwise.  Only the three
+  // codes the header documents mean the same thing everywhere.
+  bool bad_code = false;
+  for (int64_t e = 0; e < pb.n_edges; ++e) bad_code |= (uint32_t)(pb.edge_thresh[e] + 1) > 2u;   // no early exit: vectorised
+  if (bad_code) throw BadArg("edge_thresh must be -1, 0 or 1");
 }
 
 // Fisher-Yates with splitmix64: identical on every host.

@@ -1564,11 +1564,12 @@ void row_result(RowPlan& rp, topolow_result& res, bool interrupted) {
 
 void row_info(const RowPlan& rp, int64_t* out, int cap) {
   const RowDev& dv = rp.dv;
-  const int64_t v[18] = {dv.slots, dv.D, dv.Dp, dv.G, dv.rank, dv.row0, dv.rows, dv.chunks, rp.n_recs, rp.n_mrecs, rp.launches,
+  const int64_t v[20] = {dv.slots, dv.D, dv.Dp, dv.G, dv.rank, dv.row0, dv.rows, dv.chunks, rp.n_recs, rp.n_mrecs, rp.launches,
                          rp.h_flag ? rp.h_flag[1] : 0, rp.h_flag ? rp.h_flag[0] : 0,
                          (int64_t)(dv.G - 1) * dv.rows * dv.Dp * 4,   // position bytes this rank stores into its peers per iteration
-                         rp.rep_items, rp.rep_ctas, rp.rep_form, rp.tensor_iters};
-  for (int i = 0; i < cap && i < 18; ++i) out[i] = v[i];
+                         rp.rep_items, rp.rep_ctas, rp.rep_form, rp.tensor_iters,
+                         rp.deep_ring ? 8 : 4, rp.walk_ctas};
+  for (int i = 0; i < cap && i < 20; ++i) out[i] = v[i];
 }
 
 }  // namespace tl

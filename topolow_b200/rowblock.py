@@ -25,7 +25,7 @@ from ._lib import OK, TopolowError
 INFO_KEYS = ["slots", "ndim", "stride", "n_ranks", "rank", "row0", "own_rows", "partner_chunks", "spring_records",
              "mae_records", "launches", "iterations_done", "stopped", "peer_store_bytes_per_iteration",
              "repulsion_items", "repulsion_ctas", "repulsion_form",
-             "tensor_form_iterations"]
+             "tensor_form_iterations", "walk_ring", "walk_ctas"]
 KERNELS = ["repulse", "spring", "mae", "controller", "snapshot"]
 
 
@@ -92,8 +92,8 @@ class Shard:
         return _lib.result_dict(res, out, tr)
 
     def info(self):
-        v = (C.c_int64 * 18)()
-        self._L.topolow_shard_info(self._h, v, 18)
+        v = (C.c_int64 * len(INFO_KEYS))()
+        self._L.topolow_shard_info(self._h, v, len(INFO_KEYS))
         return dict(zip(INFO_KEYS, [int(x) for x in v]))
 
     def close(self):
